@@ -9,6 +9,11 @@ head-tracking grid, one HRTF set per rank -> weak scaling, no data-path collecti
 ONE JSON line.  `value` is device-resident throughput (inputs already in HBM, CUDA events on the
 library's stream, max over ranks); `e2e` goes through the public host API (pinned host buffers,
 H2D + D2H inside the timed region, plus the NCCL gather of the banks onto rank 0 for N > 1).
+
+`--dump-outputs DIR` writes what the last timed step designed on rank 0, so that two builds can be compared output
+for output: DIR/wL.npy and DIR/wR.npy, float64 [orientation, microphone, tap], the filters of a fixed sample of
+DUMP_SETS orientations of the batch (every orientation when the batch is that small; indices in ascending order,
+drawn with seed DUMP_SEED).  The inputs are synthetic and seeded, so equal arguments give equal inputs.
 """
 from __future__ import annotations
 
@@ -31,6 +36,8 @@ UNIT = "filter sets/s"
 ORDER, LEN = 4, 512
 # SURVEY.md 8(d): direct formulation, per filter set (512 bins): 22.3 GFLOP
 ALGO_GFLOP_PER_SET = 22.3
+# 128 filter-set pairs of 2 x 32 x 512 doubles: 32 MiB on disk
+DUMP_SETS, DUMP_SEED = 128, 0
 
 
 def parse():
@@ -45,7 +52,12 @@ def parse():
     ap.add_argument("--no-render", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-spot-check", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a fixed sample of the filters the last timed step designed to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def problem(rank: int, n_orient: int):
@@ -259,6 +271,12 @@ def main():
             ev[i][1].record(stream)
         torch.cuda.synchronize()
     emdist.barrier()
+    if args.dump_outputs and rank == 0:     # before the steps below write the banks again
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        pick = np.sort(np.random.default_rng(DUMP_SEED).choice(B, size=min(B, DUMP_SETS), replace=False))
+        pick = torch.from_numpy(pick).to(dev)
+        for name, bank in (("wL", d_wL), ("wR", d_wR)):
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), bank.index_select(0, pick).cpu().numpy())
     ms_local = sum(a.elapsed_time(b) for a, b in ev)
     ms = emdist.max_over_ranks(ms_local, dev)
     prof = h.profile_read()
@@ -302,7 +320,7 @@ def main():
         torch.cuda.synchronize()     # every host shard (and rank 0's gathered device banks) is complete here
         return emdist.max_over_ranks(time.perf_counter() - t0, dev)
 
-    e2e_steps = max(5, min(args.steps, 10))
+    e2e_steps = args.steps
     e2e_s = timed_e2e(sd, e2e_steps)
     e2e_value = world * B * e2e_steps / e2e_s
     # the e2e path and the device-resident path must have produced the same banks (same inputs)
@@ -328,7 +346,7 @@ def main():
         pr0 = problem(0, args.orient)
         ss = emdist.ShardedDesigner(h, pr0["hL"], pr0["hR"], pr0["az"], pr0["ze"], pr0["r"], pr0["maz"], pr0["mze"],
                                     ORDER, pr0["fs"], LEN, pr0["R"], config=cfg)
-        s_steps = max(5, min(args.steps, 10))
+        s_steps = args.steps
         s_s = timed_e2e(ss, s_steps)
         strong = {"orientations_total": int(ss.n_total), "orientations_per_gpu": int(ss.n_local),
                   "ms_per_batch": s_s / s_steps * 1e3, "value": ss.n_total * s_steps / s_s, "unit": UNIT,
