@@ -74,6 +74,12 @@ SIGNATURES = {
     "emagls_binaural_decode": (C.c_int, [C.c_void_p, c_dp, C.c_longlong, C.c_int, c_dp, c_dp, C.c_int, C.c_int, c_dp]),
     "emagls_binaural_decode_dev": (C.c_int, [C.c_void_p, c_dp, C.c_longlong, C.c_int, c_dp, c_dp, C.c_int, C.c_int,
                                              c_dp]),
+    "emagls_binaural_decode_tracked": (C.c_int, [C.c_void_p, c_dp, C.c_longlong, C.c_int, c_dp, c_dp, C.c_int, C.c_int,
+                                                 C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.c_longlong, C.c_int,
+                                                 c_dp]),
+    "emagls_binaural_decode_tracked_dev": (C.c_int, [C.c_void_p, c_dp, C.c_longlong, C.c_int, c_dp, c_dp, C.c_int,
+                                                     C.c_int, C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.c_longlong,
+                                                     C.c_int, c_dp]),
     "emagls_get_sh": (C.c_int, [C.c_void_p, C.c_int, c_dp, c_dp, C.c_int, C.c_int, c_dp]),
     "emagls_group_delay": (C.c_int, [C.c_void_p, c_dp, C.c_int, C.c_int, C.c_int, C.c_double, c_dp, c_dp]),
     "emagls_sph_modal_coeffs": (C.c_int, [C.c_void_p, C.c_int, c_dp, C.c_int, C.c_int, c_dp]),

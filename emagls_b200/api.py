@@ -23,7 +23,7 @@ from ._lib import Config, EmaglsError, Handle, RadialParams, default_handle  # n
 
 __all__ = ["getEMagLs2Filters", "getEMagLsFilters", "getMagLsFilters", "getLsFilters",
            "getEMagLsFiltersFromAtf", "getEMagLsFiltersEMAinCH", "getEMagLsFiltersEMAinSH",
-           "getSMAIRMatrix", "binauralDecode", "getSH", "sphModalCoeffs", "regularizedApply", "grpdelay",
+           "getSMAIRMatrix", "binauralDecode", "binauralDecodeTracked", "getSH", "sphModalCoeffs", "regularizedApply", "grpdelay",
            "getRadialFilter", "applyRadialFilter", "encodeSH", "encodeCH", "rotateSH", "getMagLsFilters2D",
            "getMagLsSphericalHeadFilter", "getMagLsArrayDiffuseFilter", "Handle", "EmaglsError"]
 
@@ -425,6 +425,44 @@ def binauralDecode(inp, inFs, decodingFilterLeft, decodingFilterRight, decodingF
         return dec(x, wL, wR)
     # complex-basis signals and filters (shDefinition = 'complex'): the reference keeps real(sum_ch x * w)
     # (binauralDecode.m:59-64) = sum_ch (Re x * Re w - Im x * Im w): two real renders on the device
+    out = dec(x.real, wL.real, wR.real)
+    xi, wli, wri = np.imag(x), np.imag(wL), np.imag(wR)
+    if np.any(xi) and (np.any(wli) or np.any(wri)):
+        out -= dec(xi, wli, wri)
+    return out
+
+
+def binauralDecodeTracked(inp, wL, wR, track, hop, fade=None, compensateDelay=False, *, firstSample=0, handle=None):
+    """Head-tracked binauralDecode (not in the reference API; emagls_binaural_decode_tracked): ``inp`` [samples, ch]
+    rendered with page ``track[f]`` (0-based) of the bank ``wL``, ``wR`` [len, ch, pages] (a [len, ch] filter pair is
+    one page) for the samples [f hop, (f + 1) hop) of the track's time axis, crossfading linearly from the previous
+    frame's page over the first ``fade`` samples of every frame (default ``hop``; 0 switches hard).  ``firstSample`` is
+    the position of inp[0] on the track's time axis.  Complex signals or banks (complex-basis designers) are rendered as
+    real(sum_ch x * w), like binauralDecode: two real tracked renders (the crossfade weights are real)."""
+    h = handle or default_handle()
+    x, wL, wR = np.asarray(inp), np.asarray(wL), np.asarray(wR)
+    if wL.ndim == 2:
+        wL, wR = wL[:, :, None], wR[:, :, None]
+    if x.ndim != 2 or wL.shape != wR.shape or wL.ndim != 3 or wL.shape[1] != x.shape[1]:
+        raise ValueError("size mismatch between input channels and the filter bank")
+    trk = np.ascontiguousarray(np.asarray(track).ravel())
+    if not np.issubdtype(trk.dtype, np.integer) or (trk.size and (trk.min() < -2**31 or trk.max() >= 2**31)):
+        raise ValueError("track must hold integer page numbers")
+    trk = trk.astype(np.int32)
+    n, ch = x.shape
+    ln, _, pages = wL.shape
+    hop = int(hop)
+    fade = hop if fade is None else int(fade)
+    rows = n - (ln // 2 - 1) if compensateDelay else n
+
+    def dec(xr, wl, wr):
+        out = np.zeros((rows, 2), order="F")
+        h.check(h.lib.emagls_binaural_decode_tracked(h.ptr, _p(_f(xr)), n, ch, _p(_f(wl)), _p(_f(wr)), ln, pages,
+                                                     _p(trk), trk.size, hop, fade, int(firstSample),
+                                                     1 if compensateDelay else 0, _p(out)))
+        return out
+    if not (np.iscomplexobj(x) or np.iscomplexobj(wL) or np.iscomplexobj(wR)):
+        return dec(x, wL, wR)
     out = dec(x.real, wL.real, wR.real)
     xi, wli, wri = np.imag(x), np.imag(wL), np.imag(wR)
     if np.any(xi) and (np.any(wli) or np.any(wri)):

@@ -44,11 +44,12 @@ struct emagls_ctx {
   long long prof_n[EM_PROF_NUM] = {0};
   // render: cuFFT plans are expensive to build (milliseconds), so they live with the handle
   struct RenderPlans {
-    int N = 0, L = 0, num_ch = 0, chunk = 0;
+    int N = 0, L = 0, num_ch = 0, nbc = 0, filt_batch = 0, inv_batch = 0;
     int fwd = 0, inv = 0, filt = 0;   // cufftHandle values (0 = not created)
     int edge = 0;                     // one boundary block of every channel (zero-padded staging)
     std::vector<std::pair<int, int>> direct;  // (batch, plan): interior blocks read straight from the input
   } render_plans;
+  RenderPlans tracked_plans;          // head-tracked render (tracked_render.cu), kept apart from the static render's
   // per-channel FIR of the front end (frontend.cu): cuFFT plans keyed by (size, batch, direction)
   struct FirPlan { int N, batch, inverse, plan; };
   std::vector<FirPlan> fir_plans;
@@ -180,7 +181,7 @@ struct DesignArgs {
   const double* Y_mic = nullptr;
 };
 void design_factored(emagls_ctx* h, const emagls_config& cfg, const DesignArgs& a);
-void destroy_render_plans(emagls_ctx* h);  // render.cu
+void destroy_render_plans(emagls_ctx* h);  // render.cu (static and head-tracked render)
 void destroy_fir_plans(emagls_ctx* h);     // frontend.cu
 // radFilts [K][(order+1)] (row index k) on the device (getRadialFilter.m:42-70)
 void radial_filter_dev(emagls_ctx* h, Arena& ar, const emagls_config& cfg, const emagls_radial_params& rp, int order,

@@ -2,27 +2,20 @@
 // i.e. the first num_samples samples of the multichannel linear convolution, as a partitioned
 // overlap-save convolution.  cuFFT performs the D2Z / Z2D transforms only; the per-bin
 // multiply-accumulate over channels (the HBM-bound part) is the hand-written kernel below.
-#include <cufft.h>
 #include <algorithm>
 #include <cstdint>
 #include <cstdlib>
 #include <vector>
-#include "engine.h"
+#include "render.h"
 
 namespace emagls {
-namespace {
 
-#define EM_FFT(expr)                                                                              \
-  do {                                                                                            \
-    cufftResult _r = (expr);                                                                      \
-    if (_r != CUFFT_SUCCESS)                                                                      \
-      throw ::emagls::Fail{EMAGLS_ERR_CUDA, std::string(#expr) + ": cufft error " + std::to_string((int)_r)}; \
-  } while (0)
+int env_int(const char* name, int dflt) {
+  const char* e = getenv(name);
+  return e ? atoi(e) : dflt;
+}
 
-constexpr int MAX_EDGE = 8;  // staged boundary blocks per chunk (head + tail)
-
-void drop_plans(emagls_ctx* h) {
-  auto& rp = h->render_plans;
+void drop_plans(emagls_ctx::RenderPlans& rp) {
   if (rp.fwd) cufftDestroy(rp.fwd);
   if (rp.inv) cufftDestroy(rp.inv);
   if (rp.filt) cufftDestroy(rp.filt);
@@ -31,19 +24,20 @@ void drop_plans(emagls_ctx* h) {
   rp = emagls_ctx::RenderPlans{};
 }
 
-// (Re)build the plans of the render for this geometry; cached in the handle between calls.
-void ensure_plans(emagls_ctx* h, int N, int L, int num_ch, int chunk, int nbc) {
-  auto& rp = h->render_plans;
-  if (rp.N == N && rp.L == L && rp.num_ch == num_ch && rp.chunk == chunk && rp.fwd && rp.inv && rp.filt) return;
-  drop_plans(h);
+void ensure_plans(emagls_ctx* h, emagls_ctx::RenderPlans& rp, int N, int L, int num_ch, int nbc, int filt_batch,
+                  int inv_batch) {
+  if (rp.N == N && rp.L == L && rp.num_ch == num_ch && rp.nbc == nbc && rp.filt_batch == filt_batch &&
+      rp.inv_batch == inv_batch && rp.fwd && rp.inv && rp.filt)
+    return;
+  drop_plans(rp);
   const int F = N / 2 + 1;
   int n[1] = {N};
   cufftHandle pf = 0, pi = 0, pw = 0;
-  EM_FFT(cufftPlanMany(&pw, 1, n, nullptr, 1, N, nullptr, 1, F, CUFFT_D2Z, 2 * num_ch));
+  EM_FFT(cufftPlanMany(&pw, 1, n, nullptr, 1, N, nullptr, 1, F, CUFFT_D2Z, filt_batch));
   // overlapping input batches: block j of channel ch starts at (ch * nbc + j) * L
   int inembed[1] = {N}, onembed[1] = {F};
   EM_FFT(cufftPlanMany(&pf, 1, n, inembed, 1, L, onembed, 1, F, CUFFT_D2Z, num_ch * nbc));
-  EM_FFT(cufftPlanMany(&pi, 1, n, nullptr, 1, F, nullptr, 1, N, CUFFT_Z2D, 2 * chunk));
+  EM_FFT(cufftPlanMany(&pi, 1, n, nullptr, 1, F, nullptr, 1, N, CUFFT_Z2D, inv_batch));
   // boundary block e of every channel: in xe[ch][e][N], out X[ch][b][F]
   cufftHandle pe = 0;
   int e_in[1] = {N};
@@ -52,13 +46,15 @@ void ensure_plans(emagls_ctx* h, int N, int L, int num_ch, int chunk, int nbc) {
   EM_FFT(cufftSetStream(pf, h->stream));
   EM_FFT(cufftSetStream(pi, h->stream));
   EM_FFT(cufftSetStream(pe, h->stream));
-  rp.N = N; rp.L = L; rp.num_ch = num_ch; rp.chunk = chunk; rp.fwd = pf; rp.inv = pi; rp.filt = pw; rp.edge = pe;
+  rp.N = N; rp.L = L; rp.num_ch = num_ch; rp.nbc = nbc; rp.filt_batch = filt_batch; rp.inv_batch = inv_batch;
+  rp.fwd = pf; rp.inv = pi; rp.filt = pw; rp.edge = pe;
 }
+
+namespace {
 
 // interior blocks of one channel straight from the caller's signal: `batch` overlapping transforms at
 // distance L (cuFFT plans have a fixed batch: one plan per distinct count, normally one or two)
-cufftHandle direct_plan(emagls_ctx* h, int N, int L, int batch) {
-  auto& rp = h->render_plans;
+cufftHandle direct_plan(emagls_ctx* h, emagls_ctx::RenderPlans& rp, int N, int L, int batch) {
   for (auto& d : rp.direct)
     if (d.first == batch) return d.second;
   const int F = N / 2 + 1;
@@ -601,12 +597,72 @@ fused_render16_kernel(const double* __restrict__ in, long long num_samples, int 
   }
 }
 
-int env_int(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
+}  // namespace
+
+ForwardStage::ForwardStage(emagls_ctx* h_, emagls_ctx::RenderPlans& rp_, Arena& ar, const double* in_,
+                           long long num_samples_, int num_ch_, int N_, int L_, int ov_, int nbc_)
+    : h(h_), rp(rp_), in(in_), num_samples(num_samples_), num_ch(num_ch_), N(N_), L(L_), ov(ov_), nbc(nbc_) {
+  seg_len = (long long)nbc * L;
+  direct = env_int("EMAGLS_RENDER_DIRECT", 1) != 0 && (num_samples % 2 == 0) &&
+           (reinterpret_cast<uintptr_t>(in) % 16 == 0);
+  b_int_lo = extra_blocks(ov, L);                                                          // input starts at >= 0
+  b_int_hi = (num_samples - N + ov >= 0) ? (num_samples - N + ov) / L : -1;                // ends inside
+  // the last nex blocks of the last channel read up to N samples past the staged segments
+  xp = direct ? ar.get<double>((size_t)MAX_EDGE * N * num_ch) : ar.get<double>((size_t)seg_len * num_ch + N);
+  if (!direct) EM_CUDA(cudaMemsetAsync(xp + seg_len * num_ch, 0, (size_t)N * sizeof(double), h->stream));
 }
 
-}  // namespace
+void ForwardStage::run(long long b0, long long nbk, cplx* X) {
+  cudaStream_t st = h->stream;
+  const int F = N / 2 + 1;
+  if (direct) {
+    const long long lo = std::max(b0, b_int_lo), hi = std::min(b0 + nbk - 1, b_int_hi);
+    if (hi >= lo) {
+      ProfSpan ps(h, EM_PROF_RENDER_FFT);
+      cufftHandle pd = direct_plan(h, rp, N, L, (int)(hi - lo + 1));
+      for (int ch = 0; ch < num_ch; ++ch)
+        EM_FFT(cufftExecD2Z(pd, const_cast<double*>(in) + (long long)ch * num_samples + lo * L - ov,
+                            reinterpret_cast<cufftDoubleComplex*>(X + ((long long)ch * nbc + (lo - b0)) * F)));
+    }
+    // boundary blocks of this chunk, MAX_EDGE at a time
+    long long eb[MAX_EDGE];
+    int ne = 0;
+    auto flush = [&]() {
+      for (int e = 0; e < ne; ++e) {
+        ProfSpan ps(h, EM_PROF_RENDER_STAGE);
+        long long total = (long long)N * num_ch;
+        stage_input_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(in, num_samples, num_ch, eb[e] * L - ov, N,
+                                                                          (long long)MAX_EDGE * N, xp + (long long)e * N);
+        EM_CUDA(cudaGetLastError());
+      }
+      for (int e = 0; e < ne; ++e) {
+        ProfSpan ps(h, EM_PROF_RENDER_FFT);
+        EM_FFT(cufftExecD2Z(rp.edge, xp + (long long)e * N, reinterpret_cast<cufftDoubleComplex*>(X + (eb[e] - b0) * F)));
+      }
+      h->launches += ne;
+      ne = 0;
+    };
+    for (long long b = b0; b < b0 + nbk; ++b) {
+      if (b >= lo && b <= hi) { b = hi; continue; }
+      eb[ne++] = b;
+      if (ne == MAX_EDGE) flush();
+    }
+    flush();
+  } else {
+    {
+      ProfSpan ps(h, EM_PROF_RENDER_STAGE);
+      long long total = seg_len * num_ch;
+      stage_input_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(in, num_samples, num_ch, b0 * L - ov, seg_len,
+                                                                        seg_len, xp);
+      EM_CUDA(cudaGetLastError());
+    }
+    {
+      ProfSpan ps(h, EM_PROF_RENDER_FFT);
+      EM_FFT(cufftExecD2Z(rp.fwd, xp, reinterpret_cast<cufftDoubleComplex*>(X)));
+    }
+    h->launches += 1;
+  }
+}
 
 // Overlap-save geometry: FFT size N (power of two), overlap ov >= len - 1 (even), hop L = N - ov.
 // Block b takes the N input samples starting at b*L - ov and yields output samples [b*L, (b+1)*L).
@@ -635,7 +691,7 @@ void binaural_decode_dev(emagls_ctx* h, const double* in, long long num_samples,
   const long long out_rows = num_samples - skip;
   EM_REQUIRE(out_rows > 0, "signal shorter than the compensated delay");
   const long long nblk_total = (num_samples + L - 1) / L;
-  const int nex = (ov + L - 1) / L;   // extra hops per channel so that the overlapping batch has a uniform distance L
+  const int nex = ForwardStage::extra_blocks(ov, L);  // extra hops per channel: the overlapping batch has a uniform distance L
   // blocks per chunk: as many as a memory budget allows (measured on B200: launch-bound below a few
   // hundred blocks; one chunk for a 10-minute signal is fastest, the intermediates do not need to stay
   // in L2).  EMAGLS_RENDER_CHUNK / EMAGLS_RENDER_WS_MB override.
@@ -653,9 +709,8 @@ void binaural_decode_dev(emagls_ctx* h, const double* in, long long num_samples,
   }
   const int chunk = (int)std::min<long long>({nblk_total, (long long)chunk_max, 65535LL * 4});
   const int nbc = chunk + nex;
-  const long long seg_len = (long long)nbc * L;
-  ensure_plans(h, N, L, num_ch, chunk, nbc);
-  const auto& rp = h->render_plans;
+  auto& rp = h->render_plans;
+  ensure_plans(h, rp, N, L, num_ch, nbc, 2 * num_ch, 2 * chunk);
 
   // filter spectra Hw[ear][ch][F]
   cplx* Hw = ar.get<cplx>((size_t)2 * num_ch * F);
@@ -733,71 +788,14 @@ void binaural_decode_dev(emagls_ctx* h, const double* in, long long num_samples,
     return;
   }
 
-  // Forward transforms.  Direct route (default when every channel of the caller's signal is 16-byte
-  // aligned): interior blocks are transformed in place from `in`, one cuFFT call per channel, and only
-  // the blocks that overlap the ends of the signal are staged zero-padded.  Staged route: the whole
-  // chunk is copied into a segment buffer first (one cuFFT call per chunk).
-  const bool direct = env_int("EMAGLS_RENDER_DIRECT", 1) != 0 && (num_samples % 2 == 0) &&
-                      (reinterpret_cast<uintptr_t>(in) % 16 == 0);
-  const long long b_int_lo = nex;                                                   // input starts at >= 0
-  const long long b_int_hi = (num_samples - N + ov >= 0) ? (num_samples - N + ov) / L : -1;  // ends inside
-  // the last nex blocks of the last channel read up to N samples past the staged segments
-  double* xp = direct ? ar.get<double>((size_t)MAX_EDGE * N * num_ch) : ar.get<double>((size_t)seg_len * num_ch + N);
+  ForwardStage fwd(h, rp, ar, in, num_samples, num_ch, N, L, ov, nbc);
   cplx* X = ar.get<cplx>((size_t)num_ch * nbc * F);
   cplx* Y = ar.get<cplx>((size_t)2 * chunk * F);
   double* yseg = ar.get<double>((size_t)2 * chunk * N);
-  if (!direct) EM_CUDA(cudaMemsetAsync(xp + seg_len * num_ch, 0, (size_t)N * sizeof(double), st));
   constexpr int BT = 4, CU = 4;
   for (long long b0 = 0; b0 < nblk_total; b0 += chunk) {
     const long long s0 = b0 * L;
-    if (direct) {
-      const long long nbk = std::min<long long>(chunk, nblk_total - b0);
-      const long long lo = std::max(b0, b_int_lo), hi = std::min(b0 + nbk - 1, b_int_hi);
-      if (hi >= lo) {
-        ProfSpan ps(h, EM_PROF_RENDER_FFT);
-        cufftHandle pd = direct_plan(h, N, L, (int)(hi - lo + 1));
-        for (int ch = 0; ch < num_ch; ++ch)
-          EM_FFT(cufftExecD2Z(pd, const_cast<double*>(in) + (long long)ch * num_samples + lo * L - ov,
-                              reinterpret_cast<cufftDoubleComplex*>(X + ((long long)ch * nbc + (lo - b0)) * F)));
-      }
-      // boundary blocks of this chunk, MAX_EDGE at a time
-      long long eb[MAX_EDGE];
-      int ne = 0;
-      auto flush = [&]() {
-        for (int e = 0; e < ne; ++e) {
-          ProfSpan ps(h, EM_PROF_RENDER_STAGE);
-          long long total = (long long)N * num_ch;
-          stage_input_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(in, num_samples, num_ch, eb[e] * L - ov, N,
-                                                                            (long long)MAX_EDGE * N, xp + (long long)e * N);
-          EM_CUDA(cudaGetLastError());
-        }
-        for (int e = 0; e < ne; ++e) {
-          ProfSpan ps(h, EM_PROF_RENDER_FFT);
-          EM_FFT(cufftExecD2Z(rp.edge, xp + (long long)e * N, reinterpret_cast<cufftDoubleComplex*>(X + (eb[e] - b0) * F)));
-        }
-        h->launches += ne;
-        ne = 0;
-      };
-      for (long long b = b0; b < b0 + nbk; ++b) {
-        if (b >= lo && b <= hi) { b = hi; continue; }
-        eb[ne++] = b;
-        if (ne == MAX_EDGE) flush();
-      }
-      flush();
-    } else {
-      {
-        ProfSpan ps(h, EM_PROF_RENDER_STAGE);
-        long long total = seg_len * num_ch;
-        stage_input_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(in, num_samples, num_ch, s0 - ov, seg_len,
-                                                                          seg_len, xp);
-        EM_CUDA(cudaGetLastError());
-      }
-      {
-        ProfSpan ps(h, EM_PROF_RENDER_FFT);
-        EM_FFT(cufftExecD2Z(rp.fwd, xp, reinterpret_cast<cufftDoubleComplex*>(X)));
-      }
-      h->launches += 1;
-    }
+    fwd.run(b0, std::min<long long>(chunk, nblk_total - b0), X);
     {
       ProfSpan ps(h, EM_PROF_RENDER_MAC);
       // Y is laid out [ear][chunk][F] for the fixed-size inverse plan (a partial last chunk
@@ -822,7 +820,10 @@ void binaural_decode_dev(emagls_ctx* h, const double* in, long long num_samples,
   // stream-ordered: the arena's cudaFreeAsync calls queue behind the work above
 }
 
-void destroy_render_plans(emagls_ctx* h) { drop_plans(h); }
+void destroy_render_plans(emagls_ctx* h) {
+  drop_plans(h->render_plans);
+  drop_plans(h->tracked_plans);
+}
 
 }  // namespace emagls
 

@@ -225,6 +225,31 @@ int emagls_binaural_decode_dev(emagls_handle h, const double* in, long long num_
                                int num_ch, const double* wL, const double* wR, int len,
                                int compensate_delay, double* out);
 
+/* ---- head-tracked binauralDecode (not in the reference API) ---------------------------------------------------
+ * Renders `in` [num_samples x num_ch] with a filter bank wL, wR [len x num_ch x num_pages] (column-major, the layout
+ * the designers return: page = set * num_orient + orient) while a head tracker picks the page: track[f] (0-based, int32,
+ * num_frames entries) is the page of frame f, which covers samples [f hop, (f + 1) hop) of the track's time axis, and
+ * in[0] sits at first_sample on that axis (so that consecutive pieces of a stream, or time shards, compose).  With
+ * y_p = binauralDecode with page p, t = first_sample + n, f = t / hop, i = t - f hop, c = track[f],
+ * a = track[max(f - 1, 0)] and g = (i < fade) ? (i + 0.5) / fade : 1:
+ *     out[n] = (1 - g) y_a[n] + g y_c[n]       (a == c: exactly y_c[n])
+ * a linear equal-amplitude crossfade over the first `fade` samples of every frame (fade = 0: hard switch).
+ * compensate_delay as in emagls_binaural_decode (output row r holds sample r + len/2 - 1; the frame timing refers to the
+ * input sample n).  EMAGLS_ERR_INVALID, checked on the host before anything is launched: a null pointer, hop < 1, fade
+ * outside [0, hop], first_sample < 0, num_frames < (first_sample + num_samples - 1) / hop + 1, a used track entry
+ * outside [0, num_pages), an odd len with compensate_delay.
+ * _dev: in, wL, wR and out are device pointers; `track` is HOST memory in both variants (the launch geometry is derived
+ * from it on the host), the one exception to the _dev convention.  The call returns with the work enqueued on
+ * emagls_stream(h) after the upload of its tables.                                                                  */
+int emagls_binaural_decode_tracked(emagls_handle h, const double* in, long long num_samples, int num_ch,
+                                   const double* wL, const double* wR, int len, int num_pages,
+                                   const int32_t* track, long long num_frames, int hop, int fade,
+                                   long long first_sample, int compensate_delay, double* out);
+int emagls_binaural_decode_tracked_dev(emagls_handle h, const double* in, long long num_samples, int num_ch,
+                                       const double* wL, const double* wR, int len, int num_pages,
+                                       const int32_t* track, long long num_frames, int hop, int fade,
+                                       long long first_sample, int compensate_delay, double* out);
+
 /* ======================================================================================================
  * Callers either side of the hot path (SURVEY.md section 8-f): radial filters, SH/CH encoding and
  * rotation of the recording in front of the render, the remaining lib/ designers.
