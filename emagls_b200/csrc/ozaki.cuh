@@ -18,7 +18,6 @@
 // issuer (one elected thread), warps 2..17: epilogue (TMEM -> registers -> FP64, accumulators released,
 // then the functor).
 #pragma once
-#include <algorithm>
 #include <type_traits>
 #include <cuda.h>
 #include <cuda_runtime.h>
@@ -27,28 +26,19 @@
 namespace emagls {
 namespace oz {
 
-#ifndef EMAGLS_OZ_EPI_WARPS
-#define EMAGLS_OZ_EPI_WARPS 16
-#endif
-constexpr int TILE_M = 128, TILE_N = 64, TILE_K = 64, STAGES = 3, MAX_SLICES = 6;
+constexpr int TILE_M = 128, TILE_N = 64, TILE_K = 64, STAGES = 3, MAX_SLICES = 6, EPI_WARPS = 16;
 // Tile width / ring depth per use: 64 x 3 stages by default; 80 x 2 stages for the backward product
 // (N = 400 = 5 x 80: no padded columns, the 235 MB A operand streams through L2 5 instead of 7 times;
 // 6 x 80 = 480 TMEM columns).
 // EW: epilogue warps (a multiple of 4: EW / 4 per TMEM lane group, each taking every (EW / 4)-th 8-column chunk).
 // 16 warps on an 80-column tile leave ten chunks to four warps per lane group (3 + 3 + 2 + 2); 20 warps take two each.
-// SH: thread-block cluster of two CTAs that share one operand tile (TMA multicast: the CTA of rank 0 fetches the tile
-// once from L2 into the shared memory of both).  1 = the pair works on two neighbouring column tiles of the same row
-// tile (A shared), 2 = on two neighbouring row tiles of the same column tile (B shared).  The operand ring runs at the
-// L2 -> SMEM limit of the part (12.8 TB/s, section 5 of DESIGN.md), so the shared tile is traffic taken off that path.
-template <int NT_, int ST_, int EW_ = EMAGLS_OZ_EPI_WARPS, int SH_ = 0> struct TileCfg {
-  static constexpr int NT = NT_, ST = ST_, EW = EW_, THREADS = 64 + 32 * EW_, SHARE = SH_;
+template <int NT_, int ST_, int EW_ = EPI_WARPS> struct TileCfg {
+  static constexpr int NT = NT_, ST = ST_, EW = EW_, THREADS = 64 + 32 * EW_;
   static_assert(EW_ % 4 == 0 && EW_ >= 4 && 64 + 32 * EW_ <= 1024, "epilogue warps: whole lane groups");
-  static_assert(SH_ >= 0 && SH_ <= 2, "share: none, A, B");
 };
 using TileDefault = TileCfg<TILE_N, STAGES>;
 using TileWide = TileCfg<80, 2>;
 constexpr int A_SLICE_BYTES = TILE_M * TILE_K;   // 8 KB
-constexpr int EPI_WARPS = EMAGLS_OZ_EPI_WARPS;  // default of TileCfg::EW
 
 // ------------------------------------------------------------------------------------- PTX wrappers
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -62,23 +52,8 @@ __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
-// EMAGLS_OZ_WAIT_HINT (ns) > 0: try_wait carries a suspend-time hint, so a waiting thread sleeps in hardware until the
-// phase completes (or the hint expires) instead of polling: the TMA and MMA warps share their schedulers with epilogue
-// warps, and every polling iteration (try_wait + clock + compare + branch) is an issue slot those warps do not get
-#ifndef EMAGLS_OZ_WAIT_HINT
-#define EMAGLS_OZ_WAIT_HINT 0
-#endif
 __device__ __forceinline__ bool mbar_try(uint64_t* bar, uint32_t parity) {
   uint32_t ok;
-#if EMAGLS_OZ_WAIT_HINT > 0
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity), "r"((uint32_t)EMAGLS_OZ_WAIT_HINT)
-      : "memory");
-#else
   asm volatile(
       "{\n\t.reg .pred p;\n\t"
       "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
@@ -86,18 +61,13 @@ __device__ __forceinline__ bool mbar_try(uint64_t* bar, uint32_t parity) {
       : "=r"(ok)
       : "r"(smem_u32(bar)), "r"(parity)
       : "memory");
-#endif
   return ok != 0;
 }
 // bounded wait: a protocol error becomes a trap (launch failure) instead of a hung GPU
-#ifndef EMAGLS_OZ_SPIN_SLEEP
-#define EMAGLS_OZ_SPIN_SLEEP 0
-#endif
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   if (mbar_try(bar, parity)) return;
   const long long t0 = clock64();
   while (!mbar_try(bar, parity)) {
-    if (EMAGLS_OZ_SPIN_SLEEP > 0) __nanosleep(EMAGLS_OZ_SPIN_SLEEP);   // leave the issue slots to the working warps
     if (clock64() - t0 > 4000000000LL) __trap();
   }
 }
@@ -111,34 +81,6 @@ __device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* tm, ui
       ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(tm)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
       : "memory");
 }
-// the same tile delivered to the same shared-memory offset (and signalled on the same barrier offset) of every CTA in mask
-__device__ __forceinline__ void tma_load_3d_mc(void* dst, const CUtensorMap* tm, uint64_t* bar, int c0, int c1, int c2,
-                                               uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4, %5}], [%2], %6;"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(tm)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "h"(mask)
-      : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_rank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {   // every thread of every CTA of the cluster
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// shared-memory tile -> global tensor (bulk async group of the issuing thread)
-__device__ __forceinline__ void tma_store_3d(const CUtensorMap* tm, const void* src, int c0, int c1, int c2) {
-  asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
-               ::"l"(reinterpret_cast<uint64_t>(tm)), "r"(smem_u32(src)), "r"(c0), "r"(c1), "r"(c2)
-               : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-// generic-proxy writes to shared memory become visible to the async proxy (TMA)
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* tm) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(tm)) : "memory");
 }
@@ -163,11 +105,6 @@ __device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t adesc, uint64_
 // arrive on an mbarrier once every previously issued tcgen05.mma of this thread has completed
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-// ... on the barrier at the same offset in every CTA of mask
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(smem_u32(bar)), "h"(mask) : "memory");
 }
 // 32 lanes x 8 consecutive 32-bit columns: thread i of the warp receives lane (base lane + i)
 __device__ __forceinline__ void tmem_ld8(uint32_t taddr, int32_t (&v)[8]) {
@@ -322,26 +259,6 @@ __device__ __forceinline__ void tile_origin(const GemmArgs& g, int tile, int m_t
   else { m0 = (tile % m_tiles) * TILE_M; n0 = (tile / m_tiles) * g.tile_n; }
 }
 
-// Work item of a cluster pair (share != 0): item -> the tile of the CTA of this rank; false if the pair's second
-// tile lies past the edge (odd tile count: that CTA only keeps the barrier protocol going)
-__device__ __forceinline__ bool pair_tile_origin(const GemmArgs& g, int share, int item, int rank, int m_tiles, int n_tiles,
-                                                 int& m0, int& n0) {
-  int mi, ni;
-  if (share == 1) {            // two column tiles of one row tile
-    const int n_pairs = (n_tiles + 1) >> 1;
-    int np;
-    if (g.n_fastest) { np = item % n_pairs; mi = item / n_pairs; } else { mi = item % m_tiles; np = item / m_tiles; }
-    ni = 2 * np + rank;
-  } else {                     // two row tiles of one column tile
-    const int m_pairs = (m_tiles + 1) >> 1;
-    int mp;
-    if (g.n_fastest) { ni = item % n_tiles; mp = item / n_tiles; } else { mp = item % m_pairs; ni = item / m_pairs; }
-    mi = 2 * mp + rank;
-  }
-  m0 = mi * TILE_M; n0 = ni * g.tile_n;
-  return mi < m_tiles && ni < n_tiles;
-}
-
 __device__ __forceinline__ bool elect_one() {
   uint32_t pred;
   asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
@@ -352,35 +269,19 @@ __device__ __forceinline__ bool elect_one() {
 // (already scaled, FP64).  Called only for m < M; columns >= N hold zeros and must be skipped.  A functor that
 // declares `static constexpr bool all_lanes = true` is entered by every lane of the warp (also m >= M) and
 // guards its own stores, so that it may use warp shuffles.
-// A functor that declares `static constexpr bool staged = true` provides stage() / flush(): the four warps of a
-// TMEM lane group (32 rows x NT columns of the tile) write their results into a shared-memory tile, meet at a
-// named barrier and store the tile with row-contiguous 8-byte words (STG_ROW bytes per staged row).
-constexpr int STG_ROW = 72;
-template <class E, class = void> struct epi_staged { static constexpr bool value = false; };
-template <class E> struct epi_staged<E, decltype((void)E::staged)> { static constexpr bool value = E::staged; };
-__device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
-  asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
-}
 // A functor that declares `static constexpr bool raw = true` works on the unscaled integers (combine_diagonals):
 //   begin_tile(m, n, M, N) -> TileState   loads that do not depend on the accumulators, issued before the wait
 //   apply(state, m, n0, v[8], M, N)       called for m < M
 // (the forward product only needs the direction of y, so the operand scales cancel).
 template <class E, class = void> struct epi_raw { static constexpr bool value = false; };
 template <class E> struct epi_raw<E, decltype((void)E::raw)> { static constexpr bool value = E::raw; };
-// A raw functor that declares `static constexpr int tma_stage_bytes` (= T * NT * 128) writes its int8 results into a
-// shared-memory tile [T][NT columns][128 rows] with apply_staged(); the epilogue warps meet at a named barrier and one
-// thread stores the tile through the third tensor map (cp.async.bulk.tensor, clipped at the tensor's extent -- in
-// 4-byte granules along the inner dimension (measured: with an inner extent of 2702 bytes the columns 2702 and 2703
-// are written), so apply_staged() is also entered for rows m >= M and must stage zeros there).
-template <class E, class = void> struct epi_tma_stage { static constexpr int value = 0; };
-template <class E> struct epi_tma_stage<E, decltype((void)E::tma_stage_bytes)> { static constexpr int value = E::tma_stage_bytes; };
 template <class E, class = void> struct epi_i64 { static constexpr bool value = false; };
 template <class E> struct epi_i64<E, decltype((void)E::int64_values)> { static constexpr bool value = E::int64_values; };
 template <class E, class = void> struct epi_all_lanes { static constexpr bool value = false; };
 template <class E> struct epi_all_lanes<E, decltype((void)E::all_lanes)> { static constexpr bool value = E::all_lanes; };
 
-// Balanced base-256 digits of eight values at once, packed per digit plane: word[s] holds digit s of values
-// 0..7 in its bytes (little endian), ready for one 8-byte store per plane.  Same arithmetic as slice_digits.
+// Bytes 0..2 of four words, one word per byte position: r0 = [a0 b0 c0 d0], r1 = [a1 b1 c1 d1], r2 = [a2 b2 c2 d2]
+// (the digit words of four values -> one word per digit plane).
 __device__ __forceinline__ void transpose4x3(uint32_t a, uint32_t b, uint32_t c, uint32_t d, uint32_t& r0, uint32_t& r1,
                                              uint32_t& r2) {
   const uint32_t ab_lo = __byte_perm(a, b, 0x5140), cd_lo = __byte_perm(c, d, 0x5140);   // [a0 b0 a1 b1]
@@ -388,35 +289,6 @@ __device__ __forceinline__ void transpose4x3(uint32_t a, uint32_t b, uint32_t c,
   r0 = __byte_perm(ab_lo, cd_lo, 0x5410);   // [a0 b0 c0 d0]
   r1 = __byte_perm(ab_lo, cd_lo, 0x7632);   // [a1 b1 c1 d1]
   r2 = __byte_perm(ab_hi, cd_hi, 0x5410);   // [a2 b2 c2 d2]
-}
-template <int T>
-__device__ __forceinline__ void slice_pack8(const double (&a)[8], uint2 (&word)[MAX_SLICES]) {
-  static_assert(T >= 4 && T <= 6, "hi limb: 1..3 digits, lo limb: 3 digits");
-  constexpr int nh = T - 3;
-  constexpr int bias_hi = (nh == 3) ? 0x808080 : (nh == 2 ? 0x8080 : 0x80);
-  uint32_t zl[8], zh[8];
-#pragma unroll
-  for (int q = 0; q < 8; ++q) {
-    const double ah = a[q] * (double)(1 << (8 * (nh - 1)));
-    int hi = __double2int_rn(ah);
-    const int lo = __double2int_rn((ah - (double)hi) * 16777216.0);
-    const int yl = lo + 0x808080;
-    hi += yl >> 24;
-    zl[q] = (uint32_t)(yl ^ 0x808080);          // bytes 0..2 = digits T-1, T-2, T-3
-    zh[q] = (uint32_t)((hi + bias_hi) ^ bias_hi);   // byte j = digit nh-1-j
-  }
-  uint32_t l0[2], l1[2], l2[2], h0[2], h1[2], h2[2];
-#pragma unroll
-  for (int g4 = 0; g4 < 2; ++g4) {
-    transpose4x3(zl[4 * g4], zl[4 * g4 + 1], zl[4 * g4 + 2], zl[4 * g4 + 3], l0[g4], l1[g4], l2[g4]);
-    transpose4x3(zh[4 * g4], zh[4 * g4 + 1], zh[4 * g4 + 2], zh[4 * g4 + 3], h0[g4], h1[g4], h2[g4]);
-  }
-  word[T - 1] = make_uint2(l0[0], l0[1]);
-  word[T - 2] = make_uint2(l1[0], l1[1]);
-  word[T - 3] = make_uint2(l2[0], l2[1]);
-  word[nh - 1] = make_uint2(h0[0], h0[1]);
-  if (nh >= 2) word[nh - 2] = make_uint2(h1[0], h1[1]);
-  if (nh >= 3) word[nh - 3] = make_uint2(h2[0], h2[1]);
 }
 struct EpiStoreF64 {
   double* C; long long ldc;
@@ -433,30 +305,18 @@ struct EpiStoreF64 {
 
 template <int T, class Epi, class Cfg = TileDefault>
 __global__ void __launch_bounds__(Cfg::THREADS, 1)
-ozaki_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-                  const __grid_constant__ CUtensorMap tmC, GemmArgs g, Epi epi) {
+ozaki_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, GemmArgs g, Epi epi) {
   extern __shared__ uint8_t oz_smem_raw[];
   // 1024-byte aligned carve-up: [stage][A slices | B slices]
   uint8_t* base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(oz_smem_raw) + 1023) & ~(uintptr_t)1023);
   constexpr int NT = Cfg::NT, ST = Cfg::ST, EPI_WARPS = Cfg::EW, B_SLICE_BYTES = NT * TILE_K;
   constexpr int stage_bytes = T * (A_SLICE_BYTES + B_SLICE_BYTES);
-  uint8_t* epi_stage_area = base + (size_t)ST * stage_bytes;   // only for staged functors (see launch: extra smem)
   __shared__ __align__(8) uint64_t full_bar[ST], empty_bar[ST], tmem_full_bar, tmem_empty_bar;
   __shared__ uint32_t tmem_base_s;
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int m_tiles = (g.M + TILE_M - 1) / TILE_M, n_tiles = (g.N + NT - 1) / NT;
-  // work items: tiles, or (share != 0) pairs of tiles taken by the two CTAs of a cluster in lockstep
-  constexpr int SHARE = Cfg::SHARE;
-  constexpr uint16_t PAIR_MASK = 3;
-  const int rank = SHARE ? (int)cluster_rank() : 0;
-  const int num_tiles = SHARE == 1 ? m_tiles * ((n_tiles + 1) >> 1) : (SHARE == 2 ? ((m_tiles + 1) >> 1) * n_tiles : m_tiles * n_tiles);
-  const int item0 = SHARE ? (int)(blockIdx.x >> 1) : (int)blockIdx.x, item_step = SHARE ? (int)(gridDim.x >> 1) : (int)gridDim.x;
-  auto origin = [&](int item, int& m0, int& n0) -> bool {
-    if (SHARE) return pair_tile_origin(g, SHARE, item, rank, m_tiles, n_tiles, m0, n0);
-    tile_origin(g, item, m_tiles, n_tiles, m0, n0);
-    return true;
-  };
+  const int num_tiles = m_tiles * n_tiles, tile0 = (int)blockIdx.x, tile_step = (int)gridDim.x;
   const int ksteps_total = g.Kpad / 32;
   const int num_kt = (g.Kpad + TILE_K - 1) / TILE_K;
   constexpr uint32_t tmem_cols = (T * NT <= 256) ? 256u : 512u;
@@ -464,8 +324,7 @@ ozaki_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmA);
     tma_prefetch_desc(&tmB);
-    if (epi_tma_stage<Epi>::value) tma_prefetch_desc(&tmC);
-    for (int s = 0; s < ST; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], SHARE ? 2 : 1); }   // pair: both MMA warps release a stage
+    for (int s = 0; s < ST; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
     mbar_init(&tmem_full_bar, 1);
     mbar_init(&tmem_empty_bar, EPI_WARPS);   // one arrival per epilogue warp
     fence_barrier_init();
@@ -473,7 +332,6 @@ ozaki_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
   if (warp == 1) tmem_alloc(&tmem_base_s, tmem_cols);
   tc_fence_before();
   __syncthreads();
-  if (SHARE) cluster_sync_all();   // the peer's barriers exist before anything is multicast to them
   tc_fence_after();
   const uint32_t tmem_base = tmem_base_s;
 
@@ -481,31 +339,16 @@ ozaki_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     // ================================================================= TMA producer
     if (lane == 0) {
       int stage = 0; uint32_t phase = 0;
-      for (int tile = item0; tile < num_tiles; tile += item_step) {
+      for (int tile = tile0; tile < num_tiles; tile += tile_step) {
         int m0, n0;
-        const bool valid = origin(tile, m0, n0);
+        tile_origin(g, tile, m_tiles, n_tiles, m0, n0);
         for (int kt = 0; kt < num_kt; ++kt) {
           mbar_wait(&empty_bar[stage], phase ^ 1);
           uint8_t* sa = base + (size_t)stage * stage_bytes;
           uint8_t* sb = sa + (size_t)T * A_SLICE_BYTES;
-          if (SHARE == 0) {
-            mbar_expect_tx(&full_bar[stage], (uint32_t)stage_bytes);
-            tma_load_3d(sa, &tmA, &full_bar[stage], kt * TILE_K, m0, 0);
-            tma_load_3d(sb, &tmB, &full_bar[stage], kt * TILE_K, n0, 0);
-          } else {
-            // the shared tile arrives from the CTA of rank 0 (multicast), the other one from this CTA; a CTA without
-            // a tile of its own only receives the shared one
-            constexpr uint32_t a_bytes = (uint32_t)(T * A_SLICE_BYTES), b_bytes = (uint32_t)(T * B_SLICE_BYTES);
-            const uint32_t shared_bytes = SHARE == 1 ? a_bytes : b_bytes, own_bytes = SHARE == 1 ? b_bytes : a_bytes;
-            mbar_expect_tx(&full_bar[stage], shared_bytes + (valid ? own_bytes : 0u));
-            if (SHARE == 1) {
-              if (rank == 0) tma_load_3d_mc(sa, &tmA, &full_bar[stage], kt * TILE_K, m0, 0, PAIR_MASK);
-              if (valid) tma_load_3d(sb, &tmB, &full_bar[stage], kt * TILE_K, n0, 0);
-            } else {
-              if (valid) tma_load_3d(sa, &tmA, &full_bar[stage], kt * TILE_K, m0, 0);
-              if (rank == 0) tma_load_3d_mc(sb, &tmB, &full_bar[stage], kt * TILE_K, n0, 0, PAIR_MASK);
-            }
-          }
+          mbar_expect_tx(&full_bar[stage], (uint32_t)stage_bytes);
+          tma_load_3d(sa, &tmA, &full_bar[stage], kt * TILE_K, m0, 0);
+          tma_load_3d(sb, &tmB, &full_bar[stage], kt * TILE_K, n0, 0);
           if (++stage == ST) { stage = 0; phase ^= 1; }
         }
       }
@@ -518,18 +361,9 @@ ozaki_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     // 128 x 64 x 32 MMA occupies the tensor pipe.
     int stage = 0; uint32_t phase = 0, acc_phase = 0;
     const bool leader = elect_one();
-    for (int tile = item0; tile < num_tiles; tile += item_step) {
+    for (int tile = tile0; tile < num_tiles; tile += tile_step) {
       int m0, n0;
-      const bool valid = origin(tile, m0, n0);
-      if (!valid) {   // no tile of its own: consume the stages so that the peer's ring keeps moving
-        for (int kt = 0; kt < num_kt; ++kt) {
-          mbar_wait(&full_bar[stage], phase);
-          if (leader) umma_commit_mc(&empty_bar[stage], PAIR_MASK);
-          __syncwarp();
-          if (++stage == ST) { stage = 0; phase ^= 1; }
-        }
-        continue;
-      }
+      tile_origin(g, tile, m_tiles, n_tiles, m0, n0);
       const int n_mma = min(NT, ((g.N - n0) + 15) & ~15);
       const uint32_t idesc = instr_desc_i8(TILE_M, n_mma);
       mbar_wait(&tmem_empty_bar, acc_phase ^ 1);   // epilogue has drained the accumulators
@@ -559,8 +393,7 @@ ozaki_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
               }
             }
           }
-          if (SHARE) umma_commit_mc(&empty_bar[stage], PAIR_MASK);   // both producers write into this CTA's slot
-          else umma_commit(&empty_bar[stage]);       // smem slot reusable once these MMAs retire
+          umma_commit(&empty_bar[stage]);       // smem slot reusable once these MMAs retire
           if (kt == num_kt - 1) umma_commit(&tmem_full_bar);   // accumulators complete
         }
         __syncwarp();
@@ -575,9 +408,9 @@ ozaki_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     constexpr int chunk_step = 8 * (EPI_WARPS / 4);
     constexpr int CH_PER_WARP = (NT + chunk_step - 1) / chunk_step;
     uint32_t acc_phase = 0;
-    for (int tile = item0; tile < num_tiles; tile += item_step) {
+    for (int tile = tile0; tile < num_tiles; tile += tile_step) {
       int m0, n0;
-      if (!origin(tile, m0, n0)) continue;
+      tile_origin(g, tile, m_tiles, n_tiles, m0, n0);
       const int n_mma = min(NT, ((g.N - n0) + 15) & ~15);
       const int m = m0 + lg * 32 + lane;
       const int n_lim = (g.dbg & 1) ? 0 : n_mma;
@@ -613,26 +446,10 @@ ozaki_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
         tc_fence_after();
         drain();
         if (g.dbg & 4) { acc_phase ^= 1; continue; }
-        if constexpr (epi_tma_stage<Epi>::value != 0) {
-          static_assert(epi_tma_stage<Epi>::value == T * NT * TILE_M, "staging tile: [T][NT][128] bytes");
-          const bool issuer = (warp == 2 && lane == 0);
-          if (issuer) bulk_wait_read0();                  // the previous tile's store has read the staging tile
-          named_bar_sync(1, 32 * EPI_WARPS);
-          uint8_t* stg = epi_stage_area + lg * 32 + lane;
 #pragma unroll
-          for (int ci = 0; ci < CH_PER_WARP; ++ci) {
-            const int c0 = chunk0 + ci * chunk_step;
-            if (c0 < n_lim) epi.apply_staged(ts, stg + c0 * TILE_M, m, n0 + c0, v[ci], g.M, g.N);   // m >= M: zeros
-          }
-          fence_proxy_async();
-          named_bar_sync(1, 32 * EPI_WARPS);
-          if (issuer && n_lim > 0) { tma_store_3d(&tmC, epi_stage_area, m0, n0, 0); bulk_commit(); }
-        } else {
-#pragma unroll
-          for (int ci = 0; ci < CH_PER_WARP; ++ci) {
-            const int c0 = chunk0 + ci * chunk_step;
-            if (c0 < n_lim && (epi_all_lanes<Epi>::value || m < g.M)) epi.apply(ts, m, n0 + c0, v[ci], g.M, g.N);   // all_lanes: warp-uniform entry
-          }
+        for (int ci = 0; ci < CH_PER_WARP; ++ci) {
+          const int c0 = chunk0 + ci * chunk_step;
+          if (c0 < n_lim && (epi_all_lanes<Epi>::value || m < g.M)) epi.apply(ts, m, n0 + c0, v[ci], g.M, g.N);   // all_lanes: warp-uniform entry
         }
       } else {
         mbar_wait(&tmem_full_bar, acc_phase);
@@ -650,37 +467,22 @@ ozaki_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
             }
           }
         }
-        if constexpr (epi_staged<Epi>::value) {
-          static_assert(EPI_WARPS == 16 && NT == 64, "staged epilogue: four warps per lane group, 64-column tiles");
-          uint8_t* stg = epi_stage_area + (size_t)lg * (T * 32 * STG_ROW);
 #pragma unroll
-          for (int ci = 0; ci < CH_PER_WARP; ++ci) {
-            const int c0 = chunk0 + ci * chunk_step;
-            if (c0 < n_lim) epi.stage(stg, lane, c0, m, n0 + c0, v[ci], g.M, g.N);
-          }
-          named_bar_sync(1 + lg, 128);
-          if (n_lim > 0) epi.flush(stg, ((warp - 2) >> 2) * 32 + lane, m0 + lg * 32, n0, n_lim, g.M);
-          named_bar_sync(1 + lg, 128);      // the tile is free again for the next one
-        } else {
-#pragma unroll
-          for (int ci = 0; ci < CH_PER_WARP; ++ci) {
-            const int c0 = chunk0 + ci * chunk_step;
-            if constexpr (epi_all_lanes<Epi>::value) {
-              // functors that exchange data between lanes are entered by the whole warp (c0 and n_lim are warp-uniform)
-              if (c0 < n_lim) epi(m, n0 + c0, v[ci], g.M, g.N);
-            } else {
-              if (c0 < n_lim && m < g.M) epi(m, n0 + c0, v[ci], g.M, g.N);
-            }
+        for (int ci = 0; ci < CH_PER_WARP; ++ci) {
+          const int c0 = chunk0 + ci * chunk_step;
+          if constexpr (epi_all_lanes<Epi>::value) {
+            // functors that exchange data between lanes are entered by the whole warp (c0 and n_lim are warp-uniform)
+            if (c0 < n_lim) epi(m, n0 + c0, v[ci], g.M, g.N);
+          } else {
+            if (c0 < n_lim && m < g.M) epi(m, n0 + c0, v[ci], g.M, g.N);
           }
         }
       }
       acc_phase ^= 1;
     }
-    if (epi_tma_stage<Epi>::value != 0 && warp == 2 && lane == 0) bulk_wait0();
   }
   tc_fence_before();
   __syncthreads();
-  if (SHARE) cluster_sync_all();   // the peer may still arrive on this CTA's barriers until it is done, too
   if (warp == 1) {
     tc_fence_after();
     tmem_dealloc(tmem_base, tmem_cols);
@@ -720,20 +522,6 @@ inline bool make_operand_map(CUtensorMap* tm, const int8_t* ptr, int rows, int K
   return r == CUDA_SUCCESS;
 }
 
-// int8 output [T][rows][Kpad] written by TMA from a staging tile [T][box_rows][128]: the tensor's inner extent is the
-// number of valid columns, so the padding columns (and the rows past the end) are never written.
-inline bool make_output_map(CUtensorMap* tm, int8_t* ptr, int rows, int cols_valid, int Kpad, int T, int box_rows) {
-  EncodeTiledFn fn = encode_tiled_fn();
-  if (!fn) return false;
-  cuuint64_t dims[3] = {(cuuint64_t)cols_valid, (cuuint64_t)rows, (cuuint64_t)T};
-  cuuint64_t strides[2] = {(cuuint64_t)Kpad, (cuuint64_t)Kpad * (cuuint64_t)rows};
-  cuuint32_t box[3] = {(cuuint32_t)TILE_M, (cuuint32_t)box_rows, (cuuint32_t)T};
-  cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = fn(tm, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, ptr, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                  CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  return r == CUDA_SUCCESS;
-}
-
 // int32 accumulators: a diagonal holds at most T pairs of products bounded by 2^14 each
 inline bool contraction_fits(int Kpad, int T) { return (long long)T * 16384LL * Kpad < (1LL << 31); }
 
@@ -742,32 +530,15 @@ inline size_t gemm_smem_bytes(int T) { return (size_t)Cfg::ST * T * (A_SLICE_BYT
 
 template <int T, class Epi, class Cfg = TileDefault>
 cudaError_t launch_ozaki_gemm_t(cudaStream_t st, const CUtensorMap& tmA, const CUtensorMap& tmB, GemmArgs g,
-                                Epi epi, int num_sms, const CUtensorMap* tmC = nullptr) {
+                                Epi epi, int num_sms) {
   static_assert(T * Cfg::NT <= 512 && Cfg::NT % 16 == 0, "TMEM holds 512 columns; UMMA N is a multiple of 16");
-  const size_t smem = gemm_smem_bytes<Cfg>(T) + (epi_staged<Epi>::value ? (size_t)4 * T * 32 * STG_ROW : 0) +
-                      (size_t)epi_tma_stage<Epi>::value;
-  if (epi_tma_stage<Epi>::value != 0 && !tmC) return cudaErrorInvalidValue;
+  const size_t smem = gemm_smem_bytes<Cfg>(T);
   cudaError_t e = cudaFuncSetAttribute(ozaki_gemm_kernel<T, Epi, Cfg>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   g.tile_n = Cfg::NT;
-  const int m_tiles = (g.M + TILE_M - 1) / TILE_M, n_tiles = (g.N + Cfg::NT - 1) / Cfg::NT;
-  if (Cfg::SHARE == 0) {
-    const int tiles = m_tiles * n_tiles;
-    ozaki_gemm_kernel<T, Epi, Cfg><<<tiles < num_sms ? tiles : num_sms, Cfg::THREADS, smem, st>>>(tmA, tmB, tmC ? *tmC : tmA, g, epi);
-    return cudaGetLastError();
-  }
-  static_assert(Cfg::SHARE == 0 || (epi_tma_stage<Epi>::value == 0 && !epi_staged<Epi>::value), "cluster pairs: plain functors");
-  const int pairs = Cfg::SHARE == 1 ? m_tiles * ((n_tiles + 1) / 2) : ((m_tiles + 1) / 2) * n_tiles;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)(2 * std::min(pairs, num_sms / 2)));
-  cfg.blockDim = dim3((unsigned)Cfg::THREADS);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr; cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, ozaki_gemm_kernel<T, Epi, Cfg>, tmA, tmB, tmC ? *tmC : tmA, g, epi);
+  const int tiles = ((g.M + TILE_M - 1) / TILE_M) * ((g.N + Cfg::NT - 1) / Cfg::NT);
+  ozaki_gemm_kernel<T, Epi, Cfg><<<tiles < num_sms ? tiles : num_sms, Cfg::THREADS, smem, st>>>(tmA, tmB, g, epi);
+  return cudaGetLastError();
 }
 
 // C = A * B^T from sliced operands Aq [T][M][Kpad], Bq [T][N][Kpad]

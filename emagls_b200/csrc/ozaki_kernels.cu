@@ -13,53 +13,12 @@ namespace emagls {
 
 namespace {
 
-template <int T>
-struct EpiPhaseSlice {
-  int8_t* Tq; long long slice_stride; int Kpad;   // [T][rows][Kpad], element (n, m) at n * Kpad + m
-  double* sT;                                     // [rows] scale of row n (written by the m == 0 lanes)
-  const double* absH; long long abs_set_stride, abs_ear_stride;   // this bin: [set][ear][dir]
-  const double* up; const double* sc; int scale_stride;           // 2^(6-e), 2^(e-6) at [(set*2+ear)*scale_stride]
-  int orient_per_set; int nyquist;
-  __device__ __forceinline__ void operator()(int m, int n0, const double (&v)[8], int M, int N) const {
-    // columns n0..n0+7 are the (re, im) pairs of four consecutive (problem, ear) indices j = n / 2;
-    // the HRTF set of a problem is found with one division per call and then tracked incrementally
-    int prob = n0 >> 2;
-    int set = prob / orient_per_set;
-    int left = (set + 1) * orient_per_set - prob;     // problems left in this set, >= 1
-#pragma unroll
-    for (int q = 0; q < 8; q += 2) {
-      const int n = n0 + q;
-      if (n >= N) break;
-      const int ear = (n >> 1) & 1;
-      const double mag = absH[(long long)set * abs_set_stride + (long long)ear * abs_ear_stride + m];
-      const double re = v[q], im = v[q + 1];
-      const double a2 = fma(re, re, im * im);
-      double tr, ti;
-      if (a2 > 1e-290 && a2 < 1e290) {
-        const double inv = mag * rsqrt(a2);
-        tr = re * inv; ti = im * inv;
-      } else if (a2 > 0.0) {
-        const double inv = mag / sqrt(a2);
-        tr = re * inv; ti = im * inv;
-      } else { tr = mag; ti = 0.0; }          // angle(0) = 0
-      if (nyquist) ti = 0.0;
-      const int si = (set * 2 + ear) * scale_stride;
-      const double u = up[si];
-      int8_t* p = Tq + (long long)n * Kpad + m;   // |tr u|, |ti u| <= 64 (u = 2^(6-e), 2^e > max_d |H_k|)
-      oz::slice_digits<T>(tr * u, [&](int s, int q_) { p[(long long)s * slice_stride] = (int8_t)q_; });
-      oz::slice_digits<T>(ti * u, [&](int s, int q_) { p[(long long)s * slice_stride + Kpad] = (int8_t)q_; });
-      if (m == 0) { const double s_ = sc[si]; sT[n] = s_; sT[n + 1] = s_; }
-      if (ear == 1 && --left == 0) { ++set; left = orient_per_set; }   // next pair belongs to the next problem
-    }
-  }
-};
-
-// The same epilogue on the unscaled integer results (oz::epi_raw): y / |y| does not depend on a common scale, so
-// the row scale of Y_h and the weight of the digit planes are not applied (only the scales of the re and the im
-// row of c, which differ); |H_k|, its power-of-two scale and the 256^(T-4) of the digit split are one factor per
+// Epilogue of the forward product on the unscaled integer results (oz::epi_raw): y / |y| does not depend on a common
+// scale, so the row scale of Y_h and the weight of the digit planes are not applied (only the scales of the re and the
+// im row of c, which differ); |H_k|, its power-of-two scale and the 256^(T-4) of the digit split are one factor per
 // (set, ear, direction), fetched before the accumulators are waited for; the digits come out of the FP64 / integer
-// pipes (oz::slice_words) instead of F2I / I2F.  Bitwise the same digits as EpiPhaseSlice (every factor that moved
-// is a power of two).
+// pipes (oz::slice_words) instead of F2I / I2F.  Bitwise the same digits as oz::slice_digits of the scaled phase
+// continuation (every factor that moved is a power of two).
 template <int T>
 struct EpiPhaseSliceRaw {
   static constexpr bool raw = true;
@@ -83,11 +42,20 @@ struct EpiPhaseSliceRaw {
     load_set(ts, (min(n, N - 1) >> 2) / orient_per_set, m);   // a chunk past the last column is never applied
     return ts;
   }
+  // digit j of a column goes to plane T-1-j (j < 3: bytes of zl; j >= 3: bytes of zh)
+  __device__ __forceinline__ void put_digits(int8_t* p, uint32_t zl, uint32_t zh) const {
+    p[(T - 1) * slice_stride] = (int8_t)zl;
+    p[(T - 2) * slice_stride] = (int8_t)(zl >> 8);
+    p[(T - 3) * slice_stride] = (int8_t)(zl >> 16);
+    p[(T - 4) * slice_stride] = (int8_t)zh;
+    if (T >= 5) p[(T - 5) * slice_stride] = (int8_t)(zh >> 8);
+    if (T >= 6) p[(T - 6) * slice_stride] = (int8_t)(zh >> 16);
+  }
   // columns n0..n0+7 are the (re, im) pairs of four consecutive (problem, ear) indices j = n / 2 (n0 is a multiple
   // of 8, so the ear is (q >> 1) & 1); the HRTF set of a problem is found with one division per call and then
-  // tracked incrementally.  store(q, zl, zh) receives the digit words of column n0 + q.
-  template <class Store>
-  __device__ __forceinline__ void phase_slice(TileState& ts, int m, int n0, const double (&v)[8], int N, Store&& store) const {
+  // tracked incrementally.
+  __device__ __forceinline__ void apply(TileState& ts, int m, int n0, const double (&v)[8], int M, int N) const {
+    int8_t* p = Tq + (long long)n0 * Kpad + m;
     const int prob = n0 >> 2;
     int set = prob / orient_per_set;
     int left = (set + 1) * orient_per_set - prob;     // problems left in this set, >= 1
@@ -117,24 +85,11 @@ struct EpiPhaseSliceRaw {
       if (nyquist) ti = 0.0;
       uint32_t zl, zh;                                // |tr|, |ti| <= 64 * 256^(T-4)
       oz::slice_words<T>(tr, zl, zh);
-      store(q, zl, zh);
+      put_digits(p + (long long)q * Kpad, zl, zh);
       oz::slice_words<T>(ti, zl, zh);
-      store(q + 1, zl, zh);
+      put_digits(p + (long long)(q + 1) * Kpad, zl, zh);
       if (e == 1 && --left == 0) { ++set; left = orient_per_set; }   // next pair belongs to the next problem
     }
-  }
-  template <class P>
-  static __device__ __forceinline__ void put_digits(P* p, long long plane, uint32_t zl, uint32_t zh) {
-    p[(T - 1) * plane] = (P)zl;
-    p[(T - 2) * plane] = (P)(zl >> 8);
-    p[(T - 3) * plane] = (P)(zl >> 16);
-    p[(T - 4) * plane] = (P)zh;
-    if (T >= 5) p[(T - 5) * plane] = (P)(zh >> 8);
-    if (T >= 6) p[(T - 6) * plane] = (P)(zh >> 16);
-  }
-  __device__ __forceinline__ void apply(TileState& ts, int m, int n0, const double (&v)[8], int M, int N) const {
-    int8_t* p = Tq + (long long)n0 * Kpad + m;
-    phase_slice(ts, m, n0, v, N, [&](int q, uint32_t zl, uint32_t zh) { put_digits(p + (long long)q * Kpad, slice_stride, zl, zh); });
   }
 };
 // The same epilogue without FP64 instructions in the functor (phase_fixed.cuh): FP64 work does not overlap with the
@@ -143,14 +98,14 @@ struct EpiPhaseSliceRaw {
 // count-leading-zeros and shifts, |y|^-1 comes from a 22-bit MUFU seed and one third-order correction in 64-bit
 // fixed point, and the digits are those of rn(t 2^24) formed in integer arithmetic.  Against EpiPhaseSliceRaw the last digit may differ by one unit
 // (|Z - exact| <= 0.6 instead of <= 0.53; tests/test_phase_fixed.py).
-// WORDS: the digit bytes of four columns are packed per plane, transposed across groups of four lanes (two shuffles
+// Stores: the digit bytes of four columns are packed per plane, transposed across groups of four lanes (two shuffles
 // and two byte permutes per word) and leave as 4-byte stores: lane l writes rows l & ~3 .. (l & ~3) + 3 of column
-// l & 3.  A quarter of the store instructions and of their address arithmetic; the whole warp enters apply() (lanes
-// past the last row contribute zero bytes, which land in the row padding), so N must be a multiple of 4.
-template <int T, bool WORDS = false>
+// l & 3: a quarter of the store instructions (and of their address arithmetic) of byte stores.  The whole warp enters
+// apply() (lanes past the last row contribute zero bytes, which land in the row padding), so N must be a multiple of 4.
+template <int T>
 struct EpiPhaseSliceFix {
   static constexpr bool raw = true;
-  static constexpr bool all_lanes = WORDS;
+  static constexpr bool all_lanes = true;
   static constexpr bool int64_values = true;      // the drain hands over exact 64-bit integers (no FP64 at all)
   int8_t* Tq; long long slice_stride; int Kpad;   // [T][rows][Kpad], element (n, m) at n * Kpad + m
   double* sT;                                     // [rows] scale of row n (written by the m == 0 lanes)
@@ -181,16 +136,6 @@ struct EpiPhaseSliceFix {
     load_set(ts, (min(n, N - 1) >> 2) / orient_per_set, m);   // a chunk past the last column is never applied
     return ts;
   }
-  // digit j of a column goes to plane T-1-j (j < 3: bytes of zl; j >= 3: bytes of zh): one 64-bit pointer per plane,
-  // formed once per chunk, plus a 32-bit column offset
-  static __device__ __forceinline__ void put_digits_at(int8_t* const (&pl)[T], uint32_t off, uint32_t zl, uint32_t zh) {
-    pl[T - 1][off] = (int8_t)zl;
-    pl[T - 2][off] = (int8_t)(zl >> 8);
-    pl[T - 3][off] = (int8_t)(zl >> 16);
-    pl[T - 4][off] = (int8_t)zh;
-    if (T >= 5) pl[T >= 5 ? T - 5 : 0][off] = (int8_t)(zh >> 8);
-    if (T >= 6) pl[T >= 6 ? T - 6 : 0][off] = (int8_t)(zh >> 16);
-  }
   // scale of the output rows n0 .. n0+7 (one writer per row: the m == 0 lane)
   __device__ __forceinline__ void put_scales(int n0, int N, int set, int left) const {
     for (int q = 0; q < 8 && n0 + q < N; q += 2) {
@@ -216,126 +161,31 @@ struct EpiPhaseSliceFix {
     int set = prob / orient_per_set;
     int left = (set + 1) * orient_per_set - prob;     // problems left in this set, >= 1
     if (m == 0) put_scales(n0, N, set, left);
-    if constexpr (!WORDS) {
-      int8_t* pl[T];
+    const int lane = threadIdx.x & 31, g = lane & 3;
+    const uint32_t selA = (lane & 2) ? 0x3276u : 0x5410u, selB = (lane & 1) ? 0x3715u : 0x6240u;
+    const uint32_t keep = m < M ? 0xFFFFFFFFu : 0u;
+    const bool writer = m - g < M;                  // the group's first row exists (then all four lie below Kpad)
+    const int mc = min(m, M - 1);
+    // this lane's word: column n0 + g (+ 4), rows m - g .. m - g + 3; the plane / column-group offsets are uniform
+    int8_t* const pw = Tq + ((long long)(n0 + g) * Kpad + (m - g));
+    const long long col4 = 4ll * Kpad;
 #pragma unroll
-      for (int s_ = 0; s_ < T; ++s_) pl[s_] = Tq + ((long long)s_ * slice_stride + (long long)n0 * Kpad + m);
-      const uint32_t col = (uint32_t)Kpad;
+    for (int h = 0; h < 2; ++h) {                   // four columns = both ears of one problem
+      if (n0 + 4 * h >= N) break;
+      if (set != ts.set) load_set_cold(ts, set, mc);   // warp-uniform: a tile rarely straddles two HRTF sets
+      uint32_t zl[4], zh[4];
+      pair_digits(ts, n0, 4 * h, v[4 * h], v[4 * h + 1], zl[0], zh[0], zl[1], zh[1]);
+      pair_digits(ts, n0, 4 * h + 2, v[4 * h + 2], v[4 * h + 3], zl[2], zh[2], zl[3], zh[3]);
+      if (--left == 0) { ++set; left = orient_per_set; }
+      uint32_t w[6];                                // w[j]: digit T-1-j of the four columns
+      oz::transpose4x3(zl[0], zl[1], zl[2], zl[3], w[0], w[1], w[2]);
+      oz::transpose4x3(zh[0], zh[1], zh[2], zh[3], w[3], w[4], w[5]);
 #pragma unroll
-      for (int q = 0; q < 8; q += 2) {
-        if (n0 + q >= N) break;
-        if (set != ts.set) load_set_cold(ts, set, m);   // warp-uniform: a tile rarely straddles two HRTF sets
-        uint32_t rl, rh, il, ih;
-        pair_digits(ts, n0, q, v[q], v[q + 1], rl, rh, il, ih);
-        put_digits_at(pl, (uint32_t)q * col, rl, rh);
-        put_digits_at(pl, (uint32_t)(q + 1) * col, il, ih);
-        if ((q & 2) && --left == 0) { ++set; left = orient_per_set; }   // next pair belongs to the next problem
-      }
-    } else {
-      const int lane = threadIdx.x & 31, g = lane & 3;
-      const uint32_t selA = (lane & 2) ? 0x3276u : 0x5410u, selB = (lane & 1) ? 0x3715u : 0x6240u;
-      const uint32_t keep = m < M ? 0xFFFFFFFFu : 0u;
-      const bool writer = m - g < M;                  // the group's first row exists (then all four lie below Kpad)
-      const int mc = min(m, M - 1);
-      // this lane's word: column n0 + g (+ 4), rows m - g .. m - g + 3; the plane / column-group offsets are uniform
-      int8_t* const pw = Tq + ((long long)(n0 + g) * Kpad + (m - g));
-      const long long col4 = 4ll * Kpad;
-#pragma unroll
-      for (int h = 0; h < 2; ++h) {                   // four columns = both ears of one problem
-        if (n0 + 4 * h >= N) break;
-        if (set != ts.set) load_set_cold(ts, set, mc);
-        uint32_t zl[4], zh[4];
-        pair_digits(ts, n0, 4 * h, v[4 * h], v[4 * h + 1], zl[0], zh[0], zl[1], zh[1]);
-        pair_digits(ts, n0, 4 * h + 2, v[4 * h + 2], v[4 * h + 3], zl[2], zh[2], zl[3], zh[3]);
-        if (--left == 0) { ++set; left = orient_per_set; }
-        uint32_t w[6];                                // w[j]: digit T-1-j of the four columns
-        oz::transpose4x3(zl[0], zl[1], zl[2], zl[3], w[0], w[1], w[2]);
-        oz::transpose4x3(zh[0], zh[1], zh[2], zh[3], w[3], w[4], w[5]);
-#pragma unroll
-        for (int j = 0; j < T; ++j) {
-          uint32_t x = w[j] & keep;
-          x = __byte_perm(x, __shfl_xor_sync(0xffffffffu, x, 2), selA);
-          x = __byte_perm(x, __shfl_xor_sync(0xffffffffu, x, 1), selB);
-          if (writer) *reinterpret_cast<uint32_t*>(pw + ((long long)(T - 1 - j) * slice_stride + h * col4)) = x;
-        }
-      }
-    }
-  }
-};
-// ... with the digits staged in shared memory and stored by TMA (oz::epi_tma_stage): the byte stores go to
-// compile-time offsets of one shared-memory address, and the tile leaves as 128-byte rows.
-template <int T>
-struct EpiPhaseSliceTma : EpiPhaseSliceRaw<T> {
-  static constexpr int tma_stage_bytes = T * oz::TILE_N * oz::TILE_M;
-  // stg: the staging byte of (this thread's row, first column of the chunk) in plane 0
-  __device__ __forceinline__ void apply_staged(typename EpiPhaseSliceRaw<T>::TileState& ts, uint8_t* stg, int m, int n0,
-                                               const double (&v)[8], int M, int N) const {
-    if (m >= M) {   // rows past the tensor's extent: the store may reach up to three of them (padding columns, zero)
-#pragma unroll
-      for (int q = 0; q < 8; ++q) EpiPhaseSliceRaw<T>::put_digits(stg + q * oz::TILE_M, (long long)(oz::TILE_N * oz::TILE_M), 0u, 0u);
-      return;
-    }
-    this->phase_slice(ts, m, n0, v, N, [&](int q, uint32_t zl, uint32_t zh) {
-      EpiPhaseSliceRaw<T>::put_digits(stg + q * oz::TILE_M, (long long)(oz::TILE_N * oz::TILE_M), zl, zh);
-    });
-  }
-};
-
-// Forward product with the operand roles swapped: rows m = (problem, ear, re/im) [4P], columns n = directions.
-// A thread owns eight consecutive directions of one row; the real and the imaginary row of a (problem, ear)
-// pair sit in neighbouring lanes and exchange their values by shuffle, every lane then forms t for its own
-// part and emits ONE 8-byte word per digit plane (six stores instead of 48 single bytes per 8 outputs).
-template <int T>
-struct EpiPhaseSliceRows {
-  static constexpr bool staged = true;            // stage() by every lane of the warp, then flush() by the lane group
-  int8_t* Tq; long long slice_stride; int Kpad;   // [T][rows][Kpad], element (m, n) at m * Kpad + n
-  double* sT;                                     // [rows] scale of row m (written by the n == 0 chunk)
-  const double* absH; long long abs_set_stride, abs_ear_stride;   // this bin: [set][ear][dir]
-  const double* up; const double* sc; int scale_stride;           // 2^(6-e), 2^(e-6) at [(set*2+ear)*scale_stride]
-  int orient_per_set; int nyquist;
-  // row `row` of the lane group's tile, columns c0 .. c0+7 (absolute: m, n0 .. n0+7)
-  __device__ __forceinline__ void stage(uint8_t* stg, int row, int c0, int m, int n0, const double (&v)[8], int M,
-                                        int N) const {
-    const bool valid = m < M;
-    const int mm = valid ? m : 0;
-    const int part = mm & 1, j = mm >> 1, ear = j & 1, prob = j >> 1;
-    const int set = prob / orient_per_set;
-    const double* mag = absH + (long long)set * abs_set_stride + (long long)ear * abs_ear_stride + n0;
-    const int si = (set * 2 + ear) * scale_stride;
-    const double u = up[si];
-    double a[8];
-#pragma unroll
-    for (int q = 0; q < 8; ++q) {
-      const double mine = v[q];
-      const double other = __shfl_xor_sync(0xffffffffu, mine, 1);
-      const double re = part ? other : mine, im = part ? mine : other;
-      const double a2 = fma(re, re, im * im);     // the same expression on both lanes (and as in EpiPhaseSlice)
-      double t;
-      const double mg = (n0 + q < N) ? mag[q] : 0.0;
-      if (a2 > 1e-290 && a2 < 1e290) t = mine * (mg * rsqrt(a2));
-      else if (a2 > 0.0) t = mine * (mg / sqrt(a2));
-      else t = part ? 0.0 : mg;                   // angle(0) = 0
-      if (nyquist && part) t = 0.0;
-      a[q] = t * u;                               // |t u| <= 64 (u = 2^(6-e), 2^e > max_d |H_k|)
-    }
-    if (!valid) return;
-    uint2 word[oz::MAX_SLICES];
-    oz::slice_pack8<T>(a, word);
-#pragma unroll
-    for (int s = 0; s < T; ++s) *reinterpret_cast<uint2*>(stg + (s * 32 + row) * oz::STG_ROW + c0) = word[s];
-    if (n0 == 0) sT[m] = sc[si];
-  }
-  // t = 0 .. 127 within the lane group; rows m_base .. m_base+31, columns n0 .. n0+n_lim-1 of the tile
-  __device__ __forceinline__ void flush(const uint8_t* stg, int t, int m_base, int n0, int n_lim, int M) const {
-#pragma unroll
-    for (int s = 0; s < T; ++s) {
-#pragma unroll
-      for (int it = 0; it < 2; ++it) {
-        const int idx = it * 128 + t, row = idx >> 3, piece = (idx & 7) * 8;
-        if (piece < n_lim && m_base + row < M) {
-          const uint2 w = *reinterpret_cast<const uint2*>(stg + (s * 32 + row) * oz::STG_ROW + piece);
-          *reinterpret_cast<uint2*>(Tq + (long long)s * slice_stride + (long long)(m_base + row) * Kpad + n0 + piece) = w;
-        }
+      for (int j = 0; j < T; ++j) {
+        uint32_t x = w[j] & keep;
+        x = __byte_perm(x, __shfl_xor_sync(0xffffffffu, x, 2), selA);
+        x = __byte_perm(x, __shfl_xor_sync(0xffffffffu, x, 1), selB);
+        if (writer) *reinterpret_cast<uint32_t*>(pw + ((long long)(T - 1 - j) * slice_stride + h * col4)) = x;
       }
     }
   }
@@ -387,95 +237,44 @@ cudaError_t launch_row_scale(cudaStream_t st, const double* x, long long rows, i
   return cudaGetLastError();
 }
 
-template <int T>
-static cudaError_t oz_fwd_rows_t(cudaStream_t st, const OzFwdArgs& a) {
-  CUtensorMap tmA, tmB;
-  if (!oz::make_operand_map(&tmA, a.Cv_q, a.rows, a.KpS, T, oz::TILE_M) ||
-      !oz::make_operand_map(&tmB, a.YhA_q, a.D, a.KpS, T, oz::TILE_N))
-    return cudaErrorInvalidValue;
-  // n fastest: consecutive tiles (neighbouring SMs) share the rows of the large operand (the Cv digits)
-  oz::GemmArgs g{a.rows, a.D, a.KpS, a.sCv, a.sYhA, 0, 1, oz::TILE_N};
-  EpiPhaseSliceRows<T> epi{a.Tt_q, (long long)a.rows * a.KpD, a.KpD, a.sT, a.absH, a.abs_set_stride, a.abs_ear_stride,
-                           a.up, a.sc, a.scale_stride, a.orient_per_set, a.nyquist};
-  return oz::launch_ozaki_gemm_t<T, EpiPhaseSliceRows<T>, oz::TileCfg<64, 2>>(st, tmA, tmB, g, epi, sm_count());
-}
-
 int oz_fwd_debug = 0;   // GemmArgs::dbg of the forward launches (tools/microbench/oz_fwd_bench.cu)
 
 template <int T, class Epi, class Cfg = oz::TileDefault>
 static cudaError_t oz_fwd_t(cudaStream_t st, const OzFwdArgs& a) {
-  CUtensorMap tmA, tmB, tmC;
+  CUtensorMap tmA, tmB;
   if (!oz::make_operand_map(&tmA, a.YhA_q, a.D, a.KpS, T, oz::TILE_M) ||
       !oz::make_operand_map(&tmB, a.Cv_q, a.rows, a.KpS, T, Cfg::NT))
     return cudaErrorInvalidValue;
-  const bool tma_out = oz::epi_tma_stage<Epi>::value != 0;
-  if (tma_out && !oz::make_output_map(&tmC, a.Tt_q, a.rows, a.D, a.KpD, T, oz::TILE_N)) return cudaErrorInvalidValue;
   oz::GemmArgs g{a.D, a.rows, a.KpS, a.sYhA, a.sCv, oz_fwd_debug, 0, Cfg::NT};   // m fastest: the 42 MB of Cv digits are the shared operand
   Epi epi{a.Tt_q, (long long)a.rows * a.KpD, a.KpD, a.sT, a.absH, a.abs_set_stride, a.abs_ear_stride,
-          a.up, a.sc, a.scale_stride, a.orient_per_set, a.nyquist};
-  if constexpr (oz::epi_raw<Epi>::value) epi.sB = a.sCv;
-  return oz::launch_ozaki_gemm_t<T, Epi, Cfg>(st, tmA, tmB, g, epi, sm_count(), tma_out ? &tmC : nullptr);
+          a.up, a.sc, a.scale_stride, a.orient_per_set, a.nyquist, a.sCv};
+  return oz::launch_ozaki_gemm_t<T, Epi, Cfg>(st, tmA, tmB, g, epi, sm_count());
 }
 
 cudaError_t launch_oz_fwd(cudaStream_t st, const OzFwdArgs& a) {
   if (!oz::contraction_fits(a.KpS, a.T)) return cudaErrorInvalidValue;
-  // EMAGLS_OZ_FWD_ROWS=1 (A/B switch): operand roles swapped, a thread owns eight directions of one (problem, ear,
-  // re/im) row, packs 8-byte digit words, and the lane group stores its 32 x 64 tile row-contiguously through a
-  // shared-memory stage.  (Without the stage the 8-byte words of 32 different rows cost four times the L2 sectors of
-  // the default orientation's byte stores: 250 ms against 225 ms per step, profiles/r02_v7.)
-  static const bool by_rows = getenv("EMAGLS_OZ_FWD_ROWS") != nullptr;
-  if (by_rows && (a.rows & 1) == 0) {
-    switch (a.T) {
-      case 4: return oz_fwd_rows_t<4>(st, a);
-      case 6: return oz_fwd_rows_t<6>(st, a);
-      default: return cudaErrorInvalidValue;
-    }
-  }
-  // Default for six digits: the FP64-free functor (EpiPhaseSliceFix: its integer work overlaps with the MMAs of the
-  // next tile, FP64 work does not; 0.34 against 0.425 ms per launch, profiles/r02_v40_fwd_fix.txt) on 128 x 80 tiles
-  // when that takes fewer rounds of tiles.  With four digits the MMAs of a tile are too short to hide the longer
-  // integer functor, so the FP64 functor on the raw accumulators stays (0.076 against 0.078 ms).
-  // A/B switches: EMAGLS_OZ_FWD=raw is that FP64 functor for every digit count (bitwise the digits of round 1),
-  // =fix the integer functor for every digit count, =scaled the epilogue of round 1 on the scaled FP64 values
-  // (F2I / I2F slicing), =tma the raw functor with the digits staged in shared memory and stored by TMA (two-stage
-  // operand ring to make room; 0.44 against 0.425 ms per launch, profiles/r02_v16_fwd_microbench.txt).  raw, scaled and
-  // tma write the same bytes; fix may differ from them by one unit of the last digit (phase_fixed.cuh).
-  static const int mode = [] {
+  // Six digits: the FP64-free functor (EpiPhaseSliceFix: its integer work overlaps with the MMAs of the next tile, FP64
+  // work does not; 0.34 against 0.425 ms per launch, profiles/r02_v40_fwd_fix.txt) on 128 x 80 tiles when that takes
+  // fewer rounds of tiles.  With four digits the MMAs of a tile are too short to hide the longer integer functor, so
+  // the FP64 functor on the raw accumulators stays (0.076 against 0.078 ms).
+  // EMAGLS_OZ_FWD=raw runs that FP64 functor for six digits too: the reference the integer functor is tested against
+  // (it may differ from it by one unit of the last digit, phase_fixed.cuh).
+  static const bool raw = [] {
     const char* e = getenv("EMAGLS_OZ_FWD");
-    if (!e) return 4;
-    const std::string v(e);
-    return v == "scaled" ? 2 : (v == "tma" ? 0 : (v == "fix" ? 3 : (v == "raw" ? 1 : 4)));
+    return e && std::string(e) == "raw";
   }();
-  using Ring2 = oz::TileCfg<oz::TILE_N, 2>;
-  const bool fix = mode == 3 || (mode == 4 && a.T == 6);
-  if (fix) {
-    const int sms = sm_count();
-    const long long m_tiles = (a.D + oz::TILE_M - 1) / oz::TILE_M;
-    auto cost = [&](int nt) { return ((m_tiles * ((a.rows + nt - 1) / nt) + sms - 1) / sms) * (long long)(128 + nt); };
-    const bool wide = cost(oz::TileWide::NT) < cost(oz::TILE_N);
-    // 4-byte digit stores (lane-transposed) unless EMAGLS_OZ_FWD_BYTES is set or the row count is not a multiple of 4
-    static const bool bytes = getenv("EMAGLS_OZ_FWD_BYTES") != nullptr;
-    if (bytes || (a.rows & 3)) {
-      if (a.T == 6) return wide ? oz_fwd_t<6, EpiPhaseSliceFix<6>, oz::TileWide>(st, a) : oz_fwd_t<6, EpiPhaseSliceFix<6>>(st, a);
-      if (a.T == 4) return wide ? oz_fwd_t<4, EpiPhaseSliceFix<4>, oz::TileWide>(st, a) : oz_fwd_t<4, EpiPhaseSliceFix<4>>(st, a);
-      return cudaErrorInvalidValue;
-    }
-    // 80 columns = ten chunks per lane group: 20 epilogue warps take two each (16 leave 3 + 3 + 2 + 2; 0.321 against
-    // 0.334 ms per launch, profiles/r02_v46_cluster.txt)
-    using Wide20 = oz::TileCfg<80, 2, 20>;
-    if (a.T == 6) return wide ? oz_fwd_t<6, EpiPhaseSliceFix<6, true>, Wide20>(st, a) : oz_fwd_t<6, EpiPhaseSliceFix<6, true>>(st, a);
-    if (a.T == 4) return wide ? oz_fwd_t<4, EpiPhaseSliceFix<4, true>, Wide20>(st, a) : oz_fwd_t<4, EpiPhaseSliceFix<4, true>>(st, a);
-    return cudaErrorInvalidValue;
-  }
-  switch (a.T * 4 + (mode == 4 ? 1 : mode)) {
-    case 4 * 4 + 0: return oz_fwd_t<4, EpiPhaseSliceTma<4>, Ring2>(st, a);
-    case 6 * 4 + 0: return oz_fwd_t<6, EpiPhaseSliceTma<6>, Ring2>(st, a);
-    case 4 * 4 + 1: return oz_fwd_t<4, EpiPhaseSliceRaw<4>>(st, a);
-    case 6 * 4 + 1: return oz_fwd_t<6, EpiPhaseSliceRaw<6>>(st, a);
-    case 4 * 4 + 2: return oz_fwd_t<4, EpiPhaseSlice<4>>(st, a);
-    case 6 * 4 + 2: return oz_fwd_t<6, EpiPhaseSlice<6>>(st, a);
-    default: return cudaErrorInvalidValue;
-  }
+  if (a.T == 4) return oz_fwd_t<4, EpiPhaseSliceRaw<4>>(st, a);
+  if (a.T != 6) return cudaErrorInvalidValue;
+  if (raw) return oz_fwd_t<6, EpiPhaseSliceRaw<6>>(st, a);
+  if (a.rows & 3) return cudaErrorInvalidValue;   // the integer functor's 4-byte stores span four rows
+  // 80 columns = ten chunks per lane group: 20 epilogue warps take two each (16 leave 3 + 3 + 2 + 2; 0.321 against
+  // 0.334 ms per launch, profiles/r02_v46_cluster.txt)
+  using Wide20 = oz::TileCfg<80, 2, 20>;
+  const int sms = sm_count();
+  const long long m_tiles = (a.D + oz::TILE_M - 1) / oz::TILE_M;
+  auto cost = [&](int nt) { return ((m_tiles * ((a.rows + nt - 1) / nt) + sms - 1) / sms) * (long long)(128 + nt); };
+  if (cost(Wide20::NT) < cost(oz::TILE_N)) return oz_fwd_t<6, EpiPhaseSliceFix<6>, Wide20>(st, a);
+  return oz_fwd_t<6, EpiPhaseSliceFix<6>>(st, a);
 }
 
 cudaError_t launch_oz_bwd(cudaStream_t st, const int8_t* Tt_q, const double* sT, int rows, const int8_t* B_q,
@@ -491,10 +290,8 @@ cudaError_t launch_oz_bwd(cudaStream_t st, const int8_t* Tt_q, const double* sT,
     return ((tiles + sms - 1) / sms) * (long long)(128 + nt);
   };
   int nt = 64;
-  if (!getenv("EMAGLS_OZ_NARROW")) {
-    if (cost(80) <= cost(nt)) nt = 80;
-    if (cost(48) < cost(nt)) nt = 48;
-  }
+  if (cost(80) <= cost(nt)) nt = 80;
+  if (cost(48) < cost(nt)) nt = 48;
   const oz::EpiStoreF64 epi{tq, (long long)S};
   if (nt == 80) return oz::launch_ozaki_gemm<oz::EpiStoreF64, oz::TileWide>(st, Tt_q, sT, B_q, sB, rows, S, KpD, T, epi, sms);
   if (nt == 48) return oz::launch_ozaki_gemm<oz::EpiStoreF64, oz::TileCfg<48, 3>>(st, Tt_q, sT, B_q, sB, rows, S, KpD, T, epi, sms);

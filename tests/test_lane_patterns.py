@@ -1,7 +1,7 @@
 """CPU mirrors of two warp-level data-flow patterns of the CUDA path (no GPU needed): the lanes of a warp are the
 rows of a NumPy array, `__shfl_xor_sync(x, m)` is `x[lane ^ m]`, `__byte_perm` is restated below.
 
-* `EpiPhaseSliceFix<T, true>::apply` (emagls_b200/csrc/ozaki_kernels.cu): the digit bytes of four columns, packed per
+* `EpiPhaseSliceFix<T>::apply` (emagls_b200/csrc/ozaki_kernels.cu): the digit bytes of four columns, packed per
   digit plane, are transposed across groups of four lanes with two shuffles and two byte permutes, so that lane l
   holds rows l & ~3 .. (l & ~3) + 3 of column l & 3 and stores one 4-byte word.
 * `wsum2c` (emagls_b200/csrc/reflect.cuh): the warp sums of two complex values by reduce-scatter over the first two

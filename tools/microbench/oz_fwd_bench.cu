@@ -1,6 +1,9 @@
 // Timing + digit checksum of the forward direction-grid product of the MagLS recursion (launch_oz_fwd:
 // int8 tensor-core GEMM with the fused phase continuation / digit slicing epilogue) on synthetic digits of the
-// BASELINE config-2 shape, one epilogue variant per process (EMAGLS_OZ_FWD=scaled|raw|<unset>).
+// BASELINE config-2 shape.  Every epilogue variant launch_oz_fwd can take runs in turn: its digits are compared with
+// those of the FP64 functor (raw), and it is timed whole and in parts (GemmArgs::dbg).  Then, for six digits, synthetic
+// functors of one kind of work each run against the MMAs (interference study).
+// usage: oz_fwd_bench [P [sets [reps [T = 4 | 6 [variant: run it alone for about five seconds]]]]]
 // build: nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -o tools/microbench/bin/oz_fwd_bench
 //        tools/microbench/oz_fwd_bench.cu -lcuda ; run on a B200.
 #include <cstdio>
@@ -58,6 +61,7 @@ int main(int argc, char** argv) {
   const int P = argc > 1 ? atoi(argv[1]) : 3600, sets = argc > 2 ? atoi(argv[2]) : 1, reps = argc > 3 ? atoi(argv[3]) : 20;
   const int long_mode = argc > 5 ? atoi(argv[5]) : -1;   // >= 0: run this variant for about five seconds (clock sampling)
   const int T = argc > 4 ? atoi(argv[4]) : 6;
+  if (T != 4 && T != 6) { printf("T=%d: the forward product takes 4 or 6 digits\n", T); return 1; }
   const int D = 2702, S = 400, K = 8;
   const int rows = 4 * P * sets, KpS = emagls::oz_pad32(S), KpD = emagls::oz_pad32(D);
   std::mt19937_64 rng(7);
@@ -83,41 +87,17 @@ int main(int argc, char** argv) {
   emagls::OzFwdArgs fa{qY, sY, D, KpS, qC, sC, rows, T, qT, KpD, sT, dAbs + (size_t)kb * D, 2LL * K * D, (long long)K * D,
                        up + kb, sc + kb, K, P, 0};
   using namespace emagls;
-  using Ring2 = oz::TileCfg<oz::TILE_N, 2>;
+  // the forward epilogues the library launches: raw (the only one for four digits; for six digits the reference of
+  // EMAGLS_OZ_FWD=raw), and for six digits the integer functor on 128 x 64 tiles and on 128 x 80 tiles with 20 warps
   auto run = [&](int mode) -> cudaError_t {
-    if (T == 6) {
-      if (mode == 0) return oz_fwd_t<6, EpiPhaseSlice<6>>(0, fa);
-      if (mode == 1) return oz_fwd_t<6, EpiPhaseSliceRaw<6>>(0, fa);
-      if (mode == 3) return oz_fwd_t<6, EpiPhaseSliceRaw<6>, oz::TileWide>(0, fa);
-      if (mode == 4) return oz_fwd_t<6, EpiPhaseSliceRaw<6>, oz::TileCfg<48, 3>>(0, fa);
-      if (mode == 5) return oz_fwd_t<6, EpiPhaseSliceFix<6>>(0, fa);
-      if (mode == 6) return oz_fwd_t<6, EpiPhaseSliceFix<6>, oz::TileWide>(0, fa);
-      if (mode == 7) return oz_fwd_t<6, EpiPhaseSliceFix<6, true>>(0, fa);
-      if (mode == 8) return oz_fwd_t<6, EpiPhaseSliceFix<6, true>, oz::TileWide>(0, fa);
-      if (mode == 9) return oz_fwd_t<6, EpiPhaseSliceFix<6>, oz::TileCfg<80, 2, 20>>(0, fa);
-      if (mode == 10) return oz_fwd_t<6, EpiPhaseSliceFix<6, true>, oz::TileCfg<80, 2, 20>>(0, fa);
-      if (mode == 11) return oz_fwd_t<6, EpiPhaseSliceFix<6, true>, oz::TileCfg<80, 2, 24>>(0, fa);
-      if (mode == 12) return oz_fwd_t<6, EpiPhaseSliceFix<6, true>, oz::TileCfg<80, 2, 20, 1>>(0, fa);
-      if (mode == 13) return oz_fwd_t<6, EpiPhaseSliceFix<6, true>, oz::TileCfg<80, 2, 20, 2>>(0, fa);
-      return oz_fwd_t<6, EpiPhaseSliceTma<6>, Ring2>(0, fa);
-    }
-    if (mode == 0) return oz_fwd_t<4, EpiPhaseSlice<4>>(0, fa);
-    if (mode == 1) return oz_fwd_t<4, EpiPhaseSliceRaw<4>>(0, fa);
-    if (mode == 3) return oz_fwd_t<4, EpiPhaseSliceRaw<4>, oz::TileWide>(0, fa);
-    if (mode == 4) return oz_fwd_t<4, EpiPhaseSliceRaw<4>, oz::TileCfg<48, 3>>(0, fa);
-    if (mode == 5) return oz_fwd_t<4, EpiPhaseSliceFix<4>>(0, fa);
-    if (mode == 6) return oz_fwd_t<4, EpiPhaseSliceFix<4>, oz::TileWide>(0, fa);
-    if (mode == 7) return oz_fwd_t<4, EpiPhaseSliceFix<4, true>>(0, fa);
-    if (mode == 8) return oz_fwd_t<4, EpiPhaseSliceFix<4, true>, oz::TileWide>(0, fa);
-    if (mode == 9) return oz_fwd_t<4, EpiPhaseSliceFix<4>, oz::TileCfg<80, 2, 20>>(0, fa);
-    if (mode == 10) return oz_fwd_t<4, EpiPhaseSliceFix<4, true>, oz::TileCfg<80, 2, 20>>(0, fa);
-    if (mode == 11) return oz_fwd_t<4, EpiPhaseSliceFix<4, true>, oz::TileCfg<80, 2, 24>>(0, fa);
-    if (mode == 12) return oz_fwd_t<4, EpiPhaseSliceFix<4, true>, oz::TileCfg<80, 2, 20, 1>>(0, fa);
-    if (mode == 13) return oz_fwd_t<4, EpiPhaseSliceFix<4, true>, oz::TileCfg<80, 2, 20, 2>>(0, fa);
-    return oz_fwd_t<4, EpiPhaseSliceTma<4>, Ring2>(0, fa);
+    if (T == 4) return oz_fwd_t<4, EpiPhaseSliceRaw<4>>(0, fa);
+    if (mode == 0) return oz_fwd_t<6, EpiPhaseSliceRaw<6>>(0, fa);
+    if (mode == 1) return oz_fwd_t<6, EpiPhaseSliceFix<6>>(0, fa);
+    return oz_fwd_t<6, EpiPhaseSliceFix<6>, oz::TileCfg<80, 2, 20>>(0, fa);
   };
-  const char* names[14] = {"scaled", "raw", "tma", "raw80", "raw48", "fix", "fix80", "fixw", "fixw80", "fix80e20", "fixw80e20", "fixw80e24", "fixw80e20A", "fixw80e20B"};
-  const int mode_list[4] = {0, 1, 5, 10};   // ...A / ...B: cluster pairs with the A / B tile multicast   // fix*: FP64-free functor (byte stores), fixw*: the same with 4-byte stores
+  const char* names[3] = {"raw", "fix", "fix80e20"};
+  const int n_modes = T == 6 ? 3 : 1;
+  if (long_mode >= n_modes) { printf("variant %d: not run for T=%d\n", long_mode, T); return 1; }
   std::vector<int8_t> fixref;
   const size_t nq = (size_t)T * rows * KpD;
   std::vector<int8_t> ref(nq), got(nq);
@@ -136,7 +116,7 @@ int main(int argc, char** argv) {
     printf("long run %s: %.4f ms per launch after 12000 launches\n", names[long_mode], msl / 2000);
     return 0;
   }
-  for (int mode : mode_list) {
+  for (int mode = 0; mode < n_modes; ++mode) {
     CK(cudaMemset(qT, 0, nq));
     CK(cudaMemset(sT, 0, (size_t)rows * 8));
     CK(run(mode));
@@ -145,13 +125,13 @@ int main(int argc, char** argv) {
     CK(cudaMemcpy(sgot.data(), sT, (size_t)rows * 8, cudaMemcpyDeviceToHost));
     size_t bad = 0, bad_s = 0, shown = 0;
     double maxdiff = 0.0;
-    if (mode == 5) fixref = got;
-    if (mode > 5 && !fixref.empty()) {              // every variant of the integer functor writes the same bytes
+    if (mode == 1) fixref = got;
+    if (mode > 1) {                                  // every variant of the integer functor writes the same bytes
       size_t nb = 0;
       for (size_t i = 0; i < nq; ++i) nb += (got[i] != fixref[i]);
       printf("   %-9s vs fix: %zu of %zu bytes differ\n", names[mode], nb, nq);
     }
-    if (mode == 0) { ref = got; sref = sgot; }
+    if (mode == 0) { ref = got; sref = sgot; }   // the raw functor: the bytes of oz::slice_digits
     else {
       for (int r = 0; r < rows; ++r) {
         bad_s += (sgot[r] != sref[r]);
@@ -189,7 +169,7 @@ int main(int argc, char** argv) {
     float ms = 0;
     CK(cudaEventElapsedTime(&ms, e0, e1));
     const double ops = 2.0 * D * (double)rows * KpS * (T * (T + 1) / 2);
-    printf("oz_fwd %-9s P=%d sets=%d T=%d: %.4f ms per launch, %.0f int8 TOP/s; vs scaled: %zu of %zu values differ (max %.3g in units of the leading digit), %zu scales differ\n",
+    printf("oz_fwd %-9s P=%d sets=%d T=%d: %.4f ms per launch, %.0f int8 TOP/s; vs raw: %zu of %zu values differ (max %.3g in units of the leading digit), %zu scales differ\n",
            names[mode], P, sets, T, ms / reps, ops / (ms / reps * 1e-3) / 1e12, bad, (size_t)rows * KpD, maxdiff, bad_s);
   }
 

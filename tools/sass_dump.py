@@ -12,9 +12,9 @@ tag = sys.argv[1] if len(sys.argv) > 1 else "r02"
 out = os.path.join(ROOT, "profiles", f"{tag}_sass")
 os.makedirs(out, exist_ok=True)
 # (file name, substring of the demangled name) of the instances that run in the default em32 configuration
-WANT = [("ozaki_gemm_fwd_EpiPhaseSliceFix6_words_nt80_ew20", ["ozaki_gemm_kernel<6", "EpiPhaseSliceFix<6, true>", "TileCfg<80, 2, 20, 0>"]),
-        ("ozaki_gemm_fwd_EpiPhaseSliceRaw6_nt64", ["ozaki_gemm_kernel<6", "EpiPhaseSliceRaw<6>", "TileCfg<64, 3, 16, 0>"]),
-        ("ozaki_gemm_bwd_EpiStoreF64_6_nt80", ["ozaki_gemm_kernel<6", "EpiStoreF64", "TileCfg<80, 2, 16, 0>"]),
+WANT = [("ozaki_gemm_fwd_EpiPhaseSliceFix6_words_nt80_ew20", ["ozaki_gemm_kernel<6", "EpiPhaseSliceFix<6>", "TileCfg<80, 2, 20>"]),
+        ("ozaki_gemm_fwd_EpiPhaseSliceRaw6_nt64", ["ozaki_gemm_kernel<6", "EpiPhaseSliceRaw<6>", "TileCfg<64, 3, 16>"]),
+        ("ozaki_gemm_bwd_EpiStoreF64_6_nt80", ["ozaki_gemm_kernel<6", "EpiStoreF64", "TileCfg<80, 2, 16>"]),
         ("tsqr_sep_kernel", ["tsqr_sep_kernel"]), ("svdclip_kernel_occ4", ["svdclip_kernel<4>"]),
         ("chain_bwd_sep_kernel", ["chain_bwd_sep_kernel"]), ("bwd_fused_kernel_T6", ["bwd_fused_kernel<6>"]),
         ("gram_sweep_kernel", ["gram_sweep_kernel"]), ("fused_render16_kernel_pre1", ["fused_render16_kernel<1>"])]
