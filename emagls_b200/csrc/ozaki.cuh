@@ -143,7 +143,8 @@ __device__ __forceinline__ double i2d_exact(int a) {
   return __hiloint2double(0x43300000, a ^ (int)0x80000000) - 4503601774854144.0;   // 2^52 + 2^31
 }
 // Exact integer value of one output element from its T diagonal accumulators, rounded once to FP64:
-//   v = rn(sum_d acc_d 256^(T-1-d)) = rn(H 256^(T-3) + L),  H = digits 0..2 (|H| < 2^38), L = digits 3..T-1 (|L| < 2^42)
+//   v = rn(sum_d acc_d 256^(T-1-d)) = rn(H 256^(T-3) + L),  H = digits 0..2, L = digits 3..T-1
+// (|acc_d| < 2^31: |H|, |L| < 2^48, both exact in FP64; v itself may exceed 2^53 and is rounded once)
 template <int T>
 __device__ __forceinline__ double combine_diagonals(const int32_t (&a)[MAX_SLICES][8], int q) {
   double H = i2d_exact(a[0][q]);
@@ -157,7 +158,9 @@ __device__ __forceinline__ double combine_diagonals(const int32_t (&a)[MAX_SLICE
     if (d < T) L = fma(L, 256.0, i2d_exact(a[d][q]));
   return fma(H, (double)(1 << (8 * (T - 3))), L);
 }
-// The same integer, exact, in 64-bit integer arithmetic (|v| < 2^63): multiply-adds with 64-bit accumulators (IMAD.WIDE)
+// The same integer, exact, in 64-bit integer arithmetic while |v| < 2^63, which the int32 range of the accumulators does
+// not imply: the host checks drain_i64_fits (Kpad <= 2016 for T = 6), longer contractions would wrap silently.
+// Multiply-adds with 64-bit accumulators (IMAD.WIDE)
 // instead of 11 FP64 instructions per element -- the drain is the one phase of the epilogue that cannot overlap with
 // MMAs, and FP64 is the slowest pipe it could use.  For functors that declare `int64_values`.
 template <int T>
@@ -524,6 +527,14 @@ inline bool make_operand_map(CUtensorMap* tm, const int8_t* ptr, int rows, int K
 
 // int32 accumulators: a diagonal holds at most T pairs of products bounded by 2^14 each
 inline bool contraction_fits(int Kpad, int T) { return (long long)T * 16384LL * Kpad < (1LL << 31); }
+// 64-bit drain (combine_diagonals_i64): |v| <= Kpad sum_{i+j<T} max|q_i| max|q_j| 256^(T-1-i-j) < 2^63 with |q_0| <= 64,
+// |q_s| <= 128 (T = 6: 1.0157 Kpad 2^52, so Kpad <= 2016; T = 4: always, given contraction_fits)
+inline bool drain_i64_fits(int Kpad, int T) {
+  long long per_k = 0;
+  for (int d = 0; d < T; ++d)
+    for (int i = 0; i <= d; ++i) per_k += (long long)(i ? 128 : 64) * (d - i ? 128 : 64) << (8 * (T - 1 - d));
+  return Kpad <= 0x7FFFFFFFFFFFFFFFLL / per_k;
+}
 
 template <class Cfg>
 inline size_t gemm_smem_bytes(int T) { return (size_t)Cfg::ST * T * (A_SLICE_BYTES + Cfg::NT * TILE_K) + 1024; }

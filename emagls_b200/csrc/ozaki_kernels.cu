@@ -97,7 +97,7 @@ struct EpiPhaseSliceRaw {
 // (int64_values: the kernel instance then contains no FP64 instruction at all), they are normalised by
 // count-leading-zeros and shifts, |y|^-1 comes from a 22-bit MUFU seed and one third-order correction in 64-bit
 // fixed point, and the digits are those of rn(t 2^24) formed in integer arithmetic.  Against EpiPhaseSliceRaw the last digit may differ by one unit
-// (|Z - exact| <= 0.6 instead of <= 0.53; tests/test_phase_fixed.py).
+// (|Z - exact| <= 0.6 instead of <= 0.53; tests/test_phase_fixed.py on the host, tests/test_gpu_ozaki.py on the device).
 // Stores: the digit bytes of four columns are packed per plane, transposed across groups of four lanes (two shuffles
 // and two byte permutes per word) and leave as 4-byte stores: lane l writes rows l & ~3 .. (l & ~3) + 3 of column
 // l & 3: a quarter of the store instructions (and of their address arithmetic) of byte stores.  The whole warp enters
@@ -267,6 +267,9 @@ cudaError_t launch_oz_fwd(cudaStream_t st, const OzFwdArgs& a) {
   if (a.T != 6) return cudaErrorInvalidValue;
   if (raw) return oz_fwd_t<6, EpiPhaseSliceRaw<6>>(st, a);
   if (a.rows & 3) return cudaErrorInvalidValue;   // the integer functor's 4-byte stores span four rows
+  // Contractions over more than 2016 harmonics (simulation order 44 and up) may carry |y| beyond the range of the
+  // integer functor's 64-bit drain: the FP64 functor rounds once instead of wrapping.
+  if (!oz::drain_i64_fits(a.KpS, a.T)) return oz_fwd_t<6, EpiPhaseSliceRaw<6>>(st, a);
   // 80 columns = ten chunks per lane group: 20 epilogue warps take two each (16 leave 3 + 3 + 2 + 2; 0.321 against
   // 0.334 ms per launch, profiles/r02_v46_cluster.txt)
   using Wide20 = oz::TileCfg<80, 2, 20>;

@@ -13,24 +13,7 @@ the CPU as well (the CUDA kernels themselves are tested against the oracle in th
 import numpy as np
 import pytest
 
-
-def slice_digits(a, T):
-    """oz::slice_digits<T>: |a| <= 64 -> digits q[T] with a = sum q_s 256^-s + r."""
-    nh = T - 3
-    bias_hi = {3: 0x808080, 2: 0x8080, 1: 0x80}[nh]
-    ah = a * float(1 << (8 * (nh - 1)))
-    hi = np.rint(ah).astype(np.int64)
-    lo = np.rint((ah - hi) * 16777216.0).astype(np.int64)
-    yl = lo + 0x808080
-    hi = hi + (yl >> 24)
-    zl = yl ^ 0x808080
-    sb = lambda v: ((v & 0xFF) + 128) % 256 - 128          # noqa: E731  (int)(signed char)
-    q = np.zeros((T,) + a.shape, dtype=np.int64)
-    q[T - 1], q[T - 2], q[T - 3] = sb(zl), sb(zl >> 8), sb(zl >> 16)
-    zh = (hi + bias_hi) ^ bias_hi
-    for j in range(nh):
-        q[nh - 1 - j] = sb(zh >> (8 * j))
-    return q
+from oracle.ozaki_model import slice_digits
 
 
 @pytest.mark.parametrize("T", [4, 5, 6])
