@@ -492,14 +492,13 @@ void design_factored(emagls_ctx* h, const emagls_config& cfg, const DesignArgs& 
   // ---------------- memory plan: orientation chunks of OC, Gram bin groups of NB, TSQR slots of G
   const int ne = Mc * (Mc + 1) / 2, ne_ld = (ne + 1) & ~1;
   // Mc <= 32: register-resident TSQR / Jacobi / reflector kernels of tsqr_kernels.cu ("sep" block plan);
-  // EMAGLS_FACTOR_OLD=1 (A/B switch) and Mc > 32 use the shared-memory kernel of solver_kernels.cu.
-  const bool sep = (Mc <= 32) && getenv("EMAGLS_FACTOR_OLD") == nullptr;
+  // Mc > 32 uses the shared-memory kernel of solver_kernels.cu.
+  const bool sep = Mc <= 32;
   const BlockPlan bp = sep ? make_block_plan_sep(S, Mc) : make_block_plan(S, Mc);
   const int NB = std::min(128, K - 1);
   int g_slots = sep ? 16 : 4;  // bins factorised per launch; the Jacobi kernel warm-starts along them
   if (const char* e = getenv("EMAGLS_FACTOR_SLOTS")) g_slots = std::max(1, atoi(e));
   const int G = std::min(g_slots, K - 1);
-  const bool jacobi_warm = getenv("EMAGLS_JACOBI_COLD") == nullptr;
   const long long v_stride = sep ? 32LL * S : (long long)Mc * S, tau_stride = (long long)bp.nblk * bp.MC,
                   pb_stride = (long long)Mc * Mc;
   const size_t per_orient =
@@ -584,7 +583,6 @@ void design_factored(emagls_ctx* h, const emagls_config& cfg, const DesignArgs& 
     const int pj = a.num_sets * oc;
     const ProbMap pm{oc, o0, a.num_orient};
     bool cv_ready = false;                                      // digits of u_kb already produced by a fused tail
-    const bool fuse_fwd = getenv("EMAGLS_NO_FUSE") == nullptr;  // A/B switch
     const double* Yc = Yo + (size_t)o0 * Mc * S;
     {
       ProfSpan ps(h, EM_PROF_SETUP);
@@ -643,7 +641,7 @@ void design_factored(emagls_ctx* h, const emagls_config& cfg, const DesignArgs& 
             }
             {
               ProfSpan ps(h, EM_PROF_JACOBI);
-              EM_CUDA(launch_svdclip(st, Mc, Rbuf, ops, oc, Gn, cfg.svd_regul, try_fast, jacobi_warm ? 1 : 0));
+              EM_CUDA(launch_svdclip(st, Mc, Rbuf, ops, oc, Gn, cfg.svd_regul, try_fast));
             }
             h->launches += 2;
           } else {
@@ -713,7 +711,7 @@ void design_factored(emagls_ctx* h, const emagls_config& cfg, const DesignArgs& 
           {
             ProfSpan ps(h, EM_PROF_CHAIN_BWD);
             if (gram) {
-              const bool fuse = use_oz && fuse_fwd && kb + 1 < K;
+              const bool fuse = use_oz && kb + 1 < K;
               EM_CUDA(launch_bwd_small(st, Yc, Mc, S, d_roword, bk, pbg, pm, pj, tq, 0, 0, 0, nsplit, split_stride, Wsp,
                                        w_ear, K, kb, dc_fix, fuse ? bn + (size_t)(kb + 1) * (simN + 1) : nullptr, Cv_q, sCv,
                                        KpS, oz_T, simN));

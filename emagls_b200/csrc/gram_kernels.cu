@@ -12,7 +12,6 @@
 // A warp-per-matrix Cholesky in shared memory then yields G^-1 and the rigorous bound
 // cond_2(G) <= ||G||_F ||G^-1||_F that decides whether the bin may use this route; bins that fail
 // it go through the TSQR + Jacobi kernel (solver_kernels.cu).
-#include <cstdlib>
 #include "kernels.h"
 #include "ozaki.cuh"
 #include "reflect.cuh"
@@ -315,7 +314,7 @@ gram_sweep_kernel(const double* __restrict__ Gre, const double* __restrict__ Gim
 cudaError_t launch_gram_chol(cudaStream_t st, const double* Gre, const double* Gim, int Mc, int P,
                              int ne_ld, int nbins, double thr, cplx* Pb, int* fail) {
   const long long nmat = (long long)nbins * P;
-  if (Mc <= 32 && !getenv("EMAGLS_GRAM_CHOL")) {   // EMAGLS_GRAM_CHOL: A/B switch back to the shared-memory Cholesky
+  if (Mc <= 32) {
     gram_sweep_kernel<<<(unsigned)((nmat + GC_WPC - 1) / GC_WPC), GC_WPC * 32, 0, st>>>(Gre, Gim, Mc, P, ne_ld, nmat, thr,
                                                                                     Pb, fail);
     return cudaGetLastError();
@@ -910,11 +909,10 @@ cudaError_t launch_bwd_small(cudaStream_t st, const double* Y, int Mc, int S, co
 #define EM_BWD_ARGS num_prob, Y, Mc, S, roword, bk, Pb, pm, z, z_set_stride, z_ear_stride, z_shared, nsplit, \
                     split_stride, Wsp, w_ear_stride, K, k, dc_fix, ff
   // bwd_fused_kernel: Y_o staged once in shared memory (two CTAs per SM must fit; the bulk copy moves multiples of
-  // 16 bytes); EMAGLS_BWD_OLD=1 (A/B switch) and larger problems: bwd_small_kernel, which reads Y_o twice through L2.
-  static const bool old_kernel = getenv("EMAGLS_BWD_OLD") != nullptr;
+  // 16 bytes); larger problems: bwd_small_kernel, which reads Y_o twice through L2.
   const size_t fused_smem = (((size_t)Mc * S + 1) & ~(size_t)1) * sizeof(double) +
                             (size_t)(BF_WARPS * 64 + 64 + 64 + 80) * sizeof(cplx) + (4 * BF_WARPS + 4) * sizeof(double);
-  if (!old_kernel && N >= 0 && N < 40 && Mc <= 32 && S <= 128 * BF_CH && ((Mc * S) & 1) == 0 &&
+  if (N >= 0 && N < 40 && Mc <= 32 && S <= 128 * BF_CH && ((Mc * S) & 1) == 0 &&
       fused_smem <= 113 * 1024 && (!bk_next || KpS <= 64 * BF_WARPS)) {
     switch (Tf) {
       case 0: return launch_bwd_fused_t<0>(st, fused_smem, EM_BWD_ARGS, N);

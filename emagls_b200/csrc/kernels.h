@@ -94,7 +94,7 @@ BlockPlan make_block_plan_sep(int S, int Mc);
 cudaError_t launch_tsqr_sep(cudaStream_t st, const BlockPlan& bp, const RowSource& src, const OperatorSet& ops,
                             cplx* Rout, int num_prob, int kbase, int G);
 cudaError_t launch_svdclip(cudaStream_t st, int Mc, const cplx* Rin, const OperatorSet& ops, int num_prob, int G,
-                           double regul, int try_fast, int warm);
+                           double regul, int try_fast);
 cudaError_t launch_chain_bwd_sep(cudaStream_t st, const BlockPlan& bp, const OperatorSet& ops, int slot, int G,
                                  const double* tq, long long tq_set_stride, long long tq_ear_stride, int tq_shared,
                                  int nsplit, long long split_stride, ProbMap pm, cplx* Wsp, long long w_ear_stride,

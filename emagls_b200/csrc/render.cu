@@ -160,165 +160,26 @@ __global__ void unstage_output_kernel(const double* __restrict__ yseg, int nb, i
 }
 
 // ---------------------------------------------------------------------------------------------
-// Fused overlap-save block: one CTA per block of L output frames.  For every channel the N-point real
-// FFT (as an N/2-point complex Stockham FFT, radix 4 with a leading radix-2 stage when log2(N/2) is odd,
-// ping-pong in shared memory), the multiply-accumulate with both ears' filter spectra into two
-// accumulators in shared memory, then the two inverse transforms and the store of the valid L frames.
-// The channel spectra never reach HBM: the kernel reads the input once (plus the N/L overlap) and the
-// L2-resident filter spectra, and writes the two output channels.
+// fused_render16_kernel (N = 4096): one CTA per overlap-save block of L output frames.  For every channel the
+// N-point real FFT (as an M = N/2-point complex FFT), the multiply-accumulate with both ears' filter spectra into
+// two accumulators in shared memory, then the two inverse transforms and the store of the valid L frames.  The
+// channel spectra never reach HBM: the kernel reads the input once (plus the N/L overlap) and the L2-resident
+// filter spectra, and writes the two output channels.
 //   rfft:  X[k] = (Z[k] + conj(Z[M-k])) / 2 - (i/2) W_N^k (Z[k] - conj(Z[M-k])),  z[n] = x[2n] + i x[2n+1]
 //   irfft: Zy[k] = (Y[k] + conj(Y[M-k])) + i conj(W_N^k) (Y[k] - conj(Y[M-k])),  y[2n] + i y[2n+1] = IFFT_M(Zy) / N
-// WM[q] = exp(-2 pi i q / M) (q < M/2), WN[k] = exp(-2 pi i k / N) (k <= M), M = N / 2.
+// WN[k] = exp(-2 pi i k / N) (k <= M).
+// The complex transforms are register-resident radix-16 / radix-8 Stockham passes (2048 = 16 x 16 x 8).  Four
+// channels at a time, one radix-16 butterfly per thread and pass: the first pass reads its sixteen 16-byte sample
+// pairs straight from global memory (coalesced over the butterfly index; they are issued before the previous
+// group's spectra are accumulated, so the loads fly during that phase), the other two passes run in place in
+// shared memory (read - barrier - write - barrier) on buffers padded by one element per sixteen (the stride-16
+// writes of the first pass would otherwise hit one bank).
 // ---------------------------------------------------------------------------------------------
-__global__ void render_twiddle_kernel(int M, cplx* __restrict__ WM, cplx* __restrict__ WN) {
+__global__ void render_twiddle_kernel(int M, cplx* __restrict__ WN) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < M / 2) { double s_, c_; sincospi(-2.0 * (double)i / (double)M, &s_, &c_); WM[i] = mk(c_, s_); }
   if (i <= M) { double s_, c_; sincospi(-(double)i / (double)M, &s_, &c_); WN[i] = mk(c_, s_); }
 }
 
-// Stockham FFT of length M on ping-pong buffers, NB independent transforms side by side (buffer pair q at
-// src + q * stride, dst + q * stride; the twiddles are shared); returns the offset-0 buffer holding the results
-template <bool INV, int NB>
-__device__ __forceinline__ cplx* stockham_fft(cplx* src, cplx* dst, long long stride, int M, int logM,
-                                              const cplx* __restrict__ WM, int tid, int nt) {
-  int p = 1;
-  if (logM & 1) {
-    for (int j = tid; j < M / 2; j += nt) {
-#pragma unroll
-      for (int q = 0; q < NB; ++q) {
-        const cplx u0 = src[q * stride + j], u1 = src[q * stride + j + M / 2];
-        dst[q * stride + 2 * j] = cadd(u0, u1); dst[q * stride + 2 * j + 1] = csub(u0, u1);
-      }
-    }
-    __syncthreads();
-    cplx* t_ = src; src = dst; dst = t_;
-    p = 2;
-  }
-  const int T = M / 4;
-  while (p < M) {
-    const int tw = M / (4 * p);
-    for (int t = tid; t < T; t += nt) {
-      const int k = t & (p - 1);
-      cplx w1 = WM[k * tw], w2 = WM[2 * k * tw];
-      if (INV) { w1.y = -w1.y; w2.y = -w2.y; }
-      const cplx w3 = cmul(w1, w2);
-      const int j = ((t - k) << 2) + k;
-#pragma unroll
-      for (int q = 0; q < NB; ++q) {
-        const cplx* sq = src + q * stride;
-        cplx* dq = dst + q * stride;
-        const cplx u0 = sq[t], u1 = cmul(sq[t + T], w1), u2 = cmul(sq[t + 2 * T], w2), u3 = cmul(sq[t + 3 * T], w3);
-        const cplx v0 = cadd(u0, u2), v1 = csub(u0, u2), v2 = cadd(u1, u3);
-        cplx v3 = csub(u1, u3);
-        v3 = INV ? mk(-v3.y, v3.x) : mk(v3.y, -v3.x);          // * (+i) inverse, * (-i) forward
-        dq[j] = cadd(v0, v2); dq[j + p] = cadd(v1, v3); dq[j + 2 * p] = csub(v0, v2); dq[j + 3 * p] = csub(v1, v3);
-      }
-    }
-    __syncthreads();
-    cplx* t_ = src; src = dst; dst = t_;
-    p <<= 2;
-  }
-  return src;
-}
-
-// input block of one channel -> buffer (pairs x[2n], x[2n+1] as one complex value), asynchronously with zero fill
-// outside the signal (both samples of a pair are inside or outside: the block origin and num_samples are even)
-__device__ __forceinline__ void fused_load_async(cplx* buf, const double* __restrict__ x, long long s_first,
-                                                 long long num_samples, int M, int tid, int nt) {
-  for (int n = tid; n < M; n += nt) {
-    const long long i0 = s_first + 2LL * n;
-    const bool in_range = (i0 >= 0 && i0 < num_samples);
-    cp_async16(buf + n, x + (in_range ? i0 : 0), in_range);
-  }
-}
-
-// Two channels per pass (NB = 2): buffers [A0 | A1 | B0 | B1 | accL | accR].
-__global__ void __launch_bounds__(512, 1)
-fused_render_kernel(const double* __restrict__ in, long long num_samples, int num_ch, const cplx* __restrict__ Hw,
-                    const cplx* __restrict__ WM, const cplx* __restrict__ WN, int N, int logM, int L, int ov,
-                    long long skip, long long out_rows, double* __restrict__ out) {
-  extern __shared__ __align__(16) unsigned char fr_raw[];
-  const int M = N / 2, F = M + 1, tid = threadIdx.x, nt = blockDim.x;
-  cplx* A = reinterpret_cast<cplx*>(fr_raw);        // A0, A1
-  cplx* Bf = A + 2 * M;                             // B0, B1
-  cplx* accL = Bf + 2 * M;
-  cplx* accR = accL + F;
-  const long long b = blockIdx.x;
-  const long long s_first = b * (long long)L - ov;          // even: L and ov are even
-  for (int k = tid; k < F; k += nt) { accL[k] = mk(0.0, 0.0); accR[k] = mk(0.0, 0.0); }
-  // ping-pong roles: the transform of the pair in `cur` uses `oth` as scratch and leaves the spectra in one of
-  // the two; the other one is free while the spectra are unpacked and accumulated, so the next pair of channels
-  // is prefetched into it (cp.async) and becomes `cur` of the next iteration
-  cplx* cur = A;
-  cplx* oth = Bf;
-  fused_load_async(cur, in, s_first, num_samples, M, tid, nt);
-  if (num_ch > 1) fused_load_async(cur + M, in + num_samples, s_first, num_samples, M, tid, nt);
-  cp_async_commit();
-  for (int ch = 0; ch < num_ch; ch += 2) {
-    const int nb2 = (ch + 1 < num_ch) ? 2 : 1;
-    cp_async_wait<0>();
-    __syncthreads();
-    const cplx* Z = (nb2 == 2) ? stockham_fft<false, 2>(cur, oth, M, M, logM, WM, tid, nt)
-                               : stockham_fft<false, 1>(cur, oth, M, M, logM, WM, tid, nt);
-    cplx* freeb = (Z == cur) ? oth : cur;
-    if (ch + 2 < num_ch) {
-      fused_load_async(freeb, in + (long long)(ch + 2) * num_samples, s_first, num_samples, M, tid, nt);
-      if (ch + 3 < num_ch) fused_load_async(freeb + M, in + (long long)(ch + 3) * num_samples, s_first, num_samples, M, tid, nt);
-      cp_async_commit();
-    }
-    for (int q = 0; q < nb2; ++q) {
-      const cplx* Zq = Z + (long long)q * M;
-      const cplx* hl = Hw + (long long)(ch + q) * F;
-      const cplx* hr = Hw + ((long long)num_ch + ch + q) * F;
-      for (int k = tid; k < F; k += nt) {
-        const cplx zk = Zq[k & (M - 1)], zm = cconj(Zq[(M - k) & (M - 1)]);
-        const cplx sm_ = cadd(zk, zm), df = cmul(WN[k], csub(zk, zm));
-        const cplx X = mk(0.5 * (sm_.x + df.y), 0.5 * (sm_.y - df.x));     // sm/2 - (i/2) df
-        cfma(accL[k], X, hl[k]);
-        cfma(accR[k], X, hr[k]);
-      }
-    }
-    oth = (freeb == cur) ? oth : cur;
-    cur = freeb;
-    // the barrier at the top of the next iteration orders the reads of Z before the next transform's writes
-  }
-  __syncthreads();
-  // both ears side by side
-  const double inv_n = 1.0 / (double)N;
-  for (int k = tid; k < M; k += nt) {
-#pragma unroll
-    for (int ear = 0; ear < 2; ++ear) {
-      const cplx* acc = ear ? accR : accL;
-      const cplx yk = acc[k], ym = cconj(acc[M - k]);
-      const cplx sm_ = cadd(yk, ym), df = cmul(cconj(WN[k]), csub(yk, ym));
-      A[ear * M + k] = mk(sm_.x - df.y, sm_.y + df.x);               // sm + i df
-    }
-  }
-  __syncthreads();
-  const cplx* zy = stockham_fft<true, 2>(A, Bf, M, M, logM, WM, tid, nt);
-  for (int n = tid; n < M; n += nt) {
-    const int i = 2 * n;
-    if (i < ov) continue;
-    const long long s0 = b * (long long)L + (i - ov);
-#pragma unroll
-    for (int ear = 0; ear < 2; ++ear) {
-      const cplx v = zy[ear * M + n];
-      if (s0 < num_samples && s0 >= skip) out[(long long)ear * out_rows + (s0 - skip)] = v.x * inv_n;
-      if (s0 + 1 < num_samples && s0 + 1 >= skip) out[(long long)ear * out_rows + (s0 + 1 - skip)] = v.y * inv_n;
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------------------------
-// fused_render16_kernel (N = 4096, EMAGLS_RENDER_FUSED=2): the same overlap-save block per CTA with
-// register-resident radix-16 / radix-8 Stockham passes (2048 = 16 x 16 x 8).  Four channels at a time, one
-// radix-16 butterfly per thread and pass: the first pass reads its sixteen 16-byte sample pairs straight from
-// global memory (coalesced over the butterfly index; they are issued before the previous group's spectra are
-// accumulated, so the loads fly during that phase), the other two passes run in place in shared memory
-// (read - barrier - write - barrier) on buffers padded by one element per sixteen (the stride-16 writes of the
-// first pass would otherwise hit one bank).  Six barriers per FOUR transforms instead of six per two, sixteen
-// independent loads per thread instead of four.
-// ---------------------------------------------------------------------------------------------
 constexpr int FR_M = 2048, FR_T = 512, FR_LD = FR_M + FR_M / 16;   // complex points, threads, padded buffer length
 __device__ __forceinline__ int fr_pad(int i) { return i + (i >> 4); }
 
@@ -326,9 +187,6 @@ __device__ __forceinline__ int fr_pad(int i) { return i + (i >> 4); }
 // P2[ji][k] = exp(-2 pi i k 2^ji / 256) (stride-16 pass, k < 16, ji < 4) at ji * 16 + k, then
 // P3[ji][tt] = exp(-2 pi i tt 2^ji / 2048) (last pass, tt < 256, ji < 3) at 64 + ji * 256 + tt.
 constexpr int FR_TW = 4 * 16 + 3 * 256;
-#ifndef EMAGLS_FR_TW_SMEM
-#define EMAGLS_FR_TW_SMEM 0     // 1: the kernel copies the table into shared memory (A/B: slower, it shrinks the L1)
-#endif
 __global__ void render_twiddle_full_kernel(cplx* __restrict__ TW) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= FR_TW) return;
@@ -459,64 +317,15 @@ __device__ __forceinline__ void fr_load_first(cplx (&v)[16], const double* __res
   }
 }
 
-__device__ __forceinline__ void fr_prefetch_first(const double* __restrict__ in, long long num_samples, int ch, bool valid,
-                                                  long long s_first, int t) {
-  if (!valid || (t & 7) != 0) return;          // one prefetch per 128-byte line (eight 16-byte pairs)
-  const double* x = in + (long long)ch * num_samples;
-#pragma unroll
-  for (int q = 0; q < 16; ++q) {
-    const long long i0 = s_first + 2LL * (t + 128 * q);
-    if (i0 >= 0 && i0 < num_samples) asm volatile("prefetch.global.L2 [%0];" ::"l"(x + i0));
-  }
-}
-
-// bin k of the spectra of channels cg .. cg + nc - 1 (packed transforms in Zb) into the two ears' accumulators; the
-// filter spectra of all CU channels are requested before anything is computed (CU = 4: full group, CU = 1: tail)
-template <int CU>
-__device__ __forceinline__ void fr_accumulate(const cplx* Zb, cplx* accL, cplx* accR, const cplx* __restrict__ Hw,
-                                              const cplx* __restrict__ WN, int num_ch, int cg, int k, int nc) {
-  constexpr int M = FR_M, F = FR_M + 1;
-  const cplx wn = WN[k];
-  cplx aL = accL[k], aR = accR[k];
-  const int ik = fr_pad(k & (M - 1)), im = fr_pad((M - k) & (M - 1));
-  for (int c0 = 0; c0 < nc; c0 += CU) {
-    cplx hl[CU], hr[CU];
-#pragma unroll
-    for (int u = 0; u < CU; ++u) {
-      const int c = min(c0 + u, nc - 1);           // a channel past the end: loaded again, not used
-      hl[u] = Hw[(long long)(cg + c) * F + k];
-      hr[u] = Hw[((long long)num_ch + cg + c) * F + k];
-    }
-#pragma unroll
-    for (int u = 0; u < CU; ++u) {
-      if (c0 + u >= nc) break;
-      const cplx zk = Zb[(c0 + u) * FR_LD + ik], zm = cconj(Zb[(c0 + u) * FR_LD + im]);
-      const cplx sm_ = cadd(zk, zm), df = cmul(wn, csub(zk, zm));
-      const cplx X = mk(0.5 * (sm_.x + df.y), 0.5 * (sm_.y - df.x));     // sm/2 - (i/2) df
-      cfma(aL, X, hl[u]);
-      cfma(aR, X, hr[u]);
-    }
-  }
-  accL[k] = aL; accR[k] = aR;
-}
-
-// PRE = 1: the next group's samples are loaded into registers before the accumulation (they fly during it);
-// PRE = 0: they are only pulled into L2 there and loaded afterwards (more registers for the filter spectra in flight)
-template <int PRE>
 __global__ void __launch_bounds__(FR_T, 1)
 fused_render16_kernel(const double* __restrict__ in, long long num_samples, int num_ch, const cplx* __restrict__ Hw,
-                      const cplx* __restrict__ TWg, const cplx* __restrict__ WN, int L, int ov, long long skip,
+                      const cplx* __restrict__ TW, const cplx* __restrict__ WN, int L, int ov, long long skip,
                       long long out_rows, double* __restrict__ out) {
   extern __shared__ __align__(16) unsigned char fr16_raw[];
   constexpr int M = FR_M, F = FR_M + 1, N = 2 * FR_M;
   cplx* Zb = reinterpret_cast<cplx*>(fr16_raw);        // [4][FR_LD]
   cplx* accL = Zb + 4 * FR_LD;                         // [F]
   cplx* accR = accL + F;
-#if EMAGLS_FR_TW_SMEM
-  cplx* TW = accR + F;                                 // [FR_TW]
-#else
-  const cplx* TW = TWg;
-#endif
   const int tid = threadIdx.x, g4 = tid >> 7, t = tid & 127;
   cplx* Z = Zb + g4 * FR_LD;
   const long long b = blockIdx.x;
@@ -524,9 +333,6 @@ fused_render16_kernel(const double* __restrict__ in, long long num_samples, int 
   cplx v[16];
   fr_load_first(v, in, num_samples, g4, g4 < num_ch, s_first, t);
   for (int k = tid; k < F; k += FR_T) { accL[k] = mk(0.0, 0.0); accR[k] = mk(0.0, 0.0); }
-#if EMAGLS_FR_TW_SMEM
-  for (int i = tid; i < FR_TW; i += FR_T) TW[i] = TWg[i];
-#endif
   for (int cg = 0; cg < num_ch; cg += 4) {
     // ---- pass 1 (stride 1, no twiddles) from the registers loaded ahead
     fr_dft16<false>(v);
@@ -542,29 +348,21 @@ fused_render16_kernel(const double* __restrict__ in, long long num_samples, int 
     // ---- this group's spectra are unpacked and accumulated while the next group's samples are on their way
     const bool more = cg + 4 < num_ch;
     const int nc = min(4, num_ch - cg);
-    if (PRE) {
-      if (more) fr_load_first(v, in, num_samples, cg + 4 + g4, cg + 4 + g4 < num_ch, s_first, t);
-      for (int j = 0; j < 5; ++j) {
-        const int k = tid + FR_T * j;
-        if (k > M) break;                              // bin M (Nyquist) belongs to thread 0
-        const cplx wn = WN[k];
-        cplx aL = accL[k], aR = accR[k];
-        const int ik = fr_pad(k & (M - 1)), im = fr_pad((M - k) & (M - 1));
-        for (int c = 0; c < nc; ++c) {
-          const cplx zk = Zb[c * FR_LD + ik], zm = cconj(Zb[c * FR_LD + im]);
-          const cplx sm_ = cadd(zk, zm), df = cmul(wn, csub(zk, zm));
-          const cplx X = mk(0.5 * (sm_.x + df.y), 0.5 * (sm_.y - df.x));     // sm/2 - (i/2) df
-          cfma(aL, X, Hw[(long long)(cg + c) * F + k]);
-          cfma(aR, X, Hw[((long long)num_ch + cg + c) * F + k]);
-        }
-        accL[k] = aL; accR[k] = aR;
+    if (more) fr_load_first(v, in, num_samples, cg + 4 + g4, cg + 4 + g4 < num_ch, s_first, t);
+    for (int j = 0; j < 5; ++j) {
+      const int k = tid + FR_T * j;
+      if (k > M) break;                              // bin M (Nyquist) belongs to thread 0
+      const cplx wn = WN[k];
+      cplx aL = accL[k], aR = accR[k];
+      const int ik = fr_pad(k & (M - 1)), im = fr_pad((M - k) & (M - 1));
+      for (int c = 0; c < nc; ++c) {
+        const cplx zk = Zb[c * FR_LD + ik], zm = cconj(Zb[c * FR_LD + im]);
+        const cplx sm_ = cadd(zk, zm), df = cmul(wn, csub(zk, zm));
+        const cplx X = mk(0.5 * (sm_.x + df.y), 0.5 * (sm_.y - df.x));     // sm/2 - (i/2) df
+        cfma(aL, X, Hw[(long long)(cg + c) * F + k]);
+        cfma(aR, X, Hw[((long long)num_ch + cg + c) * F + k]);
       }
-    } else {
-      if (more) fr_prefetch_first(in, num_samples, cg + 4 + g4, cg + 4 + g4 < num_ch, s_first, t);
-#pragma unroll
-      for (int j = 0; j < 4; ++j) fr_accumulate<4>(Zb, accL, accR, Hw, WN, num_ch, cg, tid + FR_T * j, nc);
-      if (tid == 0) fr_accumulate<4>(Zb, accL, accR, Hw, WN, num_ch, cg, M, nc);
-      if (more) fr_load_first(v, in, num_samples, cg + 4 + g4, cg + 4 + g4 < num_ch, s_first, t);
+      accL[k] = aL; accR[k] = aR;
     }
   }
   __syncthreads();
@@ -723,68 +521,30 @@ void binaural_decode_dev(emagls_ctx* h, const double* in, long long num_samples,
     h->launches += 1;
   }
 
-  // Fused route (EMAGLS_RENDER_FUSED=1; off by default): one kernel per call, the channel spectra stay in shared
-  // memory.  Needs the FFT and both accumulators in one CTA's shared memory (N <= 4096) and 16-byte aligned
-  // channels.  Measured on B200 (10 minutes, 32 channels, 512 taps; tools/gpu_render_ab.py,
-  // profiles/r01_v25_render_ab.txt): identical output to 8e-16, but 11.8 ms against 9.6 ms for the cuFFT route
-  // below (15.3 ms before two channels shared a pass and the next pair was prefetched with cp.async) -- the radix-4
-  // shared-memory FFT makes six barrier-separated passes per channel pair with one 512-thread CTA per SM; it needs
-  // register-resident radix-8/16 passes before it can win.
-  // Default route for N = 4096 (filters of 257 .. 512 taps): the register-resident fused kernel (radix 16 x 16 x 8),
-  // 6.7 ms against 9.7 ms for the cuFFT route on 10 minutes x 32 channels (profiles/r02_v27_render_reps.txt).
-  // EMAGLS_RENDER_FUSED=0 selects the cuFFT route, =1 the shared-memory radix-4 kernel of round 1, =3 the variant of
-  // the default that only pulls the next group's samples into L2 during the accumulation (8.9 ms).
-  const int fused_mode = env_int("EMAGLS_RENDER_FUSED", 2);
-  if ((fused_mode == 2 || fused_mode == 3) && N == 2 * FR_M && (num_samples % 2 == 0) && (ov % 2 == 0) &&
+  // Default route for N = 4096 (filters of 257 .. 512 taps): the fused kernel, one launch per call with the channel
+  // spectra in shared memory.  6.7 ms against 9.7 ms for the cuFFT route below on 10 minutes x 32 channels
+  // (profiles/r02_v27_render_reps.txt).  It needs 16-byte aligned channels; EMAGLS_RENDER_FUSED=0 selects the
+  // cuFFT route.
+  if (env_int("EMAGLS_RENDER_FUSED", 1) != 0 && N == 2 * FR_M && (num_samples % 2 == 0) && (ov % 2 == 0) &&
       (reinterpret_cast<uintptr_t>(in) % 16 == 0)) {
     cplx* TW = ar.get<cplx>((size_t)FR_TW);
-    cplx* WMu = ar.get<cplx>((size_t)FR_M / 2 + 1);
     cplx* WN = ar.get<cplx>((size_t)FR_M + 1);
     render_twiddle_full_kernel<<<(FR_TW + 255) / 256, 256, 0, st>>>(TW);
-    render_twiddle_kernel<<<(FR_M + 1 + 255) / 256, 256, 0, st>>>(FR_M, WMu, WN);
+    render_twiddle_kernel<<<(FR_M + 1 + 255) / 256, 256, 0, st>>>(FR_M, WN);
     EM_CUDA(cudaGetLastError());
-    const size_t smem = ((size_t)4 * FR_LD + 2 * (FR_M + 1) + (EMAGLS_FR_TW_SMEM ? FR_TW : 0)) * sizeof(cplx);
+    const size_t smem = ((size_t)4 * FR_LD + 2 * (FR_M + 1)) * sizeof(cplx);
     static bool attr_set = false;
     if (!attr_set) {
-      EM_CUDA(cudaFuncSetAttribute(fused_render16_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      EM_CUDA(cudaFuncSetAttribute(fused_render16_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      EM_CUDA(cudaFuncSetAttribute(fused_render16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       attr_set = true;
     }
     {
       ProfSpan ps(h, EM_PROF_RENDER_MAC);
-      if (fused_mode == 2)
-        fused_render16_kernel<1><<<(unsigned)nblk_total, FR_T, smem, st>>>(in, num_samples, num_ch, Hw, TW, WN, L, ov, skip,
-                                                                         out_rows, out);
-      else
-        fused_render16_kernel<0><<<(unsigned)nblk_total, FR_T, smem, st>>>(in, num_samples, num_ch, Hw, TW, WN, L, ov, skip,
-                                                                         out_rows, out);
+      fused_render16_kernel<<<(unsigned)nblk_total, FR_T, smem, st>>>(in, num_samples, num_ch, Hw, TW, WN, L, ov, skip,
+                                                                     out_rows, out);
       EM_CUDA(cudaGetLastError());
     }
     h->launches += 3;
-    return;
-  }
-  if (fused_mode == 1 && N <= 4096 && N >= 8 && (num_samples % 2 == 0) && (ov % 2 == 0) &&
-      (reinterpret_cast<uintptr_t>(in) % 16 == 0)) {
-    const int M2 = N / 2;
-    int logM = 0;
-    while ((1 << logM) < M2) ++logM;
-    cplx* WM = ar.get<cplx>((size_t)M2 / 2 + 1);
-    cplx* WN = ar.get<cplx>((size_t)M2 + 1);
-    render_twiddle_kernel<<<(M2 + 1 + 255) / 256, 256, 0, st>>>(M2, WM, WN);
-    EM_CUDA(cudaGetLastError());
-    const size_t smem = ((size_t)4 * M2 + 2 * (M2 + 1)) * sizeof(cplx);   // two channels side by side
-    static size_t set_to = 0;
-    if (smem > 48 * 1024 && smem > set_to) {
-      EM_CUDA(cudaFuncSetAttribute(fused_render_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      set_to = smem;
-    }
-    {
-      ProfSpan ps(h, EM_PROF_RENDER_MAC);
-      fused_render_kernel<<<(unsigned)nblk_total, 512, smem, st>>>(in, num_samples, num_ch, Hw, WM, WN, N, logM, L, ov, skip,
-                                                                  out_rows, out);
-      EM_CUDA(cudaGetLastError());
-    }
-    h->launches += 2;
     return;
   }
 

@@ -10,7 +10,6 @@
 //     Y_reg_inv = B * conj(Q_C) * Pb,     Pb = conj(J) diag(1/(s max(s, c s_max))) X^T.
 // When no singular value can be clipped (||R||_F ||R^-1||_F <= 1/c, a rigorous bound) the
 // Jacobi sweeps are skipped and Pb = R_C^-T (plain least squares).
-#include <cstdlib>
 #include "kernels.h"
 #include "reflect.cuh"
 
@@ -22,11 +21,9 @@ BlockPlan make_block_plan(int S, int Mc) {
   BlockPlan bp;
   bp.S = S; bp.Mc = Mc; bp.sep = 0;
   bp.MC = (Mc <= 32) ? 32 : 64;
-  // MC = 32: row blocks of 96 (three CTAs per SM).  EMAGLS_FACTOR_RB=64 selects blocks of 64 (52 KB working
-  // set, four CTAs of <= 64 registers per thread per SM): measured on B200 the factor kernel gains 2.7 %
-  // and the reflector chain, which then has 192 instead of 128 reflectors per problem, loses as much.
-  static const int rb32 = [] { const char* e = getenv("EMAGLS_FACTOR_RB"); return (e && atoi(e) == 64) ? 64 : 96; }();
-  bp.RB = (bp.MC == 32) ? rb32 : 128;
+  // MC = 32: row blocks of 96 (three CTAs per SM).  Blocks of 64 (four CTAs per SM) measured on B200: the factor
+  // kernel gains 2.7 % and the reflector chain, which then has 192 instead of 128 reflectors per problem, loses as much.
+  bp.RB = (bp.MC == 32) ? 96 : 128;
   bp.R0 = (S < Mc + bp.RB) ? S : Mc + bp.RB;
   bp.nblk = 1 + (S - bp.R0 + bp.RB - 1) / bp.RB;
   return bp;
@@ -149,7 +146,7 @@ __device__ void qr_block(cplx* Wk, int LD, int Mc, bool first, int hi, cplx* tau
 }
 
 template <int MC, int RB>
-__global__ void __launch_bounds__(FT, (MC == 32) ? (RB <= 64 ? 4 : 3) : 1)
+__global__ void __launch_bounds__(FT, (MC == 32) ? 3 : 1)
 factor_kernel(BlockPlan bp, RowSource src, OperatorSet ops, int kbase, int G, double regul, int try_fast) {
   // one element of padding per column: with LD = MC + RB the column stride is a multiple of 128 bytes and the
   // block loads / flushes below (consecutive threads -> consecutive columns) hit one bank group (ncu, round 1: 4.3-way)
@@ -304,25 +301,8 @@ factor_kernel(BlockPlan bp, RowSource src, OperatorSet ops, int kbase, int G, do
     // orders below the 1e-12 the projector is needed to, so no trailing check sweep is run after it.
     // (Offline study on the em32 bins, row-cyclic order: the same projector to every printed digit as with
     // a 1e-9 threshold, one sweep less on most bins: 9 -> 8, 8 -> 7.)
-#ifdef EMAGLS_JACOBI_INCR_NORMS
-    // Compile-time variant for the next round's A/B (not built by default, not yet measured on the GPU): the
-    // squared column norms are kept in shared memory, refreshed at the start of every sweep and updated by the
-    // rotation (a' = a - t |g|, b' = b + t |g|; de Rijk), so that only the inner product g is reduced per pair.
-    // Offline study (profiles/r01_jacobi_offline_study.txt): same sweeps and projector accuracy.
-    double* nrm = reinterpret_cast<double*>(bn_s) + 64;
-#endif
     for (sweeps = 1; sweeps <= 40; ++sweeps) {
       int big = 0;
-#ifdef EMAGLS_JACOBI_INCR_NORMS
-      for (int j = warp; j < Mc; j += FT / 32) {
-        double a_ = 0.0;
-#pragma unroll
-        for (int u = 0; u < MC / 32; ++u) a_ += cabs2(Xs[j * MC + lane + 32 * u]);
-        a_ = wsum(a_);
-        if (lane == 0) nrm[j] = a_;
-      }
-      __syncthreads();
-#endif
       for (int r = 0; r < ne - 1; ++r) {
         for (int pi = warp * 2 + half; pi < ne / 2; pi += FT / 16) {
           int p, q;
@@ -336,21 +316,14 @@ factor_kernel(BlockPlan bp, RowSource src, OperatorSet ops, int kbase, int G, do
           for (int u = 0; u < RPL; ++u) {
             int row = hl + 16 * u;
             xp[u] = Xs[p * MC + row]; xq[u] = Xs[q * MC + row];
-#ifndef EMAGLS_JACOBI_INCR_NORMS
             a += cabs2(xp[u]); b += cabs2(xq[u]);
-#endif
             cfmac(g, xp[u], xq[u]);
           }
 #pragma unroll
           for (int sft = 8; sft > 0; sft >>= 1) {
-#ifndef EMAGLS_JACOBI_INCR_NORMS
             a += __shfl_xor_sync(hmask, a, sft); b += __shfl_xor_sync(hmask, b, sft);
-#endif
             g.x += __shfl_xor_sync(hmask, g.x, sft); g.y += __shfl_xor_sync(hmask, g.y, sft);
           }
-#ifdef EMAGLS_JACOBI_INCR_NORMS
-          a = nrm[p]; b = nrm[q];
-#endif
           const double gg = cabs2(g), ab = a * b;
           if (gg > tol2 * ab && gg > 0.0) {
             if (gg > 1e-14 * ab) big = 1;
@@ -373,9 +346,6 @@ factor_kernel(BlockPlan bp, RowSource src, OperatorSet ops, int kbase, int G, do
               cplx njq = cscale(jq, cs); cfma(njq, sph, jp);
               Js[p * MC + row] = njp; Js[q * MC + row] = njq;
             }
-#ifdef EMAGLS_JACOBI_INCR_NORMS
-            if (hl == 0) { nrm[p] = fma(-tw, gg, a); nrm[q] = fma(tw, gg, b); }
-#endif
           }
         }
         __syncthreads();
@@ -428,15 +398,7 @@ cudaError_t launch_factor(cudaStream_t st, const BlockPlan& bp, const RowSource&
                           const OperatorSet& ops, int num_prob, int kbase, int G, double regul, int try_fast) {
   size_t smem = factor_smem_bytes(bp);
   cudaError_t e;
-  if (bp.MC == 32 && bp.RB == 64) {
-    static bool set32n = false;
-    if (!set32n) {
-      e = cudaFuncSetAttribute(factor_kernel<32, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      if (e != cudaSuccess) return e;
-      set32n = true;
-    }
-    factor_kernel<32, 64><<<num_prob * G, FT, smem, st>>>(bp, src, ops, kbase, G, regul, try_fast);
-  } else if (bp.MC == 32) {
+  if (bp.MC == 32) {
     static bool set32 = false;
     if (!set32) {
       e = cudaFuncSetAttribute(factor_kernel<32, 96>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

@@ -331,7 +331,7 @@ tsqr_sep_kernel(BlockPlan bp, RowSource src, OperatorSet ops, cplx* __restrict__
 // independent rotations of a phase are reduced together (the halves of the 16-lane group end up with one
 // inner product each) and their parameters are computed once per 8-lane group, then exchanged.
 // =============================================================================================
-constexpr int SV_T = 128;
+constexpr int SV_T = 128, SV_CTAS = 4;   // threads, CTAs per SM (128 registers per thread)
 
 struct RotParam { double cs, sx, sy, na, nb; int rot; };
 
@@ -400,10 +400,9 @@ __device__ __forceinline__ void rot_phase(cplx (&xa)[2], cplx (&xb)[2], cplx (&j
   if (p2.rot) { rot_apply(p2, xc, xd, jc, jd); nc = p2.na; nd = p2.nb; }
 }
 
-template <int OCC>
-__global__ void __launch_bounds__(SV_T, OCC)
-svdclip_kernel(int Mc, const cplx* __restrict__ Rin, OperatorSet ops, int G, double regul, int try_fast, int warm,
-               int split_from, int pieces, double warm_grading) {
+__global__ void __launch_bounds__(SV_T, SV_CTAS)
+svdclip_kernel(int Mc, const cplx* __restrict__ Rin, OperatorSet ops, int G, double regul, int try_fast, int split_from,
+               int pieces, double warm_grading) {
   extern __shared__ __align__(16) unsigned char sv_raw[];
   cplx* Xs = reinterpret_cast<cplx*>(sv_raw);           // column-major: X(i, c) = Xs[c*32 + i]
   cplx* Js = Xs + 1024;                                 // column-major
@@ -478,7 +477,7 @@ svdclip_kernel(int Mc, const cplx* __restrict__ Rin, OperatorSet ops, int G, dou
       // ---- starting matrix: warm (X = R^H J_prev) where the diagonal of R_C is graded by less than 1 / warm_grading
       // (the product costs eps * grading of relative accuracy in the small columns), else cold (X = R^H, J = I)
       bool use_warm = false;
-      if (warm && have_j) {
+      if (have_j) {
         if (tid < 32) {
           const double d = (tid < Mc) ? fabs(Rg[tid * 32 + tid].x) : 0.0;
           double dmax = d, dmin = (tid < Mc) ? d : 1e300;
@@ -723,20 +722,17 @@ static int sv_sm_count() {
 }
 
 cudaError_t launch_svdclip(cudaStream_t st, int Mc, const cplx* Rin, const OperatorSet& ops, int num_prob, int G,
-                           double regul, int try_fast, int warm) {
+                           double regul, int try_fast) {
   if (Mc > 32) return cudaErrorInvalidValue;
   const size_t smem = (size_t)2 * 1024 * sizeof(cplx) + (size_t)(32 + 32 + 20) * sizeof(double);
-  // EMAGLS_JACOBI_OCC=5: five CTAs per SM under a 102-register cap (A/B switch; default four CTAs, 128 registers)
-  static const int occ = [] { const char* e = getenv("EMAGLS_JACOBI_OCC"); return (e && atoi(e) == 5) ? 5 : 4; }();
   // Tail of the grid: CTAs take about equally long, so with `resident` CTAs in flight a launch lasts
   // ceil(num_prob / resident) rounds and the last round may be almost empty (3600 orientations on 592 places: 6.08
   // -> 7 rounds).  The orientations of that remainder are cut into bin ranges, as many as fit into one round, so
-  // the last round lasts 1 / pieces of a full one (plus one cold Jacobi start per piece).  EMAGLS_JACOBI_NO_SPLIT=1: off.
-  static const bool no_split = getenv("EMAGLS_JACOBI_NO_SPLIT") != nullptr;
-  const int resident = occ * sv_sm_count();
+  // the last round lasts 1 / pieces of a full one (plus one cold Jacobi start per piece).
+  const int resident = SV_CTAS * sv_sm_count();
   int split_from = num_prob, pieces = 1;
   const int rem = num_prob % resident;
-  if (!no_split && num_prob > resident && rem > 0 && G > 1) {
+  if (num_prob > resident && rem > 0 && G > 1) {
     pieces = std::min(G, resident / rem);
     if (pieces > 1) split_from = num_prob - rem; else pieces = 1;
   }
@@ -745,8 +741,7 @@ cudaError_t launch_svdclip(cudaStream_t st, int Mc, const cplx* Rin, const Opera
   // errors of bins 1-15 against exact arithmetic are the same 1e-14 with 1e-4, 1e-6 and 1e-9 (tests/test_gpu_arbitration.py,
   // profiles/r02_v51_*), the mean sweep count falls from 6.65 to 6.4 (bins 3-18 start warm: 9.2 -> 7.0-8.4 sweeps)
   static const double warm_grading = [] { const char* e = getenv("EMAGLS_JACOBI_WARM_GRADING"); return e ? atof(e) : 1e-8; }();
-  if (occ == 5) svdclip_kernel<5><<<grid, SV_T, smem, st>>>(Mc, Rin, ops, G, regul, try_fast, warm, split_from, pieces, warm_grading);
-  else svdclip_kernel<4><<<grid, SV_T, smem, st>>>(Mc, Rin, ops, G, regul, try_fast, warm, split_from, pieces, warm_grading);
+  svdclip_kernel<<<grid, SV_T, smem, st>>>(Mc, Rin, ops, G, regul, try_fast, split_from, pieces, warm_grading);
   return cudaGetLastError();
 }
 

@@ -4,7 +4,8 @@ the CPU as well (the CUDA kernels themselves are tested against the oracle in th
 * balanced base-256 slicing of `oz::slice_digits` (emagls_b200/csrc/ozaki.cuh) and the exactness of the
   sliced product with the i + j < T truncation,
 * the Hermitian sweep inversion of `gram_sweep_kernel` (emagls_b200/csrc/gram_kernels.cu),
-* the radix-2/4 Stockham FFT with real pack/unpack of `fused_render_kernel` (emagls_b200/csrc/render.cu),
+* the real pack/unpack of `fused_render16_kernel` (emagls_b200/csrc/render.cu): N-point real transforms as
+  N/2-point complex ones,
 * the row-block skipping rule of `tsqr_sep_kernel` (emagls_b200/csrc/tsqr_kernels.cu: significant_blocks) with the bound
   it relies on checked on the em32 steering factor,
 * the radix 16 x 16 x 8 passes of `fused_render16_kernel` (register layouts, twiddle tables, output placement),
@@ -74,50 +75,21 @@ def test_hermitian_sweep_inversion(M, cond):
     assert np.allclose(piv, np.abs(np.diag(L)) ** 2, rtol=1e-9)
 
 
-def stockham(a, WM, inverse):
-    """stockham_fft<INV, 1>: leading radix-2 pass when log2(M) is odd, then radix-4 passes."""
-    M = a.size
-    logM = int(round(np.log2(M)))
-    src, dst = a.copy(), np.empty_like(a)
-    p = 1
-    if logM & 1:
-        j = np.arange(M // 2)
-        dst[2 * j], dst[2 * j + 1] = src[j] + src[j + M // 2], src[j] - src[j + M // 2]
-        src, dst = dst, src
-        p = 2
-    T = M // 4
-    while p < M:
-        t = np.arange(T)
-        k = t & (p - 1)
-        tw = M // (4 * p)
-        w1, w2 = WM[k * tw], WM[2 * k * tw]
-        if inverse:
-            w1, w2 = np.conj(w1), np.conj(w2)
-        w3 = w1 * w2
-        u0, u1, u2, u3 = src[t], src[t + T] * w1, src[t + 2 * T] * w2, src[t + 3 * T] * w3
-        v0, v1, v2, v3 = u0 + u2, u0 - u2, u1 + u3, (u1 - u3) * (1j if inverse else -1j)
-        j = ((t - k) << 2) + k
-        dst[j], dst[j + p], dst[j + 2 * p], dst[j + 3 * p] = v0 + v2, v1 + v3, v0 - v2, v1 - v3
-        src, dst = dst, src
-        p <<= 2
-    return src
-
-
 @pytest.mark.parametrize("N", [8, 64, 2048, 4096])
-def test_stockham_real_fft_roundtrip(N):
+def test_real_fft_pack_unpack_roundtrip(N):
+    """N-point real transforms as M = N/2-point complex ones: rfft unpack with WN, irfft pack with conj(WN)."""
     rng = np.random.default_rng(N)
     M = N // 2
-    WM = np.exp(-2j * np.pi * np.arange(max(M // 2, 1)) / M)
     WN = np.exp(-2j * np.pi * np.arange(M + 1) / N)
     x = rng.standard_normal(N)
-    Z = stockham(x[0::2] + 1j * x[1::2], WM, False)
+    Z = np.fft.fft(x[0::2] + 1j * x[1::2])
     k = np.arange(M + 1)
     zk, zm = Z[k % M], np.conj(Z[(M - k) % M])
     X = 0.5 * (zk + zm) - 0.5j * WN[k] * (zk - zm)                               # rfft unpack
     assert np.abs(X - np.fft.rfft(x)).max() <= 1e-12 * np.abs(X).max()
     k = np.arange(M)
     yk, ym = X[k], np.conj(X[M - k])
-    zy = stockham((yk + ym) + 1j * np.conj(WN[k]) * (yk - ym), WM, True) / N     # irfft pack
+    zy = np.fft.ifft((yk + ym) + 1j * np.conj(WN[k]) * (yk - ym)) * M / N        # irfft pack
     y = np.empty(N)
     y[0::2], y[1::2] = zy.real, zy.imag
     assert np.abs(y - x).max() <= 1e-12 * np.abs(x).max()

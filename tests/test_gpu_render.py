@@ -108,29 +108,12 @@ def test_errors(em, h):
 
 @pytest.mark.parametrize("n,ch,ln,comp,fft", [(30000, 32, 512, False, 0), (9000, 25, 512, True, 0), (20000, 7, 128, False, 4096),
                                               (5000, 1, 64, True, 4096), (12288, 4, 512, False, 0)])
-@pytest.mark.parametrize("mode", ["2", "3"])
-def test_fused_radix16_route_matches_oracle(em, h, monkeypatch, n, ch, ln, comp, fft, mode):
-    """The register-resident single-kernel route (default for 4096-sample blocks; EMAGLS_RENDER_FUSED=2 / 3: radix-16 x
-    16 x 8 Stockham passes, four channels at a time) against the oracle's convolution, 1e-9 relative as for the cuFFT
-    route; channel counts that are not multiples of four, signals shorter than a block and the compensated delay
-    included."""
-    monkeypatch.setenv("EMAGLS_RENDER_FUSED", mode)
+def test_fused_radix16_route_matches_oracle(em, h, monkeypatch, n, ch, ln, comp, fft):
+    """The register-resident single-kernel route (default for 4096-sample blocks: radix-16 x 16 x 8 Stockham passes,
+    four channels at a time) against the oracle's convolution, 1e-9 relative as for the cuFFT route; channel counts
+    that are not multiples of four, signals shorter than a block and the compensated delay included."""
     if fft:
         monkeypatch.setenv("EMAGLS_RENDER_FFT", str(fft))
-    rng = np.random.default_rng(n)
-    x = rng.standard_normal((n, ch))
-    wL, wR = rng.standard_normal((ln, ch)), rng.standard_normal((ln, ch))
-    y = em.binauralDecode(x, 48000, wL, wR, 48000, comp, handle=h)
-    yo = oracle.binauralDecode(x, 48000, wL, wR, 48000, comp)
-    assert y.shape == yo.shape
-    assert np.abs(y - yo).max() / np.abs(yo).max() < 1e-9
-
-
-@pytest.mark.parametrize("n,ch,ln,comp", [(30000, 32, 512, False), (7000, 25, 256, True), (20000, 8, 128, False)])
-def test_fused_overlap_save_route_matches_oracle(em, h, monkeypatch, n, ch, ln, comp):
-    """The optional single-kernel route (EMAGLS_RENDER_FUSED=1: shared-memory Stockham FFT, multiply-accumulate and
-    inverse transform per overlap-save block) against the oracle's convolution, 1e-9 relative as for the default."""
-    monkeypatch.setenv("EMAGLS_RENDER_FUSED", "1")
     rng = np.random.default_rng(n)
     x = rng.standard_normal((n, ch))
     wL, wR = rng.standard_normal((ln, ch)), rng.standard_normal((ln, ch))

@@ -1,6 +1,6 @@
 #!/bin/bash
-# Round-2 iteration check: parity tests touching the factorisation path, short bench lines (new kernels and the
-# round-1 kernel via EMAGLS_FACTOR_OLD=1), Jacobi sweep statistics.  usage: tools/gpu_r2_iter.sh <tag> [full]
+# Round-2 iteration check: parity tests touching the factorisation path, a short bench line, Jacobi sweep
+# statistics.  usage: tools/gpu_r2_iter.sh <tag> [full]
 cd "$(dirname "$0")/.."
 TAG=${1:-r02_v1}
 mkdir -p gpurun_out
@@ -16,15 +16,6 @@ try:
     print("NEW", j["value"], j["ms_per_step"], j["roofline"].get("class_time_share"), j["roofline"].get("class_ms"))
 except Exception as e:
     print("bench parse failed", e); print(open("gpurun_out/${TAG}_bench.err").read()[-2000:])
-PY
-EMAGLS_FACTOR_OLD=1 timeout 600 python bench.py --steps 3 --warmup 3 --no-render --no-cpu-baseline > gpurun_out/${TAG}_bench_short_old.json 2>> gpurun_out/${TAG}_bench.err
-python - <<PY
-import json
-try:
-    j = json.loads(open("gpurun_out/${TAG}_bench_short_old.json").read().strip().splitlines()[-1])
-    print("OLD", j["value"], j["ms_per_step"], j["roofline"].get("class_time_share"))
-except Exception as e:
-    print("old bench parse failed", e)
 PY
 EMAGLS_DEBUG_INFO=1 timeout 300 python tools/gpu_ncu_factor.py 64 2>&1 | grep "^bin" > gpurun_out/${TAG}_sweeps.txt
 awk 'NR%6==1' gpurun_out/${TAG}_sweeps.txt | head -20

@@ -39,7 +39,7 @@ def run(reps=5):
 
 ref = None
 ffts = [int(v) for v in os.environ.get("AB_FFTS", "0").split(",")]
-for fused, fft in [(f, n_) for n_ in ffts for f in os.environ.get("AB_ROUTES", "0,1,2").split(",")]:
+for fused, fft in [(f, n_) for n_ in ffts for f in os.environ.get("AB_ROUTES", "0,2").split(",")]:
     os.environ["EMAGLS_RENDER_FUSED"] = fused
     if fft:
         os.environ["EMAGLS_RENDER_FFT"] = str(fft)

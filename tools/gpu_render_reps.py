@@ -1,5 +1,5 @@
 """Per-repetition timings of one render route on a device-resident signal (variance check).
-usage (GPU box): EMAGLS_RENDER_FUSED=0|1|2 python tools/gpu_render_reps.py [seconds] [reps]"""
+usage (GPU box): [EMAGLS_RENDER_FUSED=0] python tools/gpu_render_reps.py [seconds] [reps]"""
 import os
 import sys
 
@@ -29,5 +29,5 @@ for i in range(reps + 2):
     torch.cuda.synchronize()
     if i >= 2:
         times.append(a.elapsed_time(b))
-print(f"route {os.environ.get('EMAGLS_RENDER_FUSED', '0')} secs {secs:.0f} x ptr % 2MiB = {x.data_ptr() % (1 << 21)}: "
+print(f"route {os.environ.get('EMAGLS_RENDER_FUSED', 'default')} secs {secs:.0f} x ptr % 2MiB = {x.data_ptr() % (1 << 21)}: "
       + " ".join(f"{t:.2f}" for t in times) + f"  | median {np.median(times):.2f} ms")
