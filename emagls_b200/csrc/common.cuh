@@ -3,6 +3,9 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <math.h>
+#include <map>
+#include <mutex>
+#include <utility>
 
 namespace emagls {
 
@@ -102,5 +105,46 @@ __device__ __forceinline__ void cp_async8(void* smem, const void* gmem, bool pre
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::); }
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N)); }
+
+// ---------------------------------------------------------------- host: per-device launch state
+// Handles on several devices may launch from several host threads at once (include/emagls_cuda.h), so what the
+// launchers remember is kept per device, behind one lock.  The statics of these inline functions are shared by all
+// translation units of the library.
+inline std::mutex& launch_state_mutex() {
+  static std::mutex m;
+  return m;
+}
+
+// Lets `kernel` launch with `bytes` of dynamic shared memory on the current device.  The attribute belongs to one
+// device; it is set when `bytes` exceeds the largest value set so far for this (device, kernel).  Up to 48 KB needs
+// no opt-in.
+inline cudaError_t allow_dynamic_smem(const void* kernel, size_t bytes) {
+  if (bytes <= 48 * 1024) return cudaSuccess;
+  int dev = 0;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e != cudaSuccess) return e;
+  static std::map<std::pair<int, const void*>, size_t> set_to;
+  std::lock_guard<std::mutex> lock(launch_state_mutex());
+  size_t& cur = set_to[{dev, kernel}];
+  if (bytes <= cur) return cudaSuccess;
+  e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+  if (e == cudaSuccess) cur = bytes;
+  return e;
+}
+template <class... Args>
+inline cudaError_t allow_dynamic_smem(void (*kernel)(Args...), size_t bytes) {
+  return allow_dynamic_smem(reinterpret_cast<const void*>(kernel), bytes);
+}
+
+// Number of SMs of the current device.
+inline int sm_count() {
+  int dev = 0;
+  cudaGetDevice(&dev);
+  static std::map<int, int> count;
+  std::lock_guard<std::mutex> lock(launch_state_mutex());
+  int& n = count[dev];
+  if (!n) cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
+  return n;
+}
 
 }  // namespace emagls

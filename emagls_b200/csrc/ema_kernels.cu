@@ -128,12 +128,8 @@ cudaError_t launch_ema_sh_rows(cudaStream_t st, int order, int simN, int M, int 
   size_t smem = (size_t)((nsh * nsh + 1) & ~1) * 8 + (size_t)nsh * nsh * 16 + (size_t)M * nsh * 16 +
                 (size_t)((M * L1 + 1) & ~1) * 8 + (size_t)L1 * nsh * 16;
   if (smem > 200 * 1024) return cudaErrorInvalidValue;
-  static size_t set_to = 0;
-  if (smem > 48 * 1024 && smem > set_to) {
-    cudaError_t e = cudaFuncSetAttribute(ema_sh_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    set_to = smem;
-  }
+  const cudaError_t e = allow_dynamic_smem(ema_sh_rows_kernel, smem);
+  if (e != cudaSuccess) return e;
   ema_sh_rows_kernel<<<D, 256, smem, st>>>(order, simN, M, D, K, complex_basis, azi, zen, dec, Ym, Yhor, bn, At);
   return cudaGetLastError();
 }

@@ -18,6 +18,7 @@
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
+#include <optional>
 #include <string>
 #include <vector>
 #include "engine.h"
@@ -294,8 +295,7 @@ void design_factored(emagls_ctx* h, const emagls_config& cfg, const DesignArgs& 
   const int nLS = kls1 - 1;
 
   Arena ar(st);
-  ProfSpan* setup_span = new ProfSpan(h, EM_PROF_SETUP);
-  struct SpanGuard { ProfSpan*& p; ~SpanGuard() { delete p; p = nullptr; } } setup_guard{setup_span};
+  std::optional<ProfSpan> setup_span(std::in_place, h, EM_PROF_SETUP);
   // ---------------- grid: Y_h = Q R, Gh = Y_h^T Y_h
   double* Yh = ar.get<double>((size_t)S * D);
   double* Q = ar.get<double>((size_t)S * D);
@@ -470,6 +470,14 @@ void design_factored(emagls_ctx* h, const emagls_config& cfg, const DesignArgs& 
   if (const char* e = getenv("EMAGLS_OZAKI_SLICES")) oz_T = atoi(e);
   bool use_oz = true;
   if (const char* e = getenv("EMAGLS_GEMM")) use_oz = std::string(e) != "dmma";
+  // six digits: the FP64 forward functor, the reference of the integer one (launch_oz_fwd)
+  const char* oz_fwd = getenv("EMAGLS_OZ_FWD");
+  const int oz_fwd_raw = oz_fwd && std::string(oz_fwd) == "raw";
+  // Jacobi warm starts where min |r_ii| > warm_grading max |r_ii|.  1e-8 by measurement: the errors of bins 1-15
+  // against exact arithmetic are the same 1e-14 with 1e-4, 1e-6 and 1e-9 (tests/test_gpu_arbitration.py,
+  // profiles/r02_v51_*), the mean sweep count falls from 6.65 to 6.4 (bins 3-18 start warm: 9.2 -> 7.0-8.4 sweeps)
+  const char* wg = getenv("EMAGLS_JACOBI_WARM_GRADING");
+  const double warm_grading = wg ? atof(wg) : 1e-8;
   const int KpS = oz_pad32(S), KpD = oz_pad32(D);
   // longer contractions than the int32 accumulators hold exactly go through the DMMA GEMM instead
   if ((oz_T != 4 && oz_T != 6) || K - kls1 <= 0 || !oz_contraction_fits(KpD, oz_T) || !oz_contraction_fits(KpS, oz_T))
@@ -487,7 +495,7 @@ void design_factored(emagls_ctx* h, const emagls_config& cfg, const DesignArgs& 
     EM_CUDA(launch_row_scale(st, absH, (long long)a.num_sets * 2 * K, D, upH, scH));
     h->launches += 4;
   }
-  delete setup_span; setup_span = nullptr;
+  setup_span.reset();
 
   // ---------------- memory plan: orientation chunks of OC, Gram bin groups of NB, TSQR slots of G
   const int ne = Mc * (Mc + 1) / 2, ne_ld = (ne + 1) & ~1;
@@ -641,7 +649,7 @@ void design_factored(emagls_ctx* h, const emagls_config& cfg, const DesignArgs& 
             }
             {
               ProfSpan ps(h, EM_PROF_JACOBI);
-              EM_CUDA(launch_svdclip(st, Mc, Rbuf, ops, oc, Gn, cfg.svd_regul, try_fast));
+              EM_CUDA(launch_svdclip(st, Mc, Rbuf, ops, oc, Gn, cfg.svd_regul, try_fast, warm_grading));
             }
             h->launches += 2;
           } else {
@@ -687,7 +695,7 @@ void design_factored(emagls_ctx* h, const emagls_config& cfg, const DesignArgs& 
               ProfSpan ps(h, EM_PROF_GEMM_FWD);   // exactly one launch: the int8 tensor-core GEMM
               OzFwdArgs fa{YhA_q, sYhA, D, KpS, Cv_q, sCv, 4 * pj, oz_T, Tt_q, KpD, sTt,
                            absH + (size_t)kb * D, 2LL * K * D, (long long)K * D, upH + kb, scH + kb, K, oc,
-                           kb == K - 1 ? 1 : 0};
+                           kb == K - 1 ? 1 : 0, oz_fwd_raw};
               EM_CUDA(launch_oz_fwd(st, fa));
             }
             {

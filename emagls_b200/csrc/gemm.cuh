@@ -223,13 +223,9 @@ inline int gemm_pick_splits(int tiles, int K, int ctas_per_sm, int max_splits) {
 template <class Cfg, class Epi, bool AKC, bool BKC, bool VEC>
 inline cudaError_t launch_gemm_inst(cudaStream_t st, GemmOperand A, GemmOperand B, GemmShape sh, Epi epi, dim3 grid,
                                     int ksplit) {
-  static bool attr_set = false;
   auto kern = gemm_f64_kernel<Cfg, Epi, AKC, BKC, VEC>;
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::SMEM);
-    if (e != cudaSuccess) return e;
-    attr_set = true;
-  }
+  const cudaError_t e = allow_dynamic_smem(kern, Cfg::SMEM);
+  if (e != cudaSuccess) return e;
   kern<<<grid, GM_THREADS, Cfg::SMEM, st>>>(A, B, sh, ksplit, epi);
   return cudaGetLastError();
 }

@@ -17,6 +17,7 @@
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
+#include <optional>
 #include <vector>
 #include "engine.h"
 #include "gemm.cuh"
@@ -255,11 +256,7 @@ static void run_generic(emagls_ctx* h, Arena& ar, const GenericProblem& g) {
     // one "problem", num_ops bin slots: operator index = slot
     EM_CUDA(launch_factor(st, bp, src, ops, 1, 0, g.num_ops, g.regul, 1));
     const size_t smem = (size_t)2 * g.D * sizeof(cplx);
-    static size_t set_to = 0;
-    if (smem > 48 * 1024 && smem > set_to) {
-      EM_CUDA(cudaFuncSetAttribute(form_q_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      set_to = smem;
-    }
+    EM_CUDA(allow_dynamic_smem(form_q_kernel, smem));
     dim3 grid((g.Mc + 1) / 2, g.num_ops);
     form_q_kernel<<<grid, 32, smem, st>>>(bp, ops, QcT);
     EM_CUDA(cudaGetLastError());
@@ -277,11 +274,7 @@ static void run_generic(emagls_ctx* h, Arena& ar, const GenericProblem& g) {
     c.D = g.D; c.Mc = g.Mc; c.K = g.K; c.first_bin = g.first_bin; c.kls1 = g.kls1; c.dc_fix = g.dc_fix;
     c.nyquist_real = g.nyquist_real;
     const size_t smem = ((size_t)g.D + 2 * g.Mc) * sizeof(cplx);
-    static size_t set_to = 0;
-    if (smem > 48 * 1024 && smem > set_to) {
-      EM_CUDA(cudaFuncSetAttribute(generic_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      set_to = smem;
-    }
+    EM_CUDA(allow_dynamic_smem(generic_chain_kernel, smem));
     generic_chain_kernel<<<g.num_prob * 2, 1024, smem, st>>>(c);
     EM_CUDA(cudaGetLastError());
     h->launches += 1;
@@ -320,8 +313,7 @@ void design_magls(emagls_ctx* h, const emagls_config& cfg, const double* hL, con
   EM_REQUIRE(D >= Mc, "fewer directions than harmonics");
   const bool cplx_out = cfg.basis == EMAGLS_BASIS_COMPLEX;
   Arena ar(st);
-  ProfSpan* setup_span = new ProfSpan(h, EM_PROF_SETUP);
-  struct SetupSpanGuard { ProfSpan*& p; ~SetupSpanGuard() { delete p; p = nullptr; } } setup_span_guard{setup_span};   // also on a thrown Fail
+  std::optional<ProfSpan> setup_span(std::in_place, h, EM_PROF_SETUP);
   // Y_conj.' rows in the real basis; a complex basis is a unitary change of the output (engine.cu)
   cplx* At = ar.get<cplx>((size_t)D * Mc);
   if (harmonics_kind == 1) {
@@ -346,7 +338,7 @@ void design_magls(emagls_ctx* h, const emagls_config& cfg, const double* hL, con
       EM_CUDA(cudaGetLastError());
     }
     h->launches += 2;
-    delete setup_span; setup_span = nullptr;
+    setup_span.reset();
     cplx* W = ar.get<cplx>((size_t)2 * Mc * T);
     g.K = T; g.first_bin = 0; g.kls1 = T; g.dc_fix = 0; g.nyquist_real = 0;
     g.H = Hc; g.h_prob_stride = 0; g.h_ear_stride = (long long)T * D; g.W = W;
@@ -392,7 +384,7 @@ void design_magls(emagls_ctx* h, const emagls_config& cfg, const double* hL, con
       }
     h->launches += 1;
   }
-  delete setup_span; setup_span = nullptr;
+  setup_span.reset();
   cplx* Wsp = spectra ? reinterpret_cast<cplx*>(spectra) : ar.get<cplx>((size_t)2 * NS * Mc * K);
   g.K = K; g.first_bin = 0; g.kls1 = kls1; g.dc_fix = 0; g.nyquist_real = 1;   // lib/getMagLsFilters.m:64-72
   g.num_prob = NS;
@@ -460,8 +452,7 @@ void design_from_atf(emagls_ctx* h, const emagls_config& cfg, const double* hL, 
   const int Dn = std::min(D, Da);
   EM_REQUIRE(Dn >= M, "fewer directions than microphones");
   Arena ar(st);
-  ProfSpan* setup_span = new ProfSpan(h, EM_PROF_SETUP);
-  struct SetupSpanGuard { ProfSpan*& p; ~SetupSpanGuard() { delete p; p = nullptr; } } setup_span_guard{setup_span};   // also on a thrown Fail
+  std::optional<ProfSpan> setup_span(std::in_place, h, EM_PROF_SETUP);
   // ---- grid matching (:56-96), all orientations at once
   double* hx = ar.get<double>((size_t)3 * D);
   double* ax = ar.get<double>((size_t)3 * Da);
@@ -511,7 +502,7 @@ void design_from_atf(emagls_ctx* h, const emagls_config& cfg, const double* hL, 
       mean_dev_deg[b] = acc / (double)Dn;
     }
   }
-  delete setup_span; setup_span = nullptr;
+  setup_span.reset();
   cplx* Wsp = spectra ? reinterpret_cast<cplx*>(spectra) : ar.get<cplx>((size_t)2 * B * M * K);
   EM_CUDA(cudaMemsetAsync(Wsp, 0, (size_t)2 * B * M * K * sizeof(cplx), st));
   GenericProblem g{};
@@ -581,8 +572,7 @@ void design_ema_sh(emagls_ctx* h, const emagls_config& cfg, const double* hL, co
   EM_REQUIRE(D >= nsh, "fewer directions than harmonics");
   const bool cplx_out = cfg.basis == EMAGLS_BASIS_COMPLEX;
   Arena ar(st);
-  ProfSpan* setup_span = new ProfSpan(h, EM_PROF_SETUP);
-  struct SetupSpanGuard { ProfSpan*& p; ~SetupSpanGuard() { delete p; p = nullptr; } } setup_span_guard{setup_span};   // also on a thrown Fail
+  std::optional<ProfSpan> setup_span(std::in_place, h, EM_PROF_SETUP);
   // ---- array model pieces
   std::vector<double> kr(K);
   for (int k = 0; k < K; ++k) kr[k] = 2.0 * M_PI * ((double)k * df) / cfg.speed_of_sound * mic_radius;
@@ -632,7 +622,7 @@ void design_ema_sh(emagls_ctx* h, const emagls_config& cfg, const double* hL, co
     }
     h->launches += 3;
   }
-  delete setup_span; setup_span = nullptr;
+  setup_span.reset();
   cplx* Wsp = spectra ? reinterpret_cast<cplx*>(spectra) : ar.get<cplx>((size_t)2 * nsh * K);
   EM_CUDA(cudaMemsetAsync(Wsp, 0, (size_t)2 * nsh * K * sizeof(cplx), st));
   GenericProblem g{};

@@ -77,12 +77,8 @@ cudaError_t launch_build_F(cudaStream_t st, const double* Gh, int S, int N, cons
                            int P, int ne_ld, double* Fs, double* Fa) {
   const int wmax = 2 * N + 1;
   size_t smem = ((size_t)2 * Mc * wmax + (size_t)wmax * Mc + (size_t)Mc * (Mc + 1)) * sizeof(double);
-  static size_t set_to = 0;
-  if (smem > 48 * 1024 && smem > set_to) {
-    cudaError_t e = cudaFuncSetAttribute(build_F_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    set_to = smem;
-  }
+  const cudaError_t e = allow_dynamic_smem(build_F_kernel, smem);
+  if (e != cudaSuccess) return e;
   dim3 grid((N + 1) * (N + 2) / 2, P);
   build_F_kernel<<<grid, 256, smem, st>>>(Gh, S, Y, Mc, P, ne_ld, Fs, Fa);
   return cudaGetLastError();
@@ -324,12 +320,8 @@ cudaError_t launch_gram_chol(cudaStream_t st, const double* Gre, const double* G
   int wpc = GC_WPC;
   while (wpc > 1 && per_warp * wpc > 227 * 1024) --wpc;
   size_t smem = per_warp * wpc;
-  static size_t set_to = 0;
-  if (smem > 48 * 1024 && smem > set_to) {
-    cudaError_t e = cudaFuncSetAttribute(gram_chol_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    set_to = smem;
-  }
+  const cudaError_t e = allow_dynamic_smem(gram_chol_kernel, smem);
+  if (e != cudaSuccess) return e;
   gram_chol_kernel<<<(unsigned)((nmat + wpc - 1) / wpc), wpc * 32, smem, st>>>(Gre, Gim, Mc, P, ne_ld, nmat, thr,
                                                                                     Pb, fail);
   return cudaGetLastError();
@@ -871,12 +863,8 @@ static cudaError_t launch_bwd_fused_t(cudaStream_t st, size_t smem, int num_prob
                                       long long z_set_stride, long long z_ear_stride, int z_shared, int nsplit,
                                       long long split_stride, cplx* Wsp, long long w_ear_stride, int K, int k, int dc_fix,
                                       FwdFuse ff, int N) {
-  static size_t set_to = 0;
-  if (smem > set_to) {
-    cudaError_t e = cudaFuncSetAttribute(bwd_fused_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    set_to = smem;
-  }
+  const cudaError_t e = allow_dynamic_smem(bwd_fused_kernel<T>, smem);
+  if (e != cudaSuccess) return e;
   bwd_fused_kernel<T><<<num_prob, BF_WARPS * 32, smem, st>>>(Y, Mc, S, roword, bk, Pb, pm, z, z_set_stride, z_ear_stride,
                                                               z_shared, nsplit, split_stride, Wsp, w_ear_stride, K, k, dc_fix, ff, N);
   return cudaGetLastError();
@@ -888,12 +876,8 @@ static cudaError_t launch_bwd_small_t(cudaStream_t st, size_t smem, int num_prob
                                       long long z_set_stride, long long z_ear_stride, int z_shared, int nsplit,
                                       long long split_stride, cplx* Wsp, long long w_ear_stride, int K, int k, int dc_fix,
                                       FwdFuse ff) {
-  static size_t set_to = 0;
-  if (smem > 48 * 1024 && smem > set_to) {
-    cudaError_t e = cudaFuncSetAttribute(bwd_small_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    set_to = smem;
-  }
+  const cudaError_t e = allow_dynamic_smem(bwd_small_kernel<T>, smem);
+  if (e != cudaSuccess) return e;
   bwd_small_kernel<T><<<num_prob, 256, smem, st>>>(Y, Mc, S, roword, bk, Pb, pm, z, z_set_stride, z_ear_stride, z_shared,
                                                   nsplit, split_stride, Wsp, w_ear_stride, K, k, dc_fix, ff);
   return cudaGetLastError();

@@ -94,7 +94,7 @@ BlockPlan make_block_plan_sep(int S, int Mc);
 cudaError_t launch_tsqr_sep(cudaStream_t st, const BlockPlan& bp, const RowSource& src, const OperatorSet& ops,
                             cplx* Rout, int num_prob, int kbase, int G);
 cudaError_t launch_svdclip(cudaStream_t st, int Mc, const cplx* Rin, const OperatorSet& ops, int num_prob, int G,
-                           double regul, int try_fast);
+                           double regul, int try_fast, double warm_grading);
 cudaError_t launch_chain_bwd_sep(cudaStream_t st, const BlockPlan& bp, const OperatorSet& ops, int slot, int G,
                                  const double* tq, long long tq_set_stride, long long tq_ear_stride, int tq_shared,
                                  int nsplit, long long split_stride, ProbMap pm, cplx* Wsp, long long w_ear_stride,
@@ -160,6 +160,8 @@ struct OzFwdArgs {
   const double* absH; long long abs_set_stride, abs_ear_stride;
   const double* up; const double* sc; int scale_stride;  // this bin's |H| scales, indexed (set*2+ear)*scale_stride
   int orient_per_set, nyquist;
+  int raw;   // six digits: the FP64 functor instead of the integer one (EMAGLS_OZ_FWD=raw)
+  int dbg;   // GemmArgs::dbg (tools/microbench/oz_fwd_bench.cu)
 };
 cudaError_t launch_oz_fwd(cudaStream_t st, const OzFwdArgs& a);
 // tq [rows][S] = t^T B with B_q [T][S][KpD] (rows = harmonics, K = directions)

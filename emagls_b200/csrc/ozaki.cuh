@@ -22,6 +22,7 @@
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include "common.cuh"
 
 namespace emagls {
 namespace oz {
@@ -498,15 +499,14 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
 inline EncodeTiledFn encode_tiled_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
+  static const EncodeTiledFn fn = [] {
     void* p = nullptr;
     cudaDriverEntryPointQueryResult qres;
     if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) != cudaSuccess ||
         qres != cudaDriverEntryPointSuccess)
-      return nullptr;
-    fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
+      return EncodeTiledFn(nullptr);
+    return reinterpret_cast<EncodeTiledFn>(p);
+  }();
   return fn;
 }
 
@@ -544,7 +544,7 @@ cudaError_t launch_ozaki_gemm_t(cudaStream_t st, const CUtensorMap& tmA, const C
                                 Epi epi, int num_sms) {
   static_assert(T * Cfg::NT <= 512 && Cfg::NT % 16 == 0, "TMEM holds 512 columns; UMMA N is a multiple of 16");
   const size_t smem = gemm_smem_bytes<Cfg>(T);
-  cudaError_t e = cudaFuncSetAttribute(ozaki_gemm_kernel<T, Epi, Cfg>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  const cudaError_t e = allow_dynamic_smem(ozaki_gemm_kernel<T, Epi, Cfg>, smem);
   if (e != cudaSuccess) return e;
   g.tile_n = Cfg::NT;
   const int tiles = ((g.M + TILE_M - 1) / TILE_M) * ((g.N + Cfg::NT - 1) / Cfg::NT);

@@ -3,8 +3,6 @@
 //             continuation t = |H_k| y / |y| (lib/getEMagLs2Filters.m:95-103) fused into the epilogue,
 //             which also slices t into the int8 digits the backward product consumes;
 //   backward: t^T Y_h (or t^T Q)  (4P x S, contraction over the D directions), FP64 out.
-#include <cstdlib>
-#include <string>
 #include "kernels.h"
 #include "ozaki.cuh"
 #include "phase_fixed.cuh"
@@ -206,16 +204,6 @@ __global__ void row_scale_kernel(const double* __restrict__ x, long long rows, i
   if (lane == 0) { up[r] = scalbn(1.0, 6 - e); sc[r] = scalbn(1.0, e - 6); }
 }
 
-int sm_count() {
-  static int n = 0;
-  if (!n) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-  }
-  return n;
-}
-
 }  // namespace
 
 int oz_pad32(int k) { return (k + 31) & ~31; }
@@ -237,15 +225,13 @@ cudaError_t launch_row_scale(cudaStream_t st, const double* x, long long rows, i
   return cudaGetLastError();
 }
 
-int oz_fwd_debug = 0;   // GemmArgs::dbg of the forward launches (tools/microbench/oz_fwd_bench.cu)
-
 template <int T, class Epi, class Cfg = oz::TileDefault>
 static cudaError_t oz_fwd_t(cudaStream_t st, const OzFwdArgs& a) {
   CUtensorMap tmA, tmB;
   if (!oz::make_operand_map(&tmA, a.YhA_q, a.D, a.KpS, T, oz::TILE_M) ||
       !oz::make_operand_map(&tmB, a.Cv_q, a.rows, a.KpS, T, Cfg::NT))
     return cudaErrorInvalidValue;
-  oz::GemmArgs g{a.D, a.rows, a.KpS, a.sYhA, a.sCv, oz_fwd_debug, 0, Cfg::NT};   // m fastest: the 42 MB of Cv digits are the shared operand
+  oz::GemmArgs g{a.D, a.rows, a.KpS, a.sYhA, a.sCv, a.dbg, 0, Cfg::NT};   // m fastest: the 42 MB of Cv digits are the shared operand
   Epi epi{a.Tt_q, (long long)a.rows * a.KpD, a.KpD, a.sT, a.absH, a.abs_set_stride, a.abs_ear_stride,
           a.up, a.sc, a.scale_stride, a.orient_per_set, a.nyquist, a.sCv};
   return oz::launch_ozaki_gemm_t<T, Epi, Cfg>(st, tmA, tmB, g, epi, sm_count());
@@ -257,15 +243,11 @@ cudaError_t launch_oz_fwd(cudaStream_t st, const OzFwdArgs& a) {
   // work does not; 0.34 against 0.425 ms per launch, profiles/r02_v40_fwd_fix.txt) on 128 x 80 tiles when that takes
   // fewer rounds of tiles.  With four digits the MMAs of a tile are too short to hide the longer integer functor, so
   // the FP64 functor on the raw accumulators stays (0.076 against 0.078 ms).
-  // EMAGLS_OZ_FWD=raw runs that FP64 functor for six digits too: the reference the integer functor is tested against
-  // (it may differ from it by one unit of the last digit, phase_fixed.cuh).
-  static const bool raw = [] {
-    const char* e = getenv("EMAGLS_OZ_FWD");
-    return e && std::string(e) == "raw";
-  }();
+  // a.raw runs that FP64 functor for six digits too: the reference the integer functor is tested against (it may
+  // differ from it by one unit of the last digit, phase_fixed.cuh).
   if (a.T == 4) return oz_fwd_t<4, EpiPhaseSliceRaw<4>>(st, a);
   if (a.T != 6) return cudaErrorInvalidValue;
-  if (raw) return oz_fwd_t<6, EpiPhaseSliceRaw<6>>(st, a);
+  if (a.raw) return oz_fwd_t<6, EpiPhaseSliceRaw<6>>(st, a);
   if (a.rows & 3) return cudaErrorInvalidValue;   // the integer functor's 4-byte stores span four rows
   // Contractions over more than 2016 harmonics (simulation order 44 and up) may carry |y| beyond the range of the
   // integer functor's 64-bit drain: the FP64 functor rounds once instead of wrapping.

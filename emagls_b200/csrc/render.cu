@@ -533,11 +533,7 @@ void binaural_decode_dev(emagls_ctx* h, const double* in, long long num_samples,
     render_twiddle_kernel<<<(FR_M + 1 + 255) / 256, 256, 0, st>>>(FR_M, WN);
     EM_CUDA(cudaGetLastError());
     const size_t smem = ((size_t)4 * FR_LD + 2 * (FR_M + 1)) * sizeof(cplx);
-    static bool attr_set = false;
-    if (!attr_set) {
-      EM_CUDA(cudaFuncSetAttribute(fused_render16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      attr_set = true;
-    }
+    EM_CUDA(allow_dynamic_smem(fused_render16_kernel, smem));
     {
       ProfSpan ps(h, EM_PROF_RENDER_MAC);
       fused_render16_kernel<<<(unsigned)nblk_total, FR_T, smem, st>>>(in, num_samples, num_ch, Hw, TW, WN, L, ov, skip,

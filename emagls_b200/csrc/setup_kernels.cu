@@ -199,14 +199,9 @@ cudaError_t launch_householder_qr(cudaStream_t st, double* A, int D, int S, doub
   double* tau = work + (long long)D * S;
   double* rdiag = tau + S;
   size_t smem = (size_t)(D + 8) * sizeof(double);
-  static size_t set_to = 0;
-  if (smem > 48 * 1024 && smem > set_to) {
-    cudaError_t e = cudaFuncSetAttribute(hh_factor_step, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(hh_formq_step, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    set_to = smem;
-  }
+  cudaError_t e = allow_dynamic_smem(hh_factor_step, smem);
+  if (e == cudaSuccess) e = allow_dynamic_smem(hh_formq_step, smem);
+  if (e != cudaSuccess) return e;
   long long n = 0;
   for (int j = 0; j < S; ++j) {
     int trailing = S - 1 - j;
@@ -337,23 +332,15 @@ cudaError_t launch_chol_upper(cudaStream_t st, double* G, int S, int* flag) {
   if (S > 1024) return cudaErrorInvalidValue;
   const size_t smem = (size_t)(2 * CH_PB + (size_t)CH_PB * S) * sizeof(double);
   if (smem > 200 * 1024) return cudaErrorInvalidValue;
-  static size_t set_to = 0;
-  if (smem > 48 * 1024 && smem > set_to) {
-    cudaError_t e = cudaFuncSetAttribute(chol_upper_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    set_to = smem;
-  }
+  const cudaError_t e = allow_dynamic_smem(chol_upper_kernel, smem);
+  if (e != cudaSuccess) return e;
   chol_upper_kernel<<<1, 1024, smem, st>>>(G, S, flag);
   return cudaGetLastError();
 }
 cudaError_t launch_tri_inverse(cudaStream_t st, const double* R, int S, double* Rinv) {
   const size_t smem = (size_t)TI_WARPS * S * sizeof(double);
-  static size_t set_to = 0;
-  if (smem > 48 * 1024 && smem > set_to) {
-    cudaError_t e = cudaFuncSetAttribute(tri_inverse_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    set_to = smem;
-  }
+  const cudaError_t e = allow_dynamic_smem(tri_inverse_kernel, smem);
+  if (e != cudaSuccess) return e;
   tri_inverse_kernel<<<(S + TI_WARPS - 1) / TI_WARPS, TI_WARPS * 32, smem, st>>>(R, S, Rinv);
   return cudaGetLastError();
 }

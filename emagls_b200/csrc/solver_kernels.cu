@@ -399,20 +399,12 @@ cudaError_t launch_factor(cudaStream_t st, const BlockPlan& bp, const RowSource&
   size_t smem = factor_smem_bytes(bp);
   cudaError_t e;
   if (bp.MC == 32) {
-    static bool set32 = false;
-    if (!set32) {
-      e = cudaFuncSetAttribute(factor_kernel<32, 96>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      if (e != cudaSuccess) return e;
-      set32 = true;
-    }
+    e = allow_dynamic_smem(factor_kernel<32, 96>, smem);
+    if (e != cudaSuccess) return e;
     factor_kernel<32, 96><<<num_prob * G, FT, smem, st>>>(bp, src, ops, kbase, G, regul, try_fast);
   } else {
-    static bool set64 = false;
-    if (!set64) {
-      e = cudaFuncSetAttribute(factor_kernel<64, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      if (e != cudaSuccess) return e;
-      set64 = true;
-    }
+    e = allow_dynamic_smem(factor_kernel<64, 128>, smem);
+    if (e != cudaSuccess) return e;
     factor_kernel<64, 128><<<num_prob * G, FT, smem, st>>>(bp, src, ops, kbase, G, regul, try_fast);
   }
   return cudaGetLastError();
@@ -485,12 +477,8 @@ cudaError_t launch_chain_bwd(cudaStream_t st, const BlockPlan& bp, const Operato
                              int num_prob) {
   int w = chain_warps(bp.S);
   size_t smem = (size_t)w * 2 * bp.S * sizeof(cplx);
-  static size_t set_to = 0;
-  if (smem > 48 * 1024 && smem > set_to) {
-    cudaError_t e = cudaFuncSetAttribute(chain_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    set_to = smem;
-  }
+  const cudaError_t e = allow_dynamic_smem(chain_bwd_kernel, smem);
+  if (e != cudaSuccess) return e;
   chain_bwd_kernel<<<(num_prob + w - 1) / w, w * 32, smem, st>>>(bp, ops, slot, G, tq, tq_set_stride, tq_ear_stride, tq_shared,
                                                                  nsplit, split_stride, pm, Wsp, w_ear_stride, K, k, dc_fix,
                                                                  num_prob);

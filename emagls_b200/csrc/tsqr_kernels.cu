@@ -25,7 +25,6 @@
 // tile; entry (r, c) is the tail of reflector c of block r/32, scaled so that v = [1; tail] with the 1
 // at R-space row c), tau [nblk][32].
 #include <algorithm>
-#include <cstdlib>
 #include "kernels.h"
 #include "reflect.cuh"
 
@@ -700,36 +699,22 @@ cudaError_t launch_tsqr_sep(cudaStream_t st, const BlockPlan& bp, const RowSourc
                             cplx* Rout, int num_prob, int kbase, int G) {
   if (!bp.sep || bp.Mc > 32 || src.E == nullptr || src.N + 1 > TQ_BN) return cudaErrorInvalidValue;
   const size_t smem = tsqr_sep_smem_bytes(bp);
-  static size_t set_to = 0;
-  if (smem > 48 * 1024 && smem > set_to) {
-    cudaError_t e = cudaFuncSetAttribute(tsqr_sep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    set_to = smem;
-  }
+  const cudaError_t e = allow_dynamic_smem(tsqr_sep_kernel, smem);
+  if (e != cudaSuccess) return e;
   const int sgroups = (G + TQ_WARPS - 1) / TQ_WARPS;
   tsqr_sep_kernel<<<num_prob * sgroups, TQ_WARPS * 32, smem, st>>>(bp, src, ops, Rout, kbase, G, sgroups);
   return cudaGetLastError();
 }
 
-static int sv_sm_count() {
-  static int n = 0;
-  if (!n) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-  }
-  return n;
-}
-
 cudaError_t launch_svdclip(cudaStream_t st, int Mc, const cplx* Rin, const OperatorSet& ops, int num_prob, int G,
-                           double regul, int try_fast) {
+                           double regul, int try_fast, double warm_grading) {
   if (Mc > 32) return cudaErrorInvalidValue;
   const size_t smem = (size_t)2 * 1024 * sizeof(cplx) + (size_t)(32 + 32 + 20) * sizeof(double);
   // Tail of the grid: CTAs take about equally long, so with `resident` CTAs in flight a launch lasts
   // ceil(num_prob / resident) rounds and the last round may be almost empty (3600 orientations on 592 places: 6.08
   // -> 7 rounds).  The orientations of that remainder are cut into bin ranges, as many as fit into one round, so
   // the last round lasts 1 / pieces of a full one (plus one cold Jacobi start per piece).
-  const int resident = SV_CTAS * sv_sm_count();
+  const int resident = SV_CTAS * sm_count();
   int split_from = num_prob, pieces = 1;
   const int rem = num_prob % resident;
   if (num_prob > resident && rem > 0 && G > 1) {
@@ -737,10 +722,6 @@ cudaError_t launch_svdclip(cudaStream_t st, int Mc, const cplx* Rin, const Opera
     if (pieces > 1) split_from = num_prob - rem; else pieces = 1;
   }
   const int grid = split_from + (num_prob - split_from) * pieces;
-  // warm starts where min |r_ii| > warm_grading max |r_ii| (EMAGLS_JACOBI_WARM_GRADING).  1e-8 by measurement: the
-  // errors of bins 1-15 against exact arithmetic are the same 1e-14 with 1e-4, 1e-6 and 1e-9 (tests/test_gpu_arbitration.py,
-  // profiles/r02_v51_*), the mean sweep count falls from 6.65 to 6.4 (bins 3-18 start warm: 9.2 -> 7.0-8.4 sweeps)
-  static const double warm_grading = [] { const char* e = getenv("EMAGLS_JACOBI_WARM_GRADING"); return e ? atof(e) : 1e-8; }();
   svdclip_kernel<<<grid, SV_T, smem, st>>>(Mc, Rin, ops, G, regul, try_fast, split_from, pieces, warm_grading);
   return cudaGetLastError();
 }

@@ -63,7 +63,8 @@ typedef struct {
 /* A handle owns one CUDA stream and one private stream-ordered memory pool on `device` (scratch stays cached in
  * it between calls and is returned to the device by emagls_destroy; the device's default pool is not touched).
  * A handle is NOT thread-safe: calls on one handle must not overlap (error text, plans and profiler state are per
- * handle).  Different handles may be used from different host threads concurrently.                          */
+ * handle).  Different handles may be used from different host threads concurrently.  Handles on different devices
+ * may coexist in one process.                                                                                  */
 int emagls_create(int device, emagls_handle* out);
 int emagls_destroy(emagls_handle h);
 const char* emagls_last_error(emagls_handle h);

@@ -259,37 +259,16 @@ def test_optional_fp32_contraction_path(em, h, c1, oracle_c1):
     assert 0 < d < 1e-5, d
 
 
-_FWD_VARIANT_SNIPPET = r"""
-import sys, numpy as np
-sys.path.insert(0, {root!r})
-import emagls_b200 as em
-from emagls_b200 import synth
-g = synth.load_grids()
-az, ze = g["hrirGridAziRad"][::3], g["hrirGridZenRad"][::3]
-hL, hR = synth.synth_hrirs(az, ze, taps=64, delay=20)
-R = np.stack([np.eye(3), synth.rotation_yaw_pitch(40.0, 10.0), synth.rotation_yaw_pitch(-75.0, -20.0)])
-wL, wR = em.getEMagLs2Filters(hL, hR, az, ze, g["micRadius"], g["micGridAziRad"], g["micGridZenRad"], 4, g["fs"], 128,
-                              rotations=R, handle=em.Handle(0))
-np.savez({out!r}, wL=wL, wR=wR)
-"""
-
-
-def test_forward_functor_variants_agree(tmp_path):
+def test_forward_functor_variants_agree(em, h, grids, monkeypatch):
     """The forward tensor-core product's two epilogue functors for six digits must give the same filters
     (lib/getEMagLs2Filters.m:95-103, t = |H_k| y / |y|): the FP64-free one (default) and the FP64 one it is checked
-    against (EMAGLS_OZ_FWD=raw: may differ by one unit of the last base-256 digit, 2^-46 of a row maximum).  The switch
-    is read once per process, hence the subprocesses."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    res = {}
-    for name, env in (("default", {}), ("raw", {"EMAGLS_OZ_FWD": "raw"})):
-        out = str(tmp_path / f"{name}.npz")
-        e = dict(os.environ)
-        e.update(env)
-        subprocess.run([sys.executable, "-c", _FWD_VARIANT_SNIPPET.format(root=root, out=out)], check=True, env=e,
-                       timeout=600)
-        res[name] = np.load(out)
-    for k in ("wL", "wR"):
-        assert rel(res["default"][k], res["raw"][k]) <= 2e-10, (k, rel(res["default"][k], res["raw"][k]))
+    against (EMAGLS_OZ_FWD=raw: may differ by one unit of the last base-256 digit, 2^-46 of a row maximum)."""
+    az, ze = grids["hrirGridAziRad"][::3], grids["hrirGridZenRad"][::3]
+    hL, hR = synth.synth_hrirs(az, ze, taps=64, delay=20)
+    R = np.stack([np.eye(3), synth.rotation_yaw_pitch(40.0, 10.0), synth.rotation_yaw_pitch(-75.0, -20.0)])
+    args = (az, ze, grids["micRadius"], grids["micGridAziRad"], grids["micGridZenRad"], 4, grids["fs"], 128)
+    default = em.getEMagLs2Filters(hL, hR, *args, rotations=R, handle=h)
+    monkeypatch.setenv("EMAGLS_OZ_FWD", "raw")
+    raw = em.getEMagLs2Filters(hL, hR, *args, rotations=R, handle=h)
+    for k, a, b in zip(("wL", "wR"), default, raw):
+        assert rel(a, b) <= 2e-10, (k, rel(a, b))

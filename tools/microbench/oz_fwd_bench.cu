@@ -150,7 +150,7 @@ int main(int argc, char** argv) {
       }
     }
     for (int dbg : {1, 4}) {   // decomposition: 1 no epilogue, 2 no MMAs, 3 operand ring only, 4 drain only, 6 drain only without MMAs
-      oz_fwd_debug = dbg;
+      fa.dbg = dbg;
       CK(run(mode));
       CK(cudaEventRecord(e0));
       for (int i = 0; i < reps; ++i) CK(run(mode));
@@ -160,7 +160,7 @@ int main(int argc, char** argv) {
       CK(cudaEventElapsedTime(&msd, e0, e1));
       printf("   %-9s dbg=%d: %.4f ms\n", names[mode], dbg, msd / reps);
     }
-    oz_fwd_debug = 0;
+    fa.dbg = 0;
     for (int i = 0; i < 3; ++i) CK(run(mode));
     CK(cudaEventRecord(e0));
     for (int i = 0; i < reps; ++i) CK(run(mode));
