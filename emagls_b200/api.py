@@ -23,7 +23,7 @@ from ._lib import Config, EmaglsError, Handle, RadialParams, default_handle  # n
 
 __all__ = ["getEMagLs2Filters", "getEMagLsFilters", "getMagLsFilters", "getLsFilters",
            "getEMagLsFiltersFromAtf", "getEMagLsFiltersEMAinCH", "getEMagLsFiltersEMAinSH",
-           "getSMAIRMatrix", "binauralDecode", "binauralDecodeTracked", "getSH", "sphModalCoeffs", "regularizedApply", "grpdelay",
+           "getSMAIRMatrix", "binauralDecode", "binauralDecodeTracked", "binauralDecodeShTracked", "getSH", "sphModalCoeffs", "regularizedApply", "grpdelay",
            "getRadialFilter", "applyRadialFilter", "encodeSH", "encodeCH", "rotateSH", "getMagLsFilters2D",
            "getMagLsSphericalHeadFilter", "getMagLsArrayDiffuseFilter", "Handle", "EmaglsError"]
 
@@ -467,6 +467,39 @@ def binauralDecodeTracked(inp, wL, wR, track, hop, fade=None, compensateDelay=Fa
     xi, wli, wri = np.imag(x), np.imag(wL), np.imag(wR)
     if np.any(xi) and (np.any(wli) or np.any(wri)):
         out -= dec(xi, wli, wri)
+    return out
+
+
+def binauralDecodeShTracked(inp, wL, wR, rotations, hop, fade=None, compensateDelay=False, *, firstSample=0,
+                            handle=None):
+    """Head-tracked binauralDecode of a real SH signal by sound-field rotation (not in the reference API;
+    emagls_binaural_decode_sh_tracked): ``inp`` [samples, (order+1)^2] in the real basis is rotated per sample by
+    M = (1 - g) Q_a + g Q_c, Q_f = getSHrotMtx(rotations[f], order, 'real'), and rendered with the one filter pair
+    ``wL``, ``wR`` [len, (order+1)^2].  ``rotations`` [frames, 3, 3] is the head orientation of every frame of ``hop``
+    samples (the designers' convention: the world direction of head-frame direction u is R u); frame timing, ``fade``
+    (default ``hop``), ``compensateDelay`` and ``firstSample`` as in binauralDecodeTracked."""
+    h = handle or default_handle()
+    if np.iscomplexobj(inp) or np.iscomplexobj(wL) or np.iscomplexobj(wR):
+        raise NotImplementedError("binauralDecodeShTracked: the sound-field rotation takes real-basis SH signals")
+    x, wl, wr = _f(inp), _f(wL), _f(wR)
+    if x.ndim != 2:
+        raise ValueError("inp must be [samples, (order+1)^2]")
+    n, ch = x.shape
+    N = int(round(np.sqrt(ch))) - 1
+    if N < 0 or (N + 1) ** 2 != ch:
+        raise ValueError("the channel count of inp is not a square (order+1)^2")
+    if wl.shape != wr.shape or wl.ndim != 2 or wl.shape[1] != ch:
+        raise ValueError("size mismatch between input channels and decoding filters")
+    R = np.ascontiguousarray(np.asarray(rotations, dtype=np.float64))
+    if R.ndim != 3 or R.shape[1:] != (3, 3):
+        raise ValueError("rotations must be [frames, 3, 3]")
+    ln = wl.shape[0]
+    hop = int(hop)
+    fade = hop if fade is None else int(fade)
+    rows = n - (ln // 2 - 1) if compensateDelay else n
+    out = np.zeros((max(rows, 0), 2), order="F")
+    h.check(h.lib.emagls_binaural_decode_sh_tracked(h.ptr, _p(x), n, N, _p(wl), _p(wr), ln, _p(R), R.shape[0], hop,
+                                                    fade, int(firstSample), 1 if compensateDelay else 0, _p(out)))
     return out
 
 

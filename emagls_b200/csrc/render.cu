@@ -467,11 +467,11 @@ void ForwardStage::run(long long b0, long long nbk, cplx* X) {
 // Large N amortises the overlap (N = 8 len: 12.5 % redundant input, 0.57 spectrum bins per output
 // frame instead of 1.0 at N = 2 len); the chunk (blocks per cuFFT batch) is sized so that the
 // staged input, its spectra and the ear spectra of one chunk stay L2-resident between the kernels.
-void binaural_decode_dev(emagls_ctx* h, const double* in, long long num_samples, int num_ch,
-                         const double* wL, const double* wR, int len, int compensate_delay, double* out) {
+void binaural_decode_rows(emagls_ctx* h, const double* in, long long num_samples, int num_ch, const double* wL,
+                          const double* wR, int len, long long skip, long long out_rows, double* out) {
   EM_REQUIRE(in && wL && wR && out, "null argument");
   EM_REQUIRE(num_samples > 0 && num_ch > 0 && len > 0, "empty input");
-  EM_REQUIRE(!compensate_delay || len % 2 == 0, "compensateDelay needs an even filter length");
+  EM_REQUIRE(skip >= 0 && num_samples - skip > 0, "signal shorter than the compensated delay");
   cudaStream_t st = h->stream;
   Arena ar(st);
   const int ov = (len + 1) & ~1;
@@ -485,9 +485,6 @@ void binaural_decode_dev(emagls_ctx* h, const double* in, long long num_samples,
     while (N < want && (long long)(N - ov) < num_samples) N <<= 1;
   }
   const int L = N - ov, F = N / 2 + 1;
-  const long long skip = compensate_delay ? (len / 2 - 1) : 0;  // out(del:end,:), binauralDecode.m:55-56
-  const long long out_rows = num_samples - skip;
-  EM_REQUIRE(out_rows > 0, "signal shorter than the compensated delay");
   const long long nblk_total = (num_samples + L - 1) / L;
   const int nex = ForwardStage::extra_blocks(ov, L);  // extra hops per channel: the overlapping batch has a uniform distance L
   // blocks per chunk: as many as a memory budget allows (measured on B200: launch-bound below a few
@@ -574,6 +571,13 @@ void binaural_decode_dev(emagls_ctx* h, const double* in, long long num_samples,
     h->launches += 2;
   }
   // stream-ordered: the arena's cudaFreeAsync calls queue behind the work above
+}
+
+void binaural_decode_dev(emagls_ctx* h, const double* in, long long num_samples, int num_ch,
+                         const double* wL, const double* wR, int len, int compensate_delay, double* out) {
+  EM_REQUIRE(!compensate_delay || len % 2 == 0, "compensateDelay needs an even filter length");
+  const long long skip = compensate_delay ? (len / 2 - 1) : 0;  // out(del:end,:), binauralDecode.m:55-56
+  binaural_decode_rows(h, in, num_samples, num_ch, wL, wR, len, skip, num_samples - skip, out);
 }
 
 void destroy_render_plans(emagls_ctx* h) {

@@ -24,6 +24,12 @@ void ensure_plans(emagls_ctx* h, emagls_ctx::RenderPlans& rp, int N, int L, int 
                   int inv_batch);
 void drop_plans(emagls_ctx::RenderPlans& rp);
 
+// The static render (binauralDecode) with the first `skip` output samples dropped: out[ear * out_rows + n - skip] for
+// n in [skip, num_samples).  The public entry points pass skip = 0 or len/2 - 1 (compensateDelay) and
+// out_rows = num_samples - skip; the SH head-tracked render writes one time chunk into a longer output with it.
+void binaural_decode_rows(emagls_ctx* h, const double* in, long long num_samples, int num_ch, const double* wL,
+                          const double* wR, int len, long long skip, long long out_rows, double* out);
+
 // Forward transforms of the overlap-save blocks of a multichannel signal into X[ch][nbc][F].  Block b takes the N
 // input samples starting at b*L - ov.  Direct route (default when every channel of the signal is 16-byte aligned):
 // interior blocks are transformed in place from `in`, one cuFFT call per channel, and only the blocks that overlap the

@@ -206,13 +206,19 @@ class ShardedRenderer:
     input halo: pinned host input block -> H2D -> emagls_binaural_decode_dev -> D2H of the block's two output
     channels.  Every rank keeps its block of the output (gather with torch.distributed if one host needs it all)."""
 
-    def __init__(self, handle, block_host, wL, wR, halo: int, *, track=None, hop=None, fade=None, first_sample=0):
+    def __init__(self, handle, block_host, wL, wR, halo: int, *, track=None, rotations=None, hop=None, fade=None,
+                 first_sample=0):
         """block_host: [halo + frames of this rank, channels], the rank's input block with its halo in front.
         Head-tracked render (emagls_binaural_decode_tracked): wL, wR are a bank [taps, channels, pages], `track` the
         0-based page of every frame of `hop` samples of the whole signal, `fade` the crossfade (default hop) and
-        `first_sample` the position of block_host[0] in the whole signal (lo - halo)."""
+        `first_sample` the position of block_host[0] in the whole signal (lo - halo).
+        Head-tracked render of a real SH signal (emagls_binaural_decode_sh_tracked): `rotations` [frames, 3, 3] is the
+        head orientation of every frame of the whole signal, wL, wR one filter pair [taps, (order+1)^2]; `hop`, `fade`
+        and `first_sample` as for `track`.  The track is uploaded once, here."""
         import ctypes as C
         import numpy as np
+        if track is not None and rotations is not None:
+            raise ValueError("track= (a filter bank) and rotations= (a rotated SH signal) exclude each other")
         self.C, self.h = C, handle
         self.dev = torch.device("cuda", handle.device)
         self.stream = torch.cuda.ExternalStream(handle.stream, device=self.dev)
@@ -220,11 +226,19 @@ class ShardedRenderer:
         self.pages = int(wL.shape[2]) if np.ndim(wL) == 3 else 1
         self.halo, self.n = int(halo), int(block_host.shape[0])
         self.track = None
-        if track is not None:
-            self.track = np.ascontiguousarray(np.asarray(track), dtype=np.int32)
+        self.rot_d = None
+        if track is not None or rotations is not None:
             self.hop = int(hop)
             self.fade = self.hop if fade is None else int(fade)
             self.first_sample = int(first_sample)
+        if track is not None:
+            self.track = np.ascontiguousarray(np.asarray(track), dtype=np.int32)
+        if rotations is not None:
+            self.order = int(round(self.ch ** 0.5)) - 1
+            if (self.order + 1) ** 2 != self.ch or np.ndim(wL) != 2:
+                raise ValueError("rotations= needs one filter pair [taps, (order+1)^2]")
+            R = np.ascontiguousarray(np.asarray(rotations, dtype=np.float64).reshape(-1, 9))
+            self.rot_d = torch.from_numpy(R).to(self.dev)
         # [frames, channels] column-major == [channels, frames] row-major
         blk = np.ascontiguousarray(np.asarray(block_host, dtype=np.float64).T)
         self.x_h = torch.from_numpy(blk).pin_memory()
@@ -236,12 +250,14 @@ class ShardedRenderer:
         self.d2h_bytes = self.y_h.numel() * 8
 
     @classmethod
-    def for_signal(cls, handle, x_host, wL, wR, *, track=None, hop=None, fade=None):
+    def for_signal(cls, handle, x_host, wL, wR, *, track=None, rotations=None, hop=None, fade=None):
         """Shard the whole signal x_host [frames, channels] over the ranks of the process group (head-tracked with
-        `track`, `hop`, `fade` and a bank wL, wR [taps, channels, pages])."""
+        `track`, `hop`, `fade` and a bank wL, wR [taps, channels, pages], or with `rotations`, `hop`, `fade` and one
+        filter pair for a real SH signal)."""
         rank, _, world = env_world()
         lo, hi, halo = render_shard(int(x_host.shape[0]), int(wL.shape[0]), rank, world)
-        r = cls(handle, x_host[lo - halo:hi], wL, wR, halo, track=track, hop=hop, fade=fade, first_sample=lo - halo)
+        r = cls(handle, x_host[lo - halo:hi], wL, wR, halo, track=track, rotations=rotations, hop=hop, fade=fade,
+                first_sample=lo - halo)
         r.lo, r.hi = lo, hi
         return r
 
@@ -249,7 +265,12 @@ class ShardedRenderer:
         h = self.h
         with torch.cuda.stream(self.stream):
             self.x_d.copy_(self.x_h, non_blocking=True)
-            if self.track is None:
+            if self.rot_d is not None:
+                h.check(h.lib.emagls_binaural_decode_sh_tracked_dev(
+                    h.ptr, self.x_d.data_ptr(), self.n, self.order, self.w[0].data_ptr(), self.w[1].data_ptr(),
+                    self.taps, self.rot_d.data_ptr(), self.rot_d.shape[0], self.hop, self.fade, self.first_sample, 0,
+                    self.y_d.data_ptr()))
+            elif self.track is None:
                 h.check(h.lib.emagls_binaural_decode_dev(h.ptr, self.x_d.data_ptr(), self.n, self.ch,
                                                          self.w[0].data_ptr(), self.w[1].data_ptr(), self.taps, 0,
                                                          self.y_d.data_ptr()))

@@ -251,6 +251,37 @@ int emagls_binaural_decode_tracked_dev(emagls_handle h, const double* in, long l
                                        const int32_t* track, long long num_frames, int hop, int fade,
                                        long long first_sample, int compensate_delay, double* out);
 
+/* ---- head-tracked binauralDecode of a real SH signal by sound-field rotation (not in the reference API) -------------
+ * Renders `in` [num_samples x C], C = (order + 1)^2 and 0 <= order <= 7, a real SH signal in the library's real basis
+ * (ACN order, the basis getSH(..., 'real') returns), with ONE static filter pair wL, wR [len x C] (e.g. the output of
+ * getEMagLsFilters or getLsFilters) while the sound field is rotated against the listener's head.  rotations
+ * [num_frames x 9] holds one row-major 3x3 matrix per tracker frame: the head orientation during frame f, in the
+ * convention of the designers' `rotations` argument (the world direction of head-frame direction u is R u).  Frame
+ * timing, first_sample, hop, fade and compensate_delay mean what they mean for emagls_binaural_decode_tracked: with
+ * t = first_sample + n, f = t / hop, i = t - f hop, c = f, a = max(f - 1, 0), g = (i < fade) ? (i + 0.5) / fade : 1
+ * and Q_f = getSHrotMtx(rotations[f], order, 'real'):
+ *     M(n)  = (1 - g) Q_a + g Q_c            (exactly Q_c when rotations[a] and rotations[c] are bitwise equal)
+ *     x'[n] = in[n, :] * M(n)                (row vector times matrix)
+ *     out   = binauralDecode(x', wL, wR, compensate_delay)
+ * The signal is rotated first and then convolved (the sound-field rotation of real-time Ambisonics renderers), not
+ * crossfaded at the output like the bank render.  A linear blend of two rotation matrices is not itself a rotation: at
+ * a 100 Hz tracker the step between frames is a few degrees, and the error of the blend is of second order in it.  A
+ * constant track R renders what the static render gives with the filters designed on the HRIR grid rotated by R.
+ * EMAGLS_ERR_INVALID, checked on the host before anything is launched: a null pointer, an order outside [0, 7], hop < 1,
+ * fade outside [0, hop], first_sample < 0, num_frames < (first_sample + num_samples - 1) / hop + 1, an odd len with
+ * compensate_delay, a signal shorter than the compensated delay.
+ * _dev: in, wL, wR, rotations and out are device pointers (no launch geometry depends on the track); the work is
+ * enqueued on emagls_stream(h).  The rotated signal is held in a workspace bounded as the bank render's
+ * (EMAGLS_TRACK_WS_MB); longer signals are rendered in time chunks.                                                   */
+int emagls_binaural_decode_sh_tracked(emagls_handle h, const double* in, long long num_samples, int order,
+                                      const double* wL, const double* wR, int len,
+                                      const double* rotations, long long num_frames, int hop, int fade,
+                                      long long first_sample, int compensate_delay, double* out);
+int emagls_binaural_decode_sh_tracked_dev(emagls_handle h, const double* in, long long num_samples, int order,
+                                          const double* wL, const double* wR, int len,
+                                          const double* rotations, long long num_frames, int hop, int fade,
+                                          long long first_sample, int compensate_delay, double* out);
+
 /* ======================================================================================================
  * Callers either side of the hot path (SURVEY.md section 8-f): radial filters, SH/CH encoding and
  * rotation of the recording in front of the render, the remaining lib/ designers.
