@@ -152,6 +152,22 @@ static void fill_args(DesignArgs& a, Variant v, const double* hL, const double* 
   a.num_sets = ns; a.num_orient = no; a.rotations = rot; a.wL = wL; a.wR = wR; a.spectra = sp;
 }
 
+// Device outputs of a design called with host memory: both ears' filters and, when asked for, the spectra.
+struct DeviceOutputs {
+  DesignShape s;
+  double *wL, *wR, *sp;
+  DeviceOutputs(Arena& ar, const DesignShape& shape, bool spectra)
+      : s(shape), wL(ar.get<double>(s.filter_elems)), wR(ar.get<double>(s.filter_elems)),
+        sp(spectra ? ar.get<double>(s.spectra_elems) : nullptr) {}
+  // copies the outputs to the host and waits for them
+  void download(cudaStream_t st, double* hwL, double* hwR, double* hsp) const {
+    EM_CUDA(cudaMemcpyAsync(hwL, wL, s.filter_elems * sizeof(double), cudaMemcpyDeviceToHost, st));
+    EM_CUDA(cudaMemcpyAsync(hwR, wR, s.filter_elems * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (hsp) EM_CUDA(cudaMemcpyAsync(hsp, sp, s.spectra_elems * sizeof(double), cudaMemcpyDeviceToHost, st));
+    EM_CUDA(cudaStreamSynchronize(st));
+  }
+};
+
 static int design_host(emagls_handle h, const emagls_config* cfg, Variant v, const double* hL,
                        const double* hR, int T, int D, const double* ga, const double* gz, double r,
                        const double* ma, const double* mz, int M, int order, double fs, int len,
@@ -161,24 +177,14 @@ static int design_host(emagls_handle h, const emagls_config* cfg, Variant v, con
     EM_REQUIRE(T > 0 && D > 0 && M > 0 && ns > 0 && no > 0 && len > 0, "empty input");
     cudaStream_t st = h->stream;
     Arena ar(st);
-    const int Mc = (v == Variant::EMAGLS2) ? M : (v == Variant::EMAGLS_SH ? (order + 1) * (order + 1) : 2 * order + 1);
-    const int nfft = std::min(cfg->nfft_max_len, 2 * len);
-    const int K = nfft / 2 + 1;
-    const size_t P = (size_t)ns * no;
+    const DesignShape shape = design_shape(*cfg, v, M, order, len, bin_grid(*cfg, len, fs, T).K, (size_t)ns * no);
+    DeviceOutputs out(ar, shape, sp != nullptr);
     DesignArgs a;
-    // complex SH-domain output is interleaved complex (lib/getEMagLsFilters.m:117-120)
-    const size_t wn = (size_t)len * Mc * P * ((v != Variant::EMAGLS2 && cfg->basis == EMAGLS_BASIS_COMPLEX) ? 2 : 1);
-    double* d_wL = ar.get<double>(wn);
-    double* d_wR = ar.get<double>(wn);
-    double* d_sp = sp ? ar.get<double>((size_t)2 * K * Mc * P * 2) : nullptr;
     fill_args(a, v, ar.upload(hL, (size_t)T * D * ns), ar.upload(hR, (size_t)T * D * ns), T, D,
               ar.upload(ga, D), ar.upload(gz, D), r, ar.upload(ma, M), mz ? ar.upload(mz, M) : nullptr, M, order, fs, len,
-              ns, no, rot ? ar.upload(rot, (size_t)no * 9) : nullptr, d_wL, d_wR, d_sp);
+              ns, no, rot ? ar.upload(rot, (size_t)no * 9) : nullptr, out.wL, out.wR, out.sp);
     design_factored(h, *cfg, a);
-    EM_CUDA(cudaMemcpyAsync(wL, d_wL, wn * sizeof(double), cudaMemcpyDeviceToHost, st));
-    EM_CUDA(cudaMemcpyAsync(wR, d_wR, wn * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (sp) EM_CUDA(cudaMemcpyAsync(sp, d_sp, (size_t)2 * K * Mc * P * 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
-    EM_CUDA(cudaStreamSynchronize(st));
+    out.download(st, wL, wR, sp);
   });
 }
 
@@ -214,20 +220,15 @@ int emagls_design_sma_basis(emagls_handle h, const emagls_config* cfg, int sh_do
     EM_REQUIRE(cfg && hL && hR && Y_hrir && Y_mic && wL && wR, "null argument");
     const int T = num_samples, D = num_dirs, M = num_mics, S = num_harmonics, ns = num_sets, no = num_orient;
     EM_REQUIRE(T > 0 && D > 0 && M > 0 && ns > 0 && no > 0 && len > 0 && S > 0, "empty input");
-    const int simN = std::max(order, (int)std::ceil(fs * M_PI * mic_radius / cfg->speed_of_sound));
+    const int simN = sim_order(*cfg, order, fs, mic_radius);
     EM_REQUIRE(S == (simN + 1) * (simN + 1),
                "custom bases must be evaluated at the simulation order max(order, ceil(fs pi r / c)) (getSMAIRMatrix.m:95)");
     EM_REQUIRE(cfg->basis == EMAGLS_BASIS_REAL || sh_domain == 0, "complex SH-domain output needs the default getSH");
     const Variant v = sh_domain ? Variant::EMAGLS_SH : Variant::EMAGLS2;
     cudaStream_t st = h->stream;
     Arena ar(st);
-    const int Mc = sh_domain ? (order + 1) * (order + 1) : M;
-    const int K = std::min(cfg->nfft_max_len, 2 * len) / 2 + 1;
-    const size_t P = (size_t)ns * no;
-    const size_t wn = (size_t)len * Mc * P;
-    double* d_wL = ar.get<double>(wn);
-    double* d_wR = ar.get<double>(wn);
-    double* d_sp = spectra ? ar.get<double>((size_t)2 * K * Mc * P * 2) : nullptr;
+    const DesignShape shape = design_shape(*cfg, v, M, order, len, bin_grid(*cfg, len, fs, T).K, (size_t)ns * no);
+    DeviceOutputs out(ar, shape, spectra != nullptr);
     // MATLAB [M x S] column-major per orientation -> [orientation][M][S] (S contiguous)
     std::vector<double> ymt((size_t)no * M * S);
     for (int o = 0; o < no; ++o)
@@ -235,16 +236,12 @@ int emagls_design_sma_basis(emagls_handle h, const emagls_config* cfg, int sh_do
         for (int s_ = 0; s_ < S; ++s_) ymt[((size_t)o * M + m) * S + s_] = Y_mic[((size_t)o * S + s_) * M + m];
     DesignArgs a;
     fill_args(a, v, ar.upload(hL, (size_t)T * D * ns), ar.upload(hR, (size_t)T * D * ns), T, D, nullptr, nullptr,
-              mic_radius, nullptr, nullptr, M, order, fs, len, ns, no, nullptr, d_wL, d_wR, d_sp);
+              mic_radius, nullptr, nullptr, M, order, fs, len, ns, no, nullptr, out.wL, out.wR, out.sp);
     a.Y_hrir = ar.upload(Y_hrir, (size_t)S * D);
     a.Y_mic = ar.upload(ymt.data(), ymt.size());
     EM_CUDA(cudaStreamSynchronize(st));   // ymt is a temporary
     design_factored(h, *cfg, a);
-    EM_CUDA(cudaMemcpyAsync(wL, d_wL, wn * sizeof(double), cudaMemcpyDeviceToHost, st));
-    EM_CUDA(cudaMemcpyAsync(wR, d_wR, wn * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (spectra)
-      EM_CUDA(cudaMemcpyAsync(spectra, d_sp, (size_t)2 * K * Mc * P * 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
-    EM_CUDA(cudaStreamSynchronize(st));
+    out.download(st, wL, wR, spectra);
   });
 }
 
@@ -266,19 +263,12 @@ static int magls_host(emagls_handle h, const emagls_config* cfg, const double* h
     EM_REQUIRE(num_samples > 0 && num_dirs > 0 && len > 0 && order >= 0 && num_sets > 0, "empty input");
     cudaStream_t st = h->stream;
     Arena ar(st);
-    const int T = num_samples, D = num_dirs, Mc = (order + 1) * (order + 1), NS = num_sets;
-    const int K = std::min(cfg->nfft_max_len, 2 * len) / 2 + 1;
-    const size_t wn = (size_t)len * Mc * NS * (cfg->basis == EMAGLS_BASIS_COMPLEX ? 2 : 1);
-    double* d_wL = ar.get<double>(wn);
-    double* d_wR = ar.get<double>(wn);
-    double* d_sp = spectra ? ar.get<double>((size_t)2 * K * Mc * NS * 2) : nullptr;
+    const int T = num_samples, D = num_dirs, NS = num_sets;
+    const DesignShape shape = design_shape(*cfg, Variant::EMAGLS_SH, 0, order, len, bin_grid(*cfg, len, fs, T).K, NS);
+    DeviceOutputs out(ar, shape, spectra != nullptr);
     design_magls(h, *cfg, ar.upload(hL, (size_t)T * D * NS), ar.upload(hR, (size_t)T * D * NS), T, D,
-                 ar.upload(grid_azi, D), ar.upload(grid_zen, D), order, fs, len, false, d_wL, d_wR, d_sp, 0, NS);
-    EM_CUDA(cudaMemcpyAsync(wL, d_wL, wn * sizeof(double), cudaMemcpyDeviceToHost, st));
-    EM_CUDA(cudaMemcpyAsync(wR, d_wR, wn * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (spectra)
-      EM_CUDA(cudaMemcpyAsync(spectra, d_sp, (size_t)2 * K * Mc * NS * 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
-    EM_CUDA(cudaStreamSynchronize(st));
+                 ar.upload(grid_azi, D), ar.upload(grid_zen, D), order, fs, len, false, out.wL, out.wR, out.sp, 0, NS);
+    out.download(st, wL, wR, spectra);
   });
 }
 int emagls_design_magls(emagls_handle h, const emagls_config* cfg, const double* hL, const double* hR,
@@ -300,15 +290,11 @@ int emagls_design_ls(emagls_handle h, const emagls_config* cfg, const double* hL
     EM_REQUIRE(num_samples > 0 && num_dirs > 0 && order >= 0, "empty input");
     cudaStream_t st = h->stream;
     Arena ar(st);
-    const int T = num_samples, D = num_dirs, Mc = (order + 1) * (order + 1);
-    const size_t wn = (size_t)T * Mc * (cfg->basis == EMAGLS_BASIS_COMPLEX ? 2 : 1);
-    double* d_wL = ar.get<double>(wn);
-    double* d_wR = ar.get<double>(wn);
+    const int T = num_samples, D = num_dirs;
+    DeviceOutputs out(ar, design_shape(*cfg, Variant::EMAGLS_SH, 0, order, T, 0, 1), false);   // T taps, no spectra
     design_magls(h, *cfg, ar.upload(hL, (size_t)T * D), ar.upload(hR, (size_t)T * D), T, D, ar.upload(grid_azi, D),
-                 ar.upload(grid_zen, D), order, 0.0, 0, true, d_wL, d_wR, nullptr);
-    EM_CUDA(cudaMemcpyAsync(wL, d_wL, wn * sizeof(double), cudaMemcpyDeviceToHost, st));
-    EM_CUDA(cudaMemcpyAsync(wR, d_wR, wn * sizeof(double), cudaMemcpyDeviceToHost, st));
-    EM_CUDA(cudaStreamSynchronize(st));
+                 ar.upload(grid_zen, D), order, 0.0, 0, true, out.wL, out.wR, nullptr);
+    out.download(st, wL, wR, nullptr);
   });
 }
 static int from_atf_host(emagls_handle h, const emagls_config* cfg, const double* hL, const double* hR,
@@ -323,20 +309,14 @@ static int from_atf_host(emagls_handle h, const emagls_config* cfg, const double
     cudaStream_t st = h->stream;
     Arena ar(st);
     const int T = num_samples, D = num_dirs, M = num_mics, B = num_orient;
-    const int K = std::min(cfg->nfft_max_len, 2 * filter_len) / 2 + 1;
-    const size_t wn = (size_t)filter_len * M * B;
-    double* d_wL = ar.get<double>(wn);
-    double* d_wR = ar.get<double>(wn);
-    double* d_sp = spectra ? ar.get<double>((size_t)2 * K * M * B * 2) : nullptr;
+    // one real channel per microphone, as the EMAGLS2 variant
+    const DesignShape shape = design_shape(*cfg, Variant::EMAGLS2, M, 0, filter_len, bin_grid(*cfg, filter_len, fs, T).K, B);
+    DeviceOutputs out(ar, shape, spectra != nullptr);
     design_from_atf(h, *cfg, ar.upload(hL, (size_t)T * D), ar.upload(hR, (size_t)T * D), T, D,
                     ar.upload(hrir_grid, (size_t)2 * D), ar.upload(atf_irs, (size_t)atf_samples * M * atf_dirs),
                     atf_samples, M, atf_dirs, ar.upload(atf_grid, (size_t)2 * atf_dirs), fs, filter_len, f_trans, B,
-                    rotations ? ar.upload(rotations, (size_t)B * 9) : nullptr, d_wL, d_wR, d_sp, mean_grid_dev_deg);
-    EM_CUDA(cudaMemcpyAsync(wL, d_wL, wn * sizeof(double), cudaMemcpyDeviceToHost, st));
-    EM_CUDA(cudaMemcpyAsync(wR, d_wR, wn * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (spectra)
-      EM_CUDA(cudaMemcpyAsync(spectra, d_sp, (size_t)2 * K * M * B * 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
-    EM_CUDA(cudaStreamSynchronize(st));
+                    rotations ? ar.upload(rotations, (size_t)B * 9) : nullptr, out.wL, out.wR, out.sp, mean_grid_dev_deg);
+    out.download(st, wL, wR, spectra);
   });
 }
 int emagls_design_from_atf(emagls_handle h, const emagls_config* cfg, const double* hL, const double* hR,
@@ -390,19 +370,13 @@ int emagls_design_ema_sh(emagls_handle h, const emagls_config* cfg, const double
     EM_REQUIRE(num_samples > 0 && num_dirs > 0 && num_mics > 0 && len > 0 && order >= 0, "empty input");
     cudaStream_t st = h->stream;
     Arena ar(st);
-    const int T = num_samples, D = num_dirs, Mc = (order + 1) * (order + 1);
-    const int K = std::min(cfg->nfft_max_len, 2 * len) / 2 + 1;
-    const size_t wn = (size_t)len * Mc * (cfg->basis == EMAGLS_BASIS_COMPLEX ? 2 : 1);
-    double* d_wL = ar.get<double>(wn);
-    double* d_wR = ar.get<double>(wn);
-    double* d_sp = spectra ? ar.get<double>((size_t)2 * K * Mc * 2) : nullptr;
+    const int T = num_samples, D = num_dirs;
+    const DesignShape shape = design_shape(*cfg, Variant::EMAGLS_SH, 0, order, len, bin_grid(*cfg, len, fs, T).K, 1);
+    DeviceOutputs out(ar, shape, spectra != nullptr);
     design_ema_sh(h, *cfg, ar.upload(hL, (size_t)T * D), ar.upload(hR, (size_t)T * D), T, D, ar.upload(grid_azi, D),
                   ar.upload(grid_zen, D), mic_radius, ar.upload(mic_azi, num_mics), num_mics, order, fs, len,
-                  d_wL, d_wR, d_sp);
-    EM_CUDA(cudaMemcpyAsync(wL, d_wL, wn * sizeof(double), cudaMemcpyDeviceToHost, st));
-    EM_CUDA(cudaMemcpyAsync(wR, d_wR, wn * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (spectra) EM_CUDA(cudaMemcpyAsync(spectra, d_sp, (size_t)2 * K * Mc * 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
-    EM_CUDA(cudaStreamSynchronize(st));
+                  out.wL, out.wR, out.sp);
+    out.download(st, wL, wR, spectra);
   });
 }
 
@@ -423,15 +397,6 @@ __global__ void smair_kernel(const cplx* __restrict__ Yrows, const cplx* __restr
   out[idx] = cmul(Yrows[(long long)r * S + s], bn[(long long)k * (N + 1) + ord]);
 }
 
-// Ymic[m][s] (complex) from launch_sh_angles output [S][M] (real or complex basis)
-__global__ void sh_to_rows_kernel(const double* __restrict__ Y, int M, int S, int complex_basis,
-                                  cplx* __restrict__ rows) {
-  int idx = blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= M * S) return;
-  int m = idx / S, s = idx % S;
-  rows[idx] = complex_basis ? reinterpret_cast<const cplx*>(Y)[(long long)s * M + m] : mk(Y[(long long)s * M + m], 0.0);
-}
-
 // Yout[c][s] = sum_m Lt[(m&1)*npair + m/2][c] * Ymic[m][s]   (pinv(Y_lo) * Y_Hi, getSMAIRMatrix.m:102,119-121)
 __global__ void smair_project_kernel(const cplx* __restrict__ Lt, int npair, int nsh, int M, int S,
                                      const cplx* __restrict__ Ymic, cplx* __restrict__ Yout) {
@@ -441,13 +406,6 @@ __global__ void smair_project_kernel(const cplx* __restrict__ Lt, int npair, int
   cplx acc = mk(0.0, 0.0);
   for (int m = 0; m < M; ++m) cfma(acc, Lt[((long long)(m & 1) * npair + m / 2) * nsh + c], Ymic[(long long)m * S + s]);
   Yout[idx] = acc;
-}
-
-__global__ void unit_rows_kernel(double* rows, int npair, int D) {
-  long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= (long long)npair * 4 * D) return;
-  const int d = (int)(idx % D), row = (int)(idx / D);
-  rows[idx] = ((row & 1) == 0 && (row >> 1) == d) ? 1.0 : 0.0;
 }
 
 // smairMat(r, :, k) *= rad(k, ord(r)), and once more by real(rad) at the Nyquist bin
@@ -473,7 +431,7 @@ static int smair_impl(emagls_handle h, const emagls_config* cfg, const emagls_ra
   return guarded(h, [&] {
     EM_REQUIRE(cfg && mic_azi && mic_zen && num_mics > 0, "null argument");
     EM_REQUIRE(nfft > 0 && nfft % 2 == 0, "nfft must be even");  // getSMAIRMatrix.m:89
-    const int simN = std::max(order, (int)std::ceil(fs * M_PI * sma_radius / cfg->speed_of_sound));
+    const int simN = sim_order(*cfg, order, fs, sma_radius);
     if (sim_order_out) *sim_order_out = simN;
     if (!out) return;
     EM_REQUIRE(simN <= MAX_SH_ORDER, "simulation order too high");
@@ -482,17 +440,14 @@ static int smair_impl(emagls_handle h, const emagls_config* cfg, const emagls_ra
     const int S = (simN + 1) * (simN + 1), K = nfft / 2 + 1, M = num_mics;
     const int nsh = (order + 1) * (order + 1);
     const int cb = cfg->basis == EMAGLS_BASIS_COMPLEX ? 1 : 0;
-    std::vector<double> kr(K);
-    const double df = (fs / 2.0) / (double)(K - 1);
-    for (int k = 0; k < K; ++k) kr[k] = 2.0 * M_PI * ((double)k * df) / cfg->speed_of_sound * sma_radius;
+    const std::vector<double> kr = kr_table(*cfg, fs, sma_radius, K);
     cplx* bn = ar.get<cplx>((size_t)K * (simN + 1));
     EM_CUDA(launch_modal(st, simN, ar.upload(kr.data(), K), K, cfg->array_type, -1.0, 1, bn, simN + 1, 1));
     // Y_Hi = shFunction(simulationOrder, mics, shDefinition) as rows [M][S]
     double* Y = ar.get<double>((size_t)M * S * (cb ? 2 : 1));
     EM_CUDA(launch_sh_angles(st, simN, ar.upload(mic_azi, M), ar.upload(mic_zen, M), M, cb, Y));
     cplx* Ymic = ar.get<cplx>((size_t)M * S);
-    sh_to_rows_kernel<<<(M * S + 255) / 256, 256, 0, st>>>(Y, M, S, cb, Ymic);
-    EM_CUDA(cudaGetLastError());
+    EM_CUDA(launch_sh_rows(st, Y, M, S, cb, Ymic));
     h->launches += 3;
     const cplx* Yrows = Ymic;
     int rows = M;
@@ -502,16 +457,11 @@ static int smair_impl(emagls_handle h, const emagls_config* cfg, const emagls_ra
       cplx* Alo = ar.get<cplx>((size_t)M * nsh);
       EM_CUDA(cudaMemcpy2DAsync(Alo, (size_t)nsh * sizeof(cplx), Ymic, (size_t)S * sizeof(cplx),
                                 (size_t)nsh * sizeof(cplx), M, cudaMemcpyDeviceToDevice, st));
-      const int npair = (M + 1) / 2;
-      double* urows = ar.get<double>((size_t)npair * 4 * M);
-      long long n = (long long)npair * 4 * M;
-      unit_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(urows, npair, M);
-      cplx* Lt = ar.get<cplx>((size_t)2 * npair * nsh);
-      regularized_apply_dev(h, ar, Alo, M, nsh, urows, npair, 0.0, Lt);
+      cplx* Lt = unclipped_pinv_dev(h, ar, Alo, M, nsh);
       cplx* Yout = ar.get<cplx>((size_t)nsh * S);
-      smair_project_kernel<<<(nsh * S + 255) / 256, 256, 0, st>>>(Lt, npair, nsh, M, S, Ymic, Yout);
+      smair_project_kernel<<<(nsh * S + 255) / 256, 256, 0, st>>>(Lt, (M + 1) / 2, nsh, M, S, Ymic, Yout);
       EM_CUDA(cudaGetLastError());
-      h->launches += 2;
+      h->launches += 1;
       Yrows = Yout;
       rows = nsh;
     }
@@ -558,18 +508,12 @@ int emagls_design_magls_2d(emagls_handle h, const emagls_config* cfg, const doub
     EM_REQUIRE(num_samples > 0 && num_dirs > 0 && len > 0 && order >= 0, "empty input");
     cudaStream_t st = h->stream;
     Arena ar(st);
-    const int T = num_samples, D = num_dirs, Mc = 2 * order + 1;
-    const int K = std::min(cfg->nfft_max_len, 2 * len) / 2 + 1;
-    const size_t wn = (size_t)len * Mc * (cfg->basis == EMAGLS_BASIS_COMPLEX ? 2 : 1);
-    double* d_wL = ar.get<double>(wn);
-    double* d_wR = ar.get<double>(wn);
-    double* d_sp = spectra ? ar.get<double>((size_t)2 * K * Mc * 2) : nullptr;
+    const int T = num_samples, D = num_dirs;
+    const DesignShape shape = design_shape(*cfg, Variant::EMA_CH, 0, order, len, bin_grid(*cfg, len, fs, T).K, 1);
+    DeviceOutputs out(ar, shape, spectra != nullptr);
     design_magls(h, *cfg, ar.upload(hL, (size_t)T * D), ar.upload(hR, (size_t)T * D), T, D, ar.upload(grid_azi, D),
-                 nullptr, order, fs, len, false, d_wL, d_wR, d_sp, 1);
-    EM_CUDA(cudaMemcpyAsync(wL, d_wL, wn * sizeof(double), cudaMemcpyDeviceToHost, st));
-    EM_CUDA(cudaMemcpyAsync(wR, d_wR, wn * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (spectra) EM_CUDA(cudaMemcpyAsync(spectra, d_sp, (size_t)2 * K * Mc * 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
-    EM_CUDA(cudaStreamSynchronize(st));
+                 nullptr, order, fs, len, false, out.wL, out.wR, out.sp, 1);
+    out.download(st, wL, wR, spectra);
   });
 }
 
@@ -612,11 +556,7 @@ int emagls_group_delay(emagls_handle h, const double* hrir, int taps, int num_di
     EM_CUDA(cudaMemcpyAsync(g.data(), d_gd, g.size() * sizeof(double), cudaMemcpyDeviceToHost, st));
     EM_CUDA(cudaStreamSynchronize(st));
     if (gd) std::copy(g.begin(), g.end(), gd);
-    if (median_out) {
-      std::sort(g.begin(), g.end());
-      const size_t n = g.size();
-      *median_out = (n & 1) ? g[n / 2] : 0.5 * (g[n / 2 - 1] + g[n / 2]);
-    }
+    if (median_out) *median_out = median_of(g);
   });
 }
 

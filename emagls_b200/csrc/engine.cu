@@ -39,20 +39,20 @@ struct EpiRamp {  // H = fft(h) .* exp_omega  (applySubsampleDelay.m:10-17), col
   }
 };
 
-double median_of(std::vector<double> v) {
-  size_t n = v.size();
-  std::sort(v.begin(), v.end());
-  return (n & 1) ? v[n / 2] : 0.5 * (v[n / 2 - 1] + v[n / 2]);
-}
-
-__global__ void identity_rows_kernel(double* rows, int npair, int D, int n) {
-  // rows [(pair*2 + ear)*2 + c][D]: target t = pair*2 + ear is the unit vector e_t (t < n)
+// rows [(pair*2 + ear)*2 + c][D]: target t = pair*2 + ear is the unit vector e_t
+__global__ void unit_rows_kernel(double* rows, int npair, int D) {
   long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= (long long)npair * 4 * D) return;
-  int d = (int)(idx % D);
-  int row = (int)(idx / D);
-  int c = row & 1, t = row >> 1;
-  rows[idx] = (c == 0 && t == d && t < n) ? 1.0 : 0.0;
+  const int d = (int)(idx % D), row = (int)(idx / D);
+  rows[idx] = ((row & 1) == 0 && (row >> 1) == d) ? 1.0 : 0.0;
+}
+
+__global__ void sh_to_rows_kernel(const double* __restrict__ Y, int M, int S, int complex_basis,
+                                  cplx* __restrict__ rows) {
+  int idx = blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= M * S) return;
+  int m = idx / S, s = idx % S;
+  rows[idx] = complex_basis ? reinterpret_cast<const cplx*>(Y)[(long long)s * M + m] : mk(Y[(long long)s * M + m], 0.0);
 }
 
 __global__ void real_to_cplx_kernel(const double* in, long long n, cplx* out) {
@@ -91,6 +91,54 @@ __global__ void extract_pinv_kernel(const cplx* W, int npair, int Mc, int M, dou
 }
 
 }  // namespace
+
+cudaError_t launch_fill(cudaStream_t st, double* p, int n, double v) {
+  fill_kernel<<<(n + 127) / 128, 128, 0, st>>>(p, n, v);
+  return cudaGetLastError();
+}
+cudaError_t launch_sh_rows(cudaStream_t st, const double* Y, int M, int S, int complex_basis, cplx* rows) {
+  sh_to_rows_kernel<<<(M * S + 255) / 256, 256, 0, st>>>(Y, M, S, complex_basis, rows);
+  return cudaGetLastError();
+}
+
+BinGrid bin_grid(const emagls_config& cfg, int len, double fs, int T) {
+  EM_REQUIRE(len >= T, "len too short");  // lib/getEMagLs2Filters.m:42
+  EM_REQUIRE(len % 2 == 0, "len must be even");
+  const int nfft = std::min(cfg.nfft_max_len, 2 * len);
+  EM_REQUIRE(nfft / 2 >= len / 2, "len exceeds NFFT_MAX_LEN (reference indexes out of range here)");
+  const int K = nfft / 2 + 1;
+  return {nfft, K, (fs / 2.0) / (double)(K - 1)};
+}
+int BinGrid::kls1(double f_cut) const {
+  const int k_cut = (int)std::ceil(f_cut / df);  // 1-based MATLAB index
+  return std::min(std::max(k_cut - 1, 1), K);
+}
+
+int sim_order(const emagls_config& cfg, int order, double fs, double radius) {
+  return std::max(order, (int)std::ceil(fs * M_PI * radius / cfg.speed_of_sound));
+}
+
+std::vector<double> kr_table(const emagls_config& cfg, double fs, double radius, int K) {
+  std::vector<double> kr(K);
+  const double df = (fs / 2.0) / (double)(K - 1);
+  for (int k = 0; k < K; ++k) kr[k] = 2.0 * M_PI * ((double)k * df) / cfg.speed_of_sound * radius;
+  return kr;
+}
+
+double median_of(std::vector<double> v) {
+  size_t n = v.size();
+  std::sort(v.begin(), v.end());
+  return (n & 1) ? v[n / 2] : 0.5 * (v[n / 2 - 1] + v[n / 2]);
+}
+
+DesignShape design_shape(const emagls_config& cfg, Variant v, int M, int order, int len, int K, size_t P) {
+  DesignShape s;
+  s.nch = (v == Variant::EMAGLS2) ? M : (v == Variant::EMAGLS_SH ? (order + 1) * (order + 1) : 2 * order + 1);
+  s.cplx = v != Variant::EMAGLS2 && cfg.basis == EMAGLS_BASIS_COMPLEX;
+  s.filter_elems = (size_t)len * s.nch * P * (s.cplx ? 2 : 1);
+  s.spectra_elems = (size_t)2 * K * s.nch * P * 2;
+  return s;
+}
 
 // ---- complex SH / CH basis (shDefinition = 'complex', lib/getEMagLsFilters.m:117-120) -----------
 // pwGrid_complex = conj(T) pwGrid_real with the unitary real->complex map Y_c = Y_r T^T
@@ -258,40 +306,46 @@ void regularized_apply_dev(emagls_ctx* h, Arena& ar, const cplx* At, int D, int 
   h->launches += 2;
 }
 
+cplx* unclipped_pinv_dev(emagls_ctx* h, Arena& ar, const cplx* At, int M, int Mc) {
+  const int npair = (M + 1) / 2;
+  double* rows = ar.get<double>((size_t)npair * 4 * M);
+  const long long n = (long long)npair * 4 * M;
+  unit_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(rows, npair, M);
+  EM_CUDA(cudaGetLastError());
+  h->launches += 1;
+  cplx* Lt = ar.get<cplx>((size_t)2 * npair * Mc);
+  regularized_apply_dev(h, ar, At, M, Mc, rows, npair, 0.0, Lt);
+  return Lt;
+}
+
 void design_factored(emagls_ctx* h, const emagls_config& cfg, const DesignArgs& a) {
   cudaStream_t st = h->stream;
   // ---------------- reference arithmetic on the scalar parameters (lib/getEMagLs2Filters.m:42-48)
   EM_REQUIRE(a.T > 0 && a.D > 0 && a.M > 0 && a.len > 0, "empty input");
-  EM_REQUIRE(a.len >= a.T, "len too short");  // lib/getEMagLs2Filters.m:42
-  EM_REQUIRE(a.len % 2 == 0, "len must be even");
   EM_REQUIRE(a.num_sets >= 1 && a.num_orient >= 1, "empty batch");
   EM_REQUIRE(a.rotations != nullptr || a.num_orient == 1 || a.Y_mic != nullptr, "num_orient > 1 needs rotations");
   EM_REQUIRE((a.Y_hrir == nullptr) == (a.Y_mic == nullptr), "custom bases: Y_hrir and Y_mic must be given together");
-  const int nfft = std::min(cfg.nfft_max_len, 2 * a.len);
-  EM_REQUIRE(nfft % 2 == 0, "nfft must be even");  // getSMAIRMatrix.m:89
-  EM_REQUIRE(nfft / 2 >= a.len / 2, "len exceeds NFFT_MAX_LEN (reference indexes out of range here)");
-  const int K = nfft / 2 + 1;
-  const double df = (a.fs / 2.0) / (double)(K - 1);
-  const double f_cut = std::max(cfg.f_cut_min, 500.0 * a.order);
-  const int k_cut = (int)std::ceil(f_cut / df);  // 1-based MATLAB index
-  const int simN = std::max(a.order, (int)std::ceil(a.fs * M_PI * a.mic_radius / cfg.speed_of_sound));
+  const BinGrid bg = bin_grid(cfg, a.len, a.fs, a.T);
+  EM_REQUIRE(bg.nfft % 2 == 0, "nfft must be even");  // getSMAIRMatrix.m:89
+  const int nfft = bg.nfft, K = bg.K;
+  const int simN = sim_order(cfg, a.order, a.fs, a.mic_radius);
   EM_REQUIRE(simN <= MAX_SH_ORDER, "simulation order too high");
   const int S = (simN + 1) * (simN + 1);
-  const int nsh = (a.order + 1) * (a.order + 1);
-  const int Mc = (a.variant == Variant::EMAGLS2) ? a.M : (a.variant == Variant::EMAGLS_SH ? nsh : 2 * a.order + 1);
+  const int P = a.num_sets * a.num_orient;
+  const DesignShape shape = design_shape(cfg, a.variant, a.M, a.order, a.len, K, P);
+  const int Mc = shape.nch;
   EM_REQUIRE(Mc <= 64 && a.M <= 64, "more than 64 channels are not supported");
   if (a.variant != Variant::EMAGLS2) EM_REQUIRE(a.M >= Mc, "fewer microphones than output channels");
   if (a.D < S)
     throw Fail{EMAGLS_ERR_UNSUPPORTED, "HRIR grid has fewer directions than simulation harmonics"};
   EM_REQUIRE(S >= Mc, "fewer simulation harmonics than channels");
-  const int P = a.num_sets * a.num_orient;
   const int D = a.D, T = a.T;
   // complex SH-domain output: solved in the real basis, converted at the tail (see above)
-  const bool cplx_out = (a.variant != Variant::EMAGLS2 && cfg.basis == EMAGLS_BASIS_COMPLEX);
+  const bool cplx_out = shape.cplx;
   const int basis_kind = (a.variant == Variant::EMA_CH) ? 1 : 0;
   const int dc_fix = cplx_out ? 0 : 1;
-  // bins (0-based): LS 1 .. kls1-1, MagLS kls1 .. K-1, with kls1 = k_cut - 1
-  const int kls1 = std::min(std::max(k_cut - 1, 1), K);
+  // bins (0-based): LS 1 .. kls1-1, MagLS kls1 .. K-1
+  const int kls1 = bg.kls1(std::max(cfg.f_cut_min, 500.0 * a.order));
   const int nLS = kls1 - 1;
 
   Arena ar(st);
@@ -340,11 +394,7 @@ void design_factored(emagls_ctx* h, const emagls_config& cfg, const DesignArgs& 
   };
   if (!chol_qr) householder_qr();
   // ---------------- array: b_n table (minus sign, Nyquist real: getSMAIRMatrix.m:107,115-117)
-  std::vector<double> kr(K);
-  for (int k = 0; k < K; ++k) {
-    double f = (double)k * df;
-    kr[k] = 2.0 * M_PI * f / cfg.speed_of_sound * a.mic_radius;
-  }
+  const std::vector<double> kr = kr_table(cfg, a.fs, a.mic_radius, K);
   double* d_kr = ar.upload(kr.data(), K);
   cplx* bn = ar.get<cplx>((size_t)K * (simN + 1));
   EM_CUDA(launch_modal(st, simN, d_kr, K, cfg.array_type, -1.0, 1, bn, simN + 1, 1));
@@ -374,7 +424,7 @@ void design_factored(emagls_ctx* h, const emagls_config& cfg, const DesignArgs& 
     const double* mic_zen = a.mic_zen;
     if (!mic_zen) {  // equatorial array (lib/getEMagLsFiltersEMAinCH.m:57)
       double* z = ar.get<double>(a.M);
-      fill_kernel<<<(a.M + 63) / 64, 64, 0, st>>>(z, a.M, 1.5707963267948966);
+      EM_CUDA(launch_fill(st, z, a.M, 1.5707963267948966));
       mic_zen = z;
       h->launches += 1;
     }
@@ -405,20 +455,13 @@ void design_factored(emagls_ctx* h, const emagls_config& cfg, const DesignArgs& 
         ch_rows_kernel<<<(a.M * Mc + 127) / 128, 128, 0, st>>>(a.order, a.mic_azi, a.M, At);
         h->launches += 1;
       }
-      const int npair = (a.M + 1) / 2;
-      double* rows = ar.get<double>((size_t)npair * 4 * a.M);
-      {
-        long long n = (long long)npair * 4 * a.M;
-        identity_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(rows, npair, a.M, a.M);
-      }
-      cplx* Wp = ar.get<cplx>((size_t)2 * npair * Mc);
-      regularized_apply_dev(h, ar, At, a.M, Mc, rows, npair, 0.0, Wp);
+      cplx* Wp = unclipped_pinv_dev(h, ar, At, a.M, Mc);
       double* L = ar.get<double>((size_t)Mc * a.M);
-      extract_pinv_kernel<<<(Mc * a.M + 255) / 256, 256, 0, st>>>(Wp, npair, Mc, a.M, L);
+      extract_pinv_kernel<<<(Mc * a.M + 255) / 256, 256, 0, st>>>(Wp, (a.M + 1) / 2, Mc, a.M, L);
       double* Yeff = ar.get<double>((size_t)a.num_orient * Mc * S);
       EM_CUDA(launch_left_mul(st, L, Mc, a.M, Ym, a.num_orient, S, Yeff));
       EM_CUDA(cudaGetLastError());
-      h->launches += 3;
+      h->launches += 2;
       Yo = Yeff;
     }
   }

@@ -181,6 +181,35 @@ struct DesignArgs {
   const double* Y_mic = nullptr;
 };
 void design_factored(emagls_ctx* h, const emagls_config& cfg, const DesignArgs& a);
+
+// ---- setup shared by the designers (engine.cu) ------------------------------------------------
+// Bins of a design with filter length len (lib/getEMagLs2Filters.m:35-48): nfft = min(NFFT_MAX_LEN, 2 len),
+// K = nfft/2 + 1 bins df apart.  Requires len >= T, len even and nfft/2 >= len/2.
+struct BinGrid {
+  int nfft, K;
+  double df;
+  // 0-based first MagLS bin for the cut-over frequency f_cut: LS bins 1 .. kls1-1, MagLS bins kls1 .. K-1
+  int kls1(double f_cut) const;
+};
+BinGrid bin_grid(const emagls_config& cfg, int len, double fs, int T);
+// simulation order max(order, ceil(fs pi r / c)) (getSMAIRMatrix.m:95)
+int sim_order(const emagls_config& cfg, int order, double fs, double radius);
+// kr of bins k = 0 .. K-1 spaced (fs/2)/(K-1) apart (getSMAIRMatrix.m:107)
+std::vector<double> kr_table(const emagls_config& cfg, double fs, double radius, int K);
+double median_of(std::vector<double> v);
+// Outputs of a design: nch channels (EMAGLS2: the M microphones; EMAGLS_SH: (order+1)^2 SH; EMA_CH: 2 order + 1 CH),
+// filters [len x nch x P] per ear, interleaved complex (twice the doubles) for SH / CH output in the complex basis
+// (lib/getEMagLsFilters.m:117-120),
+// spectra complex [K x nch x P x 2 ears].
+struct DesignShape {
+  int nch;
+  bool cplx;
+  size_t filter_elems, spectra_elems;   // doubles
+};
+DesignShape design_shape(const emagls_config& cfg, Variant v, int M, int order, int len, int K, size_t P);
+cudaError_t launch_fill(cudaStream_t st, double* p, int n, double v);
+// rows [M][S] (complex) from launch_sh_angles output [S][M] (real or complex basis)
+cudaError_t launch_sh_rows(cudaStream_t st, const double* Y, int M, int S, int complex_basis, cplx* rows);
 void destroy_render_plans(emagls_ctx* h);  // render.cu (static and head-tracked render)
 void destroy_fir_plans(emagls_ctx* h);     // frontend.cu
 // radFilts [K][(order+1)] (row index k) on the device (getRadialFilter.m:42-70)
@@ -209,5 +238,8 @@ void hrir_spectrum(emagls_ctx* h, Arena& ar, const double* hp, int T, int D, int
 // W [ear][pair][Mc]
 void regularized_apply_dev(emagls_ctx* h, Arena& ar, const cplx* At, int D, int Mc, const double* rows,
                            int npair, double regul, cplx* W);
+// Unclipped pseudo-inverse of the rows At [M][Mc]: regularized_apply_dev with regul = 0 on the unit targets e_m.
+// Returns Lt [ear][pair][Mc], npair = (M + 1) / 2: target m is row (m & 1) * npair + m / 2.
+cplx* unclipped_pinv_dev(emagls_ctx* h, Arena& ar, const cplx* At, int M, int Mc);
 
 }  // namespace emagls

@@ -279,22 +279,6 @@ __global__ void extract_enc_kernel(const cplx* __restrict__ Lt, int npair, int M
   P[idx] = imag ? v.y : v.x;
 }
 
-__global__ void unit_rows2_kernel(double* rows, int npair, int D) {
-  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= (long long)npair * 4 * D) return;
-  const int d = (int)(idx % D), row = (int)(idx / D);
-  rows[idx] = ((row & 1) == 0 && (row >> 1) == d) ? 1.0 : 0.0;
-}
-
-// At[m][c] (complex) from launch_sh_angles output [Mc][M] (real or complex basis)
-__global__ void sh_rows_any_kernel(const double* __restrict__ Y, int M, int Mc, int complex_basis,
-                                   cplx* __restrict__ rows) {
-  const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= M * Mc) return;
-  const int m = idx / Mc, c = idx % Mc;
-  rows[idx] = complex_basis ? reinterpret_cast<const cplx*>(Y)[(long long)c * M + m] : mk(Y[(long long)c * M + m], 0.0);
-}
-
 // P[ci][co] = Rshd[co][ci] for Rshd = getSHrotMtx(E, N, 'real'); one CTA
 __global__ void sh_rot_matrix_kernel(int order, Rot1 R1in, double* __restrict__ P) {
   extern __shared__ double rot_Rr[];
@@ -379,13 +363,6 @@ __global__ void symmetric_spectrum_kernel(const cplx* __restrict__ W, int K, int
   out[i] = W[i < K ? i : nfft - i].x;
 }
 
-std::vector<double> kr_table(const emagls_config& cfg, double fs, double radius, int K) {
-  std::vector<double> kr(K);
-  const double df = (fs / 2.0) / (double)(K - 1);
-  for (int k = 0; k < K; ++k) kr[k] = 2.0 * M_PI * ((double)k * df) / cfg.speed_of_sound * radius;
-  return kr;
-}
-
 int radial_kind_checked(const emagls_radial_params* rp) {
   EM_REQUIRE(rp, "null argument");
   if (rp->kind < EMAGLS_RADIAL_NONE || rp->kind > EMAGLS_RADIAL_FULL)
@@ -457,27 +434,18 @@ void encode_dev(emagls_ctx* h, const emagls_config& cfg, int kind, const double*
   if (kind == 0) {
     double* Y = ar.get<double>((size_t)M * Mc * 2);
     EM_CUDA(launch_sh_angles(st, order, mic_azi, mic_zen, M, cb, Y));
-    sh_rows_any_kernel<<<(M * Mc + 255) / 256, 256, 0, st>>>(Y, M, Mc, cb, At);
-    EM_CUDA(cudaGetLastError());
+    EM_CUDA(launch_sh_rows(st, Y, M, Mc, cb, At));
     h->launches += 2;
   } else {
     EM_CUDA(launch_ch_rows(st, order, mic_azi, M, cb, At));
     h->launches += 1;
   }
-  const int npair = (M + 1) / 2;
-  double* rows = ar.get<double>((size_t)npair * 4 * M);
-  {
-    const long long tot = (long long)npair * 4 * M;
-    unit_rows2_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(rows, npair, M);
-    EM_CUDA(cudaGetLastError());
-  }
-  cplx* Lt = ar.get<cplx>((size_t)2 * npair * Mc);
-  regularized_apply_dev(h, ar, At, M, Mc, rows, npair, 0.0, Lt);
+  cplx* Lt = unclipped_pinv_dev(h, ar, At, M, Mc);
   double* P = ar.get<double>((size_t)M * Mc);
   for (int part = 0; part <= cb; ++part) {
-    extract_enc_kernel<<<(M * Mc + 255) / 256, 256, 0, st>>>(Lt, npair, M, Mc, part, P);
+    extract_enc_kernel<<<(M * Mc + 255) / 256, 256, 0, st>>>(Lt, (M + 1) / 2, M, Mc, part, P);
     EM_CUDA(cudaGetLastError());
-    h->launches += 2;
+    h->launches += 1;
     channel_mix_dev(h, in, n, M, P, Mc, out, cb ? 2 : 1, part);
   }
 }
@@ -514,12 +482,12 @@ void rotate_sh_dev(emagls_ctx* h, const double* in, long long n, int order, doub
 // getMagLsSphericalHeadFilter (mics == nullptr) / getMagLsArrayDiffuseFilter; w [len], Wfull [nfft] or nullptr
 void diffuse_filter_dev(emagls_ctx* h, const emagls_config& cfg, double radius, const double* mic_azi,
                         const double* mic_zen, int M, int order, double fs, int len, double* w, double* Wfull) {
-  EM_REQUIRE(w && len > 0 && len % 2 == 0, "len must be even");
+  EM_REQUIRE(w && len > 0, "empty input");
   cudaStream_t st = h->stream;
   Arena ar(st);
-  const int nfft = std::min(cfg.nfft_max_len, 2 * len);
-  EM_REQUIRE(nfft % 2 == 0 && nfft / 2 >= len / 2, "len exceeds NFFT_MAX_LEN (reference indexes out of range here)");
-  const int K = nfft / 2 + 1;
+  const BinGrid bg = bin_grid(cfg, len, fs, 0);
+  EM_REQUIRE(bg.nfft % 2 == 0, "nfft must be even");
+  const int nfft = bg.nfft, K = bg.K;
   const int simN = (int)std::ceil(fs * M_PI * radius / cfg.speed_of_sound);   // no max(order, .) here (:38)
   EM_REQUIRE(simN <= MAX_SH_ORDER && order <= MAX_SH_ORDER, "simulation order too high");
   EM_REQUIRE(order <= simN, "order above the simulation order (reference indexes out of range here)");
@@ -686,7 +654,7 @@ int emagls_spherical_head_filter(emagls_handle h, const emagls_config* cfg, doub
     EM_REQUIRE(cfg && w && len > 0, "null argument");
     cudaStream_t st = h->stream;
     Arena ar(st);
-    const int nfft = std::min(cfg->nfft_max_len, 2 * len);
+    const int nfft = bin_grid(*cfg, len, fs, 0).nfft;
     double* d_w = ar.get<double>(len);
     double* d_W = W_full ? ar.get<double>(nfft) : nullptr;
     diffuse_filter_dev(h, *cfg, mic_radius, nullptr, nullptr, 0, order, fs, len, d_w, d_W);

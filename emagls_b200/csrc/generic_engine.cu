@@ -281,6 +281,26 @@ static void run_generic(emagls_ctx* h, Arena& ar, const GenericProblem& g) {
   }
 }
 
+// Hc [set][ear][K][D]: HRIR spectra as complex rows (hrir_spectrum), (set, ear) advanced by delays[set * 2 + ear]
+static cplx* hrir_spectra_rows(emagls_ctx* h, Arena& ar, const double* hL, const double* hR, int T, int D, int K,
+                               int nfft, int num_sets, const std::vector<double>& delays) {
+  cudaStream_t st = h->stream;
+  cplx* Hc = ar.get<cplx>((size_t)num_sets * 2 * K * D);
+  double* tw = ar.get<double>((size_t)2 * K * T);
+  EM_CUDA(launch_dft_twiddle(st, K, T, nfft, tw));
+  double* Hd = ar.get<double>((size_t)D * 2 * K);
+  for (int s = 0; s < num_sets; ++s)
+    for (int e = 0; e < 2; ++e) {
+      hrir_spectrum(h, ar, (e ? hR : hL) + (size_t)s * T * D, T, D, K, tw, delays[(size_t)s * 2 + e], Hd);
+      dim3 grid((K + 31) / 32, (D + 31) / 32), block(32, 8);
+      spectrum_rows_kernel<<<grid, block, 0, st>>>(Hd, D, K, Hc + ((size_t)s * 2 + e) * K * D);
+      EM_CUDA(cudaGetLastError());
+      h->launches += 1;
+    }
+  h->launches += 1;
+  return Hc;
+}
+
 // tail of the SH-domain designers without the sphere model: real tail GEMM (+ basis change)
 static void tail_real(emagls_ctx* h, Arena& ar, const cplx* Wsp, int P, int Mc, int K, int nfft, int len,
                       double delayL, double delayR, double* wL, double* wR) {
@@ -357,33 +377,14 @@ void design_magls(emagls_ctx* h, const emagls_config& cfg, const double* hL, con
     }
     return;
   }
-  EM_REQUIRE(len >= T, "HRIR len too short");  // lib/getMagLsFilters.m:38
-  EM_REQUIRE(len % 2 == 0, "len must be even");
-  const int nfft = std::min(cfg.nfft_max_len, 2 * len);
-  EM_REQUIRE(nfft / 2 >= len / 2, "len exceeds NFFT_MAX_LEN (reference indexes out of range here)");
-  const int K = nfft / 2 + 1;
-  const double df = (fs / 2.0) / (double)(K - 1);
-  const int k_cut = (int)std::ceil(std::max(cfg.f_cut_min, 500.0 * order) / df);
-  const int kls1 = std::min(std::max(k_cut - 1, 1), K);
+  const BinGrid bg = bin_grid(cfg, len, fs, T);   // lib/getMagLsFilters.m:38
+  const int nfft = bg.nfft, K = bg.K;
+  const int kls1 = bg.kls1(std::max(cfg.f_cut_min, 500.0 * order));
   // HRTF-set batch (extension, not in the reference API): the one pinv(Y) operator serves every set, the sets are
   // independent problems of the chain kernel (lib/getMagLsFilters.m:48,64-72)
   const int NS = num_sets;
   const std::vector<double> grpD = group_delays(h, ar, hL, hR, T, D, K, fs, NS);
-  cplx* Hc = ar.get<cplx>((size_t)NS * 2 * K * D);
-  {
-    double* tw = ar.get<double>((size_t)2 * K * T);
-    EM_CUDA(launch_dft_twiddle(st, K, T, nfft, tw));
-    double* Hd = ar.get<double>((size_t)D * 2 * K);
-    for (int s_ = 0; s_ < NS; ++s_)
-      for (int e = 0; e < 2; ++e) {
-        hrir_spectrum(h, ar, (e ? hR : hL) + (size_t)s_ * T * D, T, D, K, tw, grpD[(size_t)s_ * 2 + e], Hd);
-        dim3 grid((K + 31) / 32, (D + 31) / 32), block(32, 8);
-        spectrum_rows_kernel<<<grid, block, 0, st>>>(Hd, D, K, Hc + ((size_t)s_ * 2 + e) * K * D);
-        EM_CUDA(cudaGetLastError());
-        h->launches += 1;
-      }
-    h->launches += 1;
-  }
+  cplx* Hc = hrir_spectra_rows(h, ar, hL, hR, T, D, K, nfft, NS, grpD);
   setup_span.reset();
   cplx* Wsp = spectra ? reinterpret_cast<cplx*>(spectra) : ar.get<cplx>((size_t)2 * NS * Mc * K);
   g.K = K; g.first_bin = 0; g.kls1 = kls1; g.dc_fix = 0; g.nyquist_real = 1;   // lib/getMagLsFilters.m:64-72
@@ -437,17 +438,13 @@ void design_from_atf(emagls_ctx* h, const emagls_config& cfg, const double* hL, 
   // nearest-neighbour-selected HRTF columns (:82-95) differ, which the chain kernel gathers on the fly.
   cudaStream_t st = h->stream;
   EM_REQUIRE(T > 0 && D > 0 && Ta > 0 && M > 0 && Da > 0 && len > 0, "empty input");
-  EM_REQUIRE(len >= T, "len too short");
-  EM_REQUIRE(len % 2 == 0, "filterLen must be even");
+  const BinGrid bg = bin_grid(cfg, len, fs, T);
+  EM_REQUIRE(bg.nfft % 2 == 0, "nfft must be even");
   EM_REQUIRE(M <= 64, "more than 64 channels are not supported");
   EM_REQUIRE(num_orient >= 1 && (rotations != nullptr || num_orient == 1), "num_orient > 1 needs rotations");
   const int B = num_orient;
-  const int nfft = std::min(cfg.nfft_max_len, 2 * len);
-  EM_REQUIRE(nfft % 2 == 0 && nfft / 2 >= len / 2, "len exceeds NFFT_MAX_LEN (reference indexes out of range here)");
-  const int K = nfft / 2 + 1;
-  const double df = (fs / 2.0) / (double)(K - 1);
-  const int kTrans = (int)std::ceil(f_trans / df);          // lib/getEMagLsFiltersFromAtf.m:38
-  const int kls1 = std::min(std::max(kTrans - 1, 1), K);
+  const int nfft = bg.nfft, K = bg.K;
+  const int kls1 = bg.kls1(f_trans);                        // lib/getEMagLsFiltersFromAtf.m:38
   const bool hrtf_smaller = D <= Da;                        // min() picks the first on a tie (:62)
   const int Dn = std::min(D, Da);
   EM_REQUIRE(Dn >= M, "fewer directions than microphones");
@@ -469,19 +466,7 @@ void design_from_atf(emagls_ctx* h, const emagls_config& cfg, const double* hL, 
   h->launches += 3;
   // ---- HRIRs: integer group-delay removal (:42-49), spectra
   const std::vector<double> grpD = group_delays(h, ar, hL, hR, T, D, K, fs, 1);
-  cplx* Hfull = ar.get<cplx>((size_t)2 * K * D);
-  {
-    double* tw = ar.get<double>((size_t)2 * K * T);
-    EM_CUDA(launch_dft_twiddle(st, K, T, nfft, tw));
-    double* Hd = ar.get<double>((size_t)D * 2 * K);
-    for (int e = 0; e < 2; ++e) {
-      hrir_spectrum(h, ar, e ? hR : hL, T, D, K, tw, matlab_round(grpD[e]), Hd);
-      dim3 grid((K + 31) / 32, (D + 31) / 32), block(32, 8);
-      spectrum_rows_kernel<<<grid, block, 0, st>>>(Hd, D, K, Hfull + (size_t)e * K * D);
-      EM_CUDA(cudaGetLastError());
-    }
-    h->launches += 3;
-  }
+  cplx* Hfull = hrir_spectra_rows(h, ar, hL, hR, T, D, K, nfft, 1, {matlab_round(grpD[0]), matlab_round(grpD[1])});
   // ---- ATF spectra (:54)
   const int Tu = std::min(Ta, nfft);   // fft(x, nfft) truncates longer responses
   double* Ad = ar.get<double>((size_t)M * Da * 2 * K);
@@ -538,33 +523,16 @@ void design_from_atf(emagls_ctx* h, const emagls_config& cfg, const double* hL, 
 // ------------------------------------------------------------------------------------------
 // getEMagLsFiltersEMAinSH (all pointers on the device)
 // ------------------------------------------------------------------------------------------
-namespace {
-__global__ void fill_value_kernel(double* p, int n, double v) {
-  int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) p[i] = v;
-}
-__global__ void identity_rows2_kernel(double* rows, int npair, int D) {
-  long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= (long long)npair * 4 * D) return;
-  const int d = (int)(idx % D), row = (int)(idx / D);
-  rows[idx] = ((row & 1) == 0 && (row >> 1) == d) ? 1.0 : 0.0;
-}
-}  // namespace
-
 void design_ema_sh(emagls_ctx* h, const emagls_config& cfg, const double* hL, const double* hR, int T, int D,
                    const double* grid_azi, const double* grid_zen, double mic_radius, const double* mic_azi, int M,
                    int order, double fs, int len, double* wL, double* wR, double* spectra) {
   cudaStream_t st = h->stream;
   EM_REQUIRE(T > 0 && D > 0 && M > 0 && len > 0, "empty input");
-  EM_REQUIRE(len >= T, "len too short");
-  EM_REQUIRE(len % 2 == 0, "len must be even");
-  const int nfft = std::min(cfg.nfft_max_len, 2 * len);
-  EM_REQUIRE(nfft % 2 == 0 && nfft / 2 >= len / 2, "len exceeds NFFT_MAX_LEN (reference indexes out of range here)");
-  const int K = nfft / 2 + 1;
-  const double df = (fs / 2.0) / (double)(K - 1);
-  const int k_cut = (int)std::ceil(std::max(cfg.f_cut_min, 500.0 * order) / df);
-  const int kls1 = std::min(std::max(k_cut - 1, 1), K);
-  const int simN = std::max(order, (int)std::ceil(fs * M_PI * mic_radius / cfg.speed_of_sound));
+  const BinGrid bg = bin_grid(cfg, len, fs, T);
+  EM_REQUIRE(bg.nfft % 2 == 0, "nfft must be even");
+  const int nfft = bg.nfft, K = bg.K;
+  const int kls1 = bg.kls1(std::max(cfg.f_cut_min, 500.0 * order));
+  const int simN = sim_order(cfg, order, fs, mic_radius);
   EM_REQUIRE(simN <= MAX_SH_ORDER, "simulation order too high");
   const int S = (simN + 1) * (simN + 1), nsh = (order + 1) * (order + 1), nch = 2 * order + 1;
   EM_REQUIRE(nsh <= 64, "more than 64 channels are not supported");
@@ -574,13 +542,12 @@ void design_ema_sh(emagls_ctx* h, const emagls_config& cfg, const double* hL, co
   Arena ar(st);
   std::optional<ProfSpan> setup_span(std::in_place, h, EM_PROF_SETUP);
   // ---- array model pieces
-  std::vector<double> kr(K);
-  for (int k = 0; k < K; ++k) kr[k] = 2.0 * M_PI * ((double)k * df) / cfg.speed_of_sound * mic_radius;
+  const std::vector<double> kr = kr_table(cfg, fs, mic_radius, K);
   cplx* bn = ar.get<cplx>((size_t)K * (simN + 1));
   EM_CUDA(launch_modal(st, simN, ar.upload(kr.data(), K), K, cfg.array_type, -1.0, 1, bn, simN + 1, 1));
   const int nmax = std::max(std::max(M, D), 1);
   double* halfpi = ar.get<double>(nmax);
-  fill_value_kernel<<<(nmax + 127) / 128, 128, 0, st>>>(halfpi, nmax, 1.5707963267948966);
+  EM_CUDA(launch_fill(st, halfpi, nmax, 1.5707963267948966));
   double* Ym = ar.get<double>((size_t)M * S);
   EM_CUDA(launch_sh_mics(st, simN, mic_azi, halfpi, M, nullptr, 1, Ym));
   double* Yhor = ar.get<double>((size_t)S * D);
@@ -594,34 +561,15 @@ void design_ema_sh(emagls_ctx* h, const emagls_config& cfg, const double* hL, co
   // pinv(YCh.') through the factorisation kernel with the clip disabled
   cplx* Ach = ar.get<cplx>((size_t)M * nch);
   EM_CUDA(launch_ch_rows(st, order, mic_azi, M, cplx_out ? 1 : 0, Ach));
-  const int npair = (M + 1) / 2;
-  double* rows = ar.get<double>((size_t)npair * 4 * M);
-  {
-    long long n = (long long)npair * 4 * M;
-    identity_rows2_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(rows, npair, M);
-  }
-  cplx* pinvT = ar.get<cplx>((size_t)2 * npair * nch);
-  regularized_apply_dev(h, ar, Ach, M, nch, rows, npair, 0.0, pinvT);
+  cplx* pinvT = unclipped_pinv_dev(h, ar, Ach, M, nch);
   cplx* dec = ar.get<cplx>((size_t)M * nsh);
-  EM_CUDA(launch_ema_dec(st, order, M, npair, cplx_out ? 1 : 0, Ysh0, pinvT, dec));
+  EM_CUDA(launch_ema_dec(st, order, M, (M + 1) / 2, cplx_out ? 1 : 0, Ysh0, pinvT, dec));
   cplx* At = ar.get<cplx>((size_t)(K - 1) * D * nsh);
   EM_CUDA(launch_ema_sh_rows(st, order, simN, M, D, K, cplx_out ? 1 : 0, grid_azi, grid_zen, dec, Ym, Yhor, bn, At));
-  h->launches += 9;
+  h->launches += 8;
   // ---- HRIRs
   const std::vector<double> grpD = group_delays(h, ar, hL, hR, T, D, K, fs, 1);
-  cplx* Hc = ar.get<cplx>((size_t)2 * K * D);
-  {
-    double* tw = ar.get<double>((size_t)2 * K * T);
-    EM_CUDA(launch_dft_twiddle(st, K, T, nfft, tw));
-    double* Hd = ar.get<double>((size_t)D * 2 * K);
-    for (int e = 0; e < 2; ++e) {
-      hrir_spectrum(h, ar, e ? hR : hL, T, D, K, tw, grpD[e], Hd);
-      dim3 grid((K + 31) / 32, (D + 31) / 32), block(32, 8);
-      spectrum_rows_kernel<<<grid, block, 0, st>>>(Hd, D, K, Hc + (size_t)e * K * D);
-      EM_CUDA(cudaGetLastError());
-    }
-    h->launches += 3;
-  }
+  cplx* Hc = hrir_spectra_rows(h, ar, hL, hR, T, D, K, nfft, 1, grpD);
   setup_span.reset();
   cplx* Wsp = spectra ? reinterpret_cast<cplx*>(spectra) : ar.get<cplx>((size_t)2 * nsh * K);
   EM_CUDA(cudaMemsetAsync(Wsp, 0, (size_t)2 * nsh * K * sizeof(cplx), st));

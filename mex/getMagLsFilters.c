@@ -13,6 +13,6 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
   mxArray* wL = emx_out(len, nsh, cfg.basis); mxArray* wR = emx_out(len, nsh, cfg.basis);
   emx_check(emagls_design_magls(emx_handle(), &cfg, mxGetDoubles(prhs[0]), mxGetDoubles(prhs[1]), T, D,
                                 mxGetDoubles(prhs[2]), mxGetDoubles(prhs[3]), order, mxGetScalar(prhs[5]), len,
-                                emx_ptr(wL), emx_ptr(wR), NULL));   /* 'HRIR len too short' on len < size(hL,1) */
+                                emx_ptr(wL), emx_ptr(wR), NULL));   /* 'len too short' on len < size(hL,1) */
   emx_return2(nlhs, plhs, wL, wR);
 }

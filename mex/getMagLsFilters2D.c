@@ -12,6 +12,6 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
   mxArray* wL = emx_out(len, nch, cfg.basis); mxArray* wR = emx_out(len, nch, cfg.basis);
   emx_check(emagls_design_magls_2d(emx_handle(), &cfg, mxGetDoubles(prhs[0]), mxGetDoubles(prhs[1]), T, D,
                                    mxGetDoubles(prhs[2]), order, mxGetScalar(prhs[4]), len, emx_ptr(wL), emx_ptr(wR),
-                                   NULL));   /* 'HRIR len too short' on len < size(hLHor,1) */
+                                   NULL));   /* 'len too short' on len < size(hLHor,1) */
   emx_return2(nlhs, plhs, wL, wR);
 }
