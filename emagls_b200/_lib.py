@@ -85,6 +85,14 @@ SIGNATURES = {
     "emagls_binaural_decode_sh_tracked_dev": (C.c_int, [C.c_void_p, c_dp, C.c_longlong, C.c_int, c_dp, c_dp, C.c_int,
                                                         c_dp, C.c_longlong, C.c_int, C.c_int, C.c_longlong, C.c_int,
                                                         c_dp]),
+    "emagls_render_stream_create": (C.c_int, [C.c_void_p, c_dp, c_dp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                              C.c_int, C.POINTER(C.c_void_p)]),
+    "emagls_render_stream_create_sh": (C.c_int, [C.c_void_p, c_dp, c_dp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                                 C.POINTER(C.c_void_p)]),
+    "emagls_render_stream_process": (C.c_int, [C.c_void_p, c_dp, C.c_longlong, C.c_void_p, c_dp, C.c_longlong, c_dp]),
+    "emagls_render_stream_process_dev": (C.c_int, [C.c_void_p, c_dp, C.c_longlong, C.c_void_p, c_dp, C.c_longlong,
+                                                   c_dp]),
+    "emagls_render_stream_destroy": (C.c_int, [C.c_void_p]),
     "emagls_get_sh": (C.c_int, [C.c_void_p, C.c_int, c_dp, c_dp, C.c_int, C.c_int, c_dp]),
     "emagls_group_delay": (C.c_int, [C.c_void_p, c_dp, C.c_int, C.c_int, C.c_int, C.c_double, c_dp, c_dp]),
     "emagls_sph_modal_coeffs": (C.c_int, [C.c_void_p, C.c_int, c_dp, C.c_int, C.c_int, c_dp]),

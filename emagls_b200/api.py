@@ -23,7 +23,7 @@ from ._lib import Config, EmaglsError, Handle, RadialParams, default_handle  # n
 
 __all__ = ["getEMagLs2Filters", "getEMagLsFilters", "getMagLsFilters", "getLsFilters",
            "getEMagLsFiltersFromAtf", "getEMagLsFiltersEMAinCH", "getEMagLsFiltersEMAinSH",
-           "getSMAIRMatrix", "binauralDecode", "binauralDecodeTracked", "binauralDecodeShTracked", "getSH", "sphModalCoeffs", "regularizedApply", "grpdelay",
+           "getSMAIRMatrix", "binauralDecode", "binauralDecodeTracked", "binauralDecodeShTracked", "RenderStream", "ShRenderStream", "getSH", "sphModalCoeffs", "regularizedApply", "grpdelay",
            "getRadialFilter", "applyRadialFilter", "encodeSH", "encodeCH", "rotateSH", "getMagLsFilters2D",
            "getMagLsSphericalHeadFilter", "getMagLsArrayDiffuseFilter", "Handle", "EmaglsError"]
 
@@ -501,6 +501,118 @@ def binauralDecodeShTracked(inp, wL, wR, rotations, hop, fade=None, compensateDe
     h.check(h.lib.emagls_binaural_decode_sh_tracked(h.ptr, _p(x), n, N, _p(wl), _p(wr), ln, _p(R), R.shape[0], hop,
                                                     fade, int(firstSample), 1 if compensateDelay else 0, _p(out)))
     return out
+
+
+class _Session:
+    """One render session (emagls_render_stream_*): owns the C session and frees it on close()."""
+
+    def __init__(self, h, ptr, num_ch):
+        self.handle = h
+        self._s = ptr
+        self.num_ch = num_ch
+
+    @property
+    def ptr(self):
+        if not self._s:
+            raise ValueError("the render session is closed")
+        return self._s
+
+    def close(self):
+        # a closed handle has already freed its sessions (emagls_destroy)
+        if getattr(self, "_s", None) and self.handle.ptr:
+            self.handle.check(self.handle.lib.emagls_render_stream_destroy(self._s))
+        self._s = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def _process(self, x, track, rotations, nnew):
+        x = _f(x)
+        if x.ndim != 2 or x.shape[1] != self.num_ch:
+            raise ValueError(f"x must be [samples, {self.num_ch}]")
+        out = np.zeros((x.shape[0], 2), order="F")
+        h = self.handle
+        h.check(h.lib.emagls_render_stream_process(self.ptr, _p(x), x.shape[0], _p(track), _p(rotations), nnew, _p(out)))
+        return out
+
+
+class RenderStream(_Session):
+    """Render session of the static render or the head-tracked bank render (not in the reference API;
+    emagls_render_stream_create): ``wL``, ``wR`` [len, ch] (static) or [len, ch, pages] (bank).  ``process(x, track)``
+    renders the next ``x`` [n, ch] (n a multiple of ``block``) and returns [n, 2]; ``track`` holds the next tracker
+    entries (0-based pages of frames of ``hop`` samples, crossfaded over ``fade`` samples, default ``hop``).  The
+    concatenated outputs equal binauralDecode / binauralDecodeTracked of the concatenated input."""
+
+    def __init__(self, wL, wR, block, hop=None, fade=None, *, handle=None):
+        h = handle or default_handle()
+        wl, wr = _f(wL), _f(wR)
+        if wl.ndim == 2:
+            wl, wr = wl[:, :, None], wr[:, :, None]
+        if wl.shape != wr.shape or wl.ndim != 3:
+            raise ValueError("wL, wR must be [len, ch] or [len, ch, pages] of equal shape")
+        wl, wr = np.asfortranarray(wl), np.asfortranarray(wr)
+        ln, ch, pages = wl.shape
+        if pages > 1 and hop is None:
+            raise ValueError("a bank session needs hop")
+        hop = 1 if hop is None else int(hop)
+        fade = (hop if pages > 1 else 0) if fade is None else int(fade)
+        s = C.c_void_p()
+        h.check(h.lib.emagls_render_stream_create(h.ptr, _p(wl), _p(wr), ln, ch, pages, int(block), hop, fade,
+                                                  C.byref(s)))
+        super().__init__(h, s, ch)
+        self.block, self.hop, self.fade, self.pages = int(block), hop, fade, pages
+
+    def process(self, x, track=None):
+        trk, n = None, 0
+        if track is not None:
+            trk = np.ascontiguousarray(np.asarray(track).ravel())
+            if not np.issubdtype(trk.dtype, np.integer) or (trk.size and (trk.min() < -2**31 or trk.max() >= 2**31)):
+                raise ValueError("track must hold integer page numbers")
+            trk = trk.astype(np.int32)
+            n = trk.size
+        return self._process(x, trk, None, n)
+
+
+class ShRenderStream(_Session):
+    """Render session of the SH head-tracked render (not in the reference API; emagls_render_stream_create_sh): one
+    filter pair ``wL``, ``wR`` [len, (order+1)^2]; ``process(x, rotations)`` renders the next ``x`` [n, (order+1)^2]
+    (n a multiple of ``block``) with the next head orientations ``rotations`` [k, 3, 3] (one per frame of ``hop``
+    samples) and returns [n, 2].  The concatenated outputs equal binauralDecodeShTracked of the concatenated input."""
+
+    def __init__(self, wL, wR, block, hop, fade=None, *, handle=None):
+        h = handle or default_handle()
+        wl, wr = _f(wL), _f(wR)
+        if wl.shape != wr.shape or wl.ndim != 2:
+            raise ValueError("wL, wR must be [len, (order+1)^2] of equal shape")
+        ln, ch = wl.shape
+        order = int(round(np.sqrt(ch))) - 1
+        if order < 0 or (order + 1) ** 2 != ch:
+            raise ValueError("the channel count of the filters is not a square (order+1)^2")
+        hop = int(hop)
+        fade = hop if fade is None else int(fade)
+        s = C.c_void_p()
+        h.check(h.lib.emagls_render_stream_create_sh(h.ptr, _p(wl), _p(wr), ln, order, int(block), hop, fade,
+                                                     C.byref(s)))
+        super().__init__(h, s, ch)
+        self.block, self.hop, self.fade, self.order = int(block), hop, fade, order
+
+    def process(self, x, rotations=None):
+        R, n = None, 0
+        if rotations is not None:
+            R = np.ascontiguousarray(np.asarray(rotations, dtype=np.float64))
+            if R.ndim != 3 or R.shape[1:] != (3, 3):
+                raise ValueError("rotations must be [frames, 3, 3]")
+            n = R.shape[0]
+        return self._process(x, None, R, n)
 
 
 # ---- callers either side of the hot path (SURVEY.md section 8(f)) --------------------------------

@@ -10,7 +10,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libemagls_cuda.so")
-SOURCES = ["setup_kernels.cu", "solver_kernels.cu", "tsqr_kernels.cu", "gram_kernels.cu", "ozaki_kernels.cu", "ema_kernels.cu", "engine.cu", "generic_engine.cu", "render.cu", "tracked_render.cu", "sh_tracked_render.cu", "frontend.cu", "api.cu"]
+SOURCES = ["setup_kernels.cu", "solver_kernels.cu", "tsqr_kernels.cu", "gram_kernels.cu", "ozaki_kernels.cu", "ema_kernels.cu", "engine.cu", "generic_engine.cu", "render.cu", "tracked_render.cu", "sh_tracked_render.cu", "stream_render.cu", "frontend.cu", "api.cu"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 
 

@@ -86,6 +86,7 @@ int emagls_destroy(emagls_handle h) {
   cudaSetDevice(h->device);
   cudaStreamSynchronize(h->stream);
   for (cudaEvent_t e : h->ev_pool) cudaEventDestroy(e);
+  emagls::destroy_render_streams(h);
   emagls::destroy_render_plans(h);
   emagls::destroy_fir_plans(h);
   unregister_stream_pool(h->stream);

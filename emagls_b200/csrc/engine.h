@@ -53,6 +53,8 @@ struct emagls_ctx {
   // per-channel FIR of the front end (frontend.cu): cuFFT plans keyed by (size, batch, direction)
   struct FirPlan { int N, batch, inverse, plan; };
   std::vector<FirPlan> fir_plans;
+  // render sessions opened on this handle (stream_render.cu); emagls_destroy frees those still open
+  std::vector<emagls_stream_ctx*> render_streams;
 };
 
 namespace emagls {
@@ -212,6 +214,7 @@ cudaError_t launch_fill(cudaStream_t st, double* p, int n, double v);
 cudaError_t launch_sh_rows(cudaStream_t st, const double* Y, int M, int S, int complex_basis, cplx* rows);
 void destroy_render_plans(emagls_ctx* h);  // render.cu (static and head-tracked render)
 void destroy_fir_plans(emagls_ctx* h);     // frontend.cu
+void destroy_render_streams(emagls_ctx* h);  // stream_render.cu
 // radFilts [K][(order+1)] (row index k) on the device (getRadialFilter.m:42-70)
 void radial_filter_dev(emagls_ctx* h, Arena& ar, const emagls_config& cfg, const emagls_radial_params& rp, int order,
                        double fs, double radius, int nfft, int nan_to_zero, cplx* out);

@@ -1,5 +1,6 @@
 // Overlap-save machinery shared by the static render (render.cu) and the head-tracked render (tracked_render.cu):
-// cuFFT plan caches and the forward transforms of the input blocks.
+// cuFFT plan caches and the forward transforms of the input blocks; the SH rotation stage shared by the SH
+// head-tracked render and the render sessions.
 #pragma once
 #include <cufft.h>
 #include <string>
@@ -29,6 +30,29 @@ void drop_plans(emagls_ctx::RenderPlans& rp);
 // out_rows = num_samples - skip; the SH head-tracked render writes one time chunk into a longer output with it.
 void binaural_decode_rows(emagls_ctx* h, const double* in, long long num_samples, int num_ch, const double* wL,
                           const double* wR, int len, long long skip, long long out_rows, double* out);
+
+// ---- sound-field rotation of the SH head-tracked render (sh_tracked_render.cu), shared with the render sessions
+// (stream_render.cu)
+
+// doubles of the block-diagonal part of a rotation matrix: sum_{l <= order} (2l + 1)^2, and the offset of band l
+__host__ __device__ constexpr int band_offset(int l) { return l * (4 * l * l - 1) / 3; }
+
+// Q[j][band_offset(l) + r (2l+1) + c] = getSHrotMtx(rot[f], order, 'real')[l^2 + r][l^2 + c] for frame f = f_base + j,
+// and same[j] = 1 when rot[f] is bitwise equal to rot[f - 1] (rot[k] holds frame rot_base + k)
+__global__ void frame_rotations_kernel(const double* __restrict__ rot, long long rot_base, long long f_base, int order,
+                                       double* __restrict__ Q, int* __restrict__ same);
+// out[ch][q] = (in[h0 + q, :] @ M)[ch] for q < m with the blended frame matrices of the contract; in has leading
+// dimension ld_in and in[0] sits at first_sample on the track's time axis; Q and same hold frames f_base ...
+__global__ void sh_track_rotate_kernel(const double* __restrict__ in, long long ld_in, long long h0, long long m,
+                                       int order, const double* __restrict__ Q, const int* __restrict__ same,
+                                       long long f_base, long long first_sample, int hop, int fade,
+                                       double* __restrict__ out);
+// the two kernels above for nfr frames / m samples on h->stream (launch counting and profiling are the caller's)
+void launch_frame_rotations(emagls_ctx* h, const double* rot, long long rot_base, long long f_base, long long nfr,
+                            int order, double* Q, int* same);
+void launch_sh_track_rotate(emagls_ctx* h, const double* in, long long ld_in, long long h0, long long m, int order,
+                            const double* Q, const int* same, long long f_base, long long first_sample, int hop,
+                            int fade, double* out);
 
 // Forward transforms of the overlap-save blocks of a multichannel signal into X[ch][nbc][F].  Block b takes the N
 // input samples starting at b*L - ov.  Direct route (default when every channel of the signal is 16-byte aligned):

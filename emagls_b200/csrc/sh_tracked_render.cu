@@ -16,8 +16,7 @@ constexpr int SHT_MAX_ORDER = 7;   // (order + 1)^2 <= 64 channels, as emagls_ro
 constexpr int SHT_T = 128;         // threads per CTA of the rotation kernel
 constexpr int SHT_S = 4;           // samples per thread (strided by 32: every load and store is a 256-byte row)
 
-// doubles of the block-diagonal part of a rotation matrix: sum_{l <= order} (2l + 1)^2, and the offset of band l
-__host__ __device__ constexpr int band_offset(int l) { return l * (4 * l * l - 1) / 3; }
+}  // namespace
 
 // Q[j][band_offset(l) + r (2l+1) + c] = getSHrotMtx(rot[f], order, 'real')[l^2 + r][l^2 + c] for frame f = f_base + j
 // (blockIdx.x), and same[j] = 1 when rot[f] is bitwise equal to rot[f - 1].  rot[k] holds frame rot_base + k.
@@ -154,6 +153,25 @@ sh_track_rotate_kernel(const double* __restrict__ in, long long ld_in, long long
     rotate_samples<1>(in, ld_in, out, m, order, qc, f > 0 ? qc - blk : qc, src1, dst1, ok1, g1, blend1);
   }
 }
+
+void launch_frame_rotations(emagls_ctx* h, const double* rot, long long rot_base, long long f_base, long long nfr,
+                            int order, double* Q, int* same) {
+  const int C = (order + 1) * (order + 1);
+  frame_rotations_kernel<<<(unsigned)nfr, 128, (size_t)C * C * sizeof(double), h->stream>>>(rot, rot_base, f_base,
+                                                                                           order, Q, same);
+  EM_CUDA(cudaGetLastError());
+}
+
+void launch_sh_track_rotate(emagls_ctx* h, const double* in, long long ld_in, long long h0, long long m, int order,
+                            const double* Q, const int* same, long long f_base, long long first_sample, int hop,
+                            int fade, double* out) {
+  const long long warps = (m + 32 * SHT_S - 1) / (32 * SHT_S);
+  sh_track_rotate_kernel<<<(unsigned)((warps * 32 + SHT_T - 1) / SHT_T), SHT_T, 0, h->stream>>>(
+      in, ld_in, h0, m, order, Q, same, f_base, first_sample, hop, fade, out);
+  EM_CUDA(cudaGetLastError());
+}
+
+namespace {
 
 void check_sh_tracked_args(const double* in, long long num_samples, int order, const double* wL, const double* wR,
                            int len, const double* rotations, long long num_frames, int hop, int fade,

@@ -282,6 +282,46 @@ int emagls_binaural_decode_sh_tracked_dev(emagls_handle h, const double* in, lon
                                           const double* rotations, long long num_frames, int hop, int fade,
                                           long long first_sample, int compensate_delay, double* out);
 
+/* ---- render sessions: block-by-block streaming of the static and head-tracked renders (not in the reference API) ---
+ * A session belongs to one handle and renders one stream that starts at sample 0 of the track's time axis with zero
+ * history.  Every process call renders the next num_samples samples (a positive multiple of `block`, 16 <= block <=
+ * 8192, any integer) and returns them at once: the session adds no latency beyond the block.  Whatever the split into
+ * calls, after T samples the concatenated outputs equal
+ *   bank session   (num_pages > 1): emagls_binaural_decode_tracked(x[0:T], wL, wR, len, num_pages, track, ..., hop,
+ *                   fade, first_sample = 0, compensate_delay = 0);
+ *   static session (num_pages == 1): emagls_binaural_decode(x[0:T], wL, wR, len, 0) (hop and fade are unused);
+ *   SH session     : emagls_binaural_decode_sh_tracked(x[0:T], order, wL, wR, len, rotations, ..., hop, fade, 0, 0).
+ * (compensate_delay is not offered: drop the first len/2 - 1 output samples.)  hop and fade mean what they mean in
+ * those renders; hop is independent of block.  A process call first appends its num_new_frames tracker entries
+ * (track: int32 pages for bank sessions; rotations: one row-major 3x3 matrix per frame for SH sessions; the other
+ * pointer NULL); after the append the entries must cover frame (T + num_samples - 1) / hop, where T counts the samples
+ * processed before the call.  Further entries are kept as look-ahead.  Calls on a static session pass no entries.
+ * Method (DESIGN.md section 13): uniformly partitioned overlap-save with FFT size 2 block and a frequency-domain delay
+ * line; the spectra of every page and partition are built once at creation and held on the device
+ * (num_pages * 2 * num_ch * ceil(len / block) * (block + 1) * 16 bytes), so a 3600-page em32 bank of 512 taps needs
+ * about 1.9 GB.  Creation copies wL, wR (host memory) and synchronises; a failed allocation leaves no session.
+ * process: in [num_samples x num_ch] and out [num_samples x 2] are host memory and the call synchronises;
+ * process_dev: in and out are device pointers (channel strides num_samples) and the call returns with the work enqueued
+ * on emagls_stream(h); track and rotations are HOST memory in both variants.  Sessions share the handle's stream: calls
+ * on sessions of one handle must not overlap (the handle rule).  emagls_destroy frees sessions still open.
+ * EMAGLS_ERR_INVALID, checked on the host before anything is launched, and a rejected call changes no session state
+ * (appended entries included): create: a null pointer, block outside [16, 8192], hop < 1, fade outside [0, hop],
+ * num_pages < 1, order outside [0, 7]; process: a null pointer, num_samples not a positive multiple of block, entries
+ * that do not cover the call, a page outside [0, num_pages), the wrong kind of tracker pointer for the session, a
+ * track on a static session, num_new_frames < 0.                                                                     */
+typedef struct emagls_stream_ctx* emagls_render_stream;
+int emagls_render_stream_create(emagls_handle h, const double* wL, const double* wR, int len, int num_ch,
+                                int num_pages, int block, int hop, int fade, emagls_render_stream* out);
+int emagls_render_stream_create_sh(emagls_handle h, const double* wL, const double* wR, int len, int order,
+                                   int block, int hop, int fade, emagls_render_stream* out);
+int emagls_render_stream_process(emagls_render_stream s, const double* in, long long num_samples,
+                                 const int32_t* track, const double* rotations, long long num_new_frames,
+                                 double* out);
+int emagls_render_stream_process_dev(emagls_render_stream s, const double* in, long long num_samples,
+                                     const int32_t* track, const double* rotations, long long num_new_frames,
+                                     double* out);
+int emagls_render_stream_destroy(emagls_render_stream s);
+
 /* ======================================================================================================
  * Callers either side of the hot path (SURVEY.md section 8-f): radial filters, SH/CH encoding and
  * rotation of the recording in front of the render, the remaining lib/ designers.
