@@ -7,8 +7,8 @@
 //   once per array      : b_n(kr_k) for all bins                              (getSMAIRMatrix.m:107)
 //   once per HRTF set   : group delays, H = fft(h) .* ramp, |H|, H*Q and H*Y_h for the LS bins
 //   once per orientation: Y_o, E_o = R-blocks * Y_o^T (TSQR route), F_o = Y_o Gh-blocks Y_o^T (Gram route)
-//   per bin k           : Gram route (no singular value clipped, decided by a rigorous bound on
-//                         cond(A_k^H A_k)):  G_k = sum conj(b_n) b_n' F_nn' (DMMA GEMM), Cholesky,
+//   per bin k           : Gram route (no singular value clipped, decided by a rigorous certificate for
+//                         cond(A_k^H A_k)):  G_k = sum conj(b_n) b_n' F_nn' (DMMA GEMM), inversion,
 //                             W_k = ((t Y_h) .* conj(b_k)) Y_o^T G_k^-T
 //                         TSQR route (clipping possible):  C = R diag(b_k) Y_o^T -> TSQR -> Jacobi ->
 //                             W_k = (t Q) conj(Q_C) Pb
@@ -553,7 +553,7 @@ void design_factored(emagls_ctx* h, const emagls_config& cfg, const DesignArgs& 
   const long long v_stride = sep ? 32LL * S : (long long)Mc * S, tau_stride = (long long)bp.nblk * bp.MC,
                   pb_stride = (long long)Mc * Mc;
   const size_t per_orient =
-      (size_t)Etot * 8 + (size_t)(nqs + nqa) * ne_ld * 8 + (size_t)2 * NB * ne_ld * 8 + (size_t)NB * pb_stride * 16 +
+      (size_t)Etot * 8 + (size_t)(nqs + nqa) * ne_ld * 8 + (size_t)2 * NB * ne_ld * 8 + (size_t)NB * pb_stride * 16 + (size_t)NB * 8 +
       (size_t)G * (v_stride + tau_stride + pb_stride + (sep ? 1024 : 0)) * 16 +
       (size_t)a.num_sets * ((size_t)(1 + 6) * 4 * S * 8 + (size_t)4 * D * 8);
   size_t free_b = 0, total_b = 0;
@@ -584,6 +584,7 @@ void design_factored(emagls_ctx* h, const emagls_config& cfg, const DesignArgs& 
   double* Gre = ar.get<double>((size_t)NB * OC * ne_ld);
   double* Gim = ar.get<double>((size_t)NB * OC * ne_ld);
   cplx* PbG = ar.get<cplx>((size_t)NB * OC * pb_stride);
+  double* sigG = ar.get<double>((size_t)NB * OC);   // shift of the condition certificate per matrix (gram_kernels.cu)
   int* d_fail = ar.get<int>(NB + 1);
   OperatorSet ops{};
   ops.v_stride = v_stride; ops.tau_stride = tau_stride; ops.pb_stride = pb_stride;
@@ -608,9 +609,10 @@ void design_factored(emagls_ctx* h, const emagls_config& cfg, const DesignArgs& 
   double* sTt = use_oz ? ar.get<double>((size_t)4 * PJ) : nullptr;
   constexpr int MAX_SPLITS = 6;
   double* tq = ar.get<double>((size_t)MAX_SPLITS * 4 * PJ * S);   // split-K partials of t * Y_h
-  // Gram route admissible iff cond_2(G) <= 1/c^2 (no singular value below c*s_max); the Frobenius
-  // bound is tested with a factor-2 margin, and normal equations are never used beyond cond(G) = 1e4.
-  double gram_thr = (cfg.svd_regul > 0.0) ? std::min(1e4, 0.5 / (cfg.svd_regul * cfg.svd_regul)) : 1e4;
+  // Gram route admissible iff cond_2(G) <= 1/c^2 (no singular value below c*s_max); the certificate of
+  // launch_gram_chol proves cond_2(G) < thr with its own rounding margin, and normal equations are never
+  // used beyond cond(G) = 1e4 (relative error floor about 2e-12 there).
+  double gram_thr = (cfg.svd_regul > 0.0) ? std::min(1e4, 1.0 / (cfg.svd_regul * cfg.svd_regul)) : 1e4;
   if (getenv("EMAGLS_NO_GRAM")) gram_thr = -1.0;
   const bool debug = getenv("EMAGLS_DEBUG_INFO") != nullptr;
   std::vector<int> fail_h(NB + 1);
@@ -663,8 +665,8 @@ void design_factored(emagls_ctx* h, const emagls_config& cfg, const DesignArgs& 
         ProfSpan ps(h, EM_PROF_GRAM);
         EM_CUDA(cudaMemsetAsync(d_fail, 0, (size_t)(NB + 1) * sizeof(int), st));
         assemble_gram(gb0, nb, oc);
-        EM_CUDA(launch_gram_chol(st, Gre, Gim, Mc, oc, ne_ld, nb, gram_thr, PbG, d_fail));
-        h->launches += 1;
+        EM_CUDA(launch_gram_chol(st, Gre, Gim, Mc, oc, ne_ld, nb, gram_thr, PbG, sigG, d_fail));
+        h->launches += 2;
         EM_CUDA(cudaMemcpyAsync(fail_h.data(), d_fail, (size_t)(nb + 1) * sizeof(int), cudaMemcpyDeviceToHost, st));
         EM_CUDA(cudaStreamSynchronize(st));
       }

@@ -9,9 +9,9 @@
 // folded by the symmetries F_n'n = F_nn'^T into a symmetric (Fs) and an antisymmetric (Fa) part:
 //     Re G = sum_{n<=n'} Re(conj(b_n) b_n') Fs_nn',    Im G = sum_{n<n'} Im(conj(b_n) b_n') Fa_nn'
 // (one real GEMM each, [bins x pairs] x [pairs x (orientation, packed lower triangle)]).
-// A warp-per-matrix Cholesky in shared memory then yields G^-1 and the rigorous bound
-// cond_2(G) <= ||G||_F ||G^-1||_F that decides whether the bin may use this route; bins that fail
-// it go through the TSQR + Jacobi kernel (solver_kernels.cu).
+// A warp-per-matrix inversion then yields X = G^-1 and the bound cond_2(G) <= ||G||_F ||X||_F; where that
+// bound alone cannot decide cond_2(G) <= tau, a Cholesky of the shifted matrix sigma I - G does
+// (gram_certify_kernel).  Bins with a refused matrix go through the TSQR + Jacobi kernels.
 #include "kernels.h"
 #include "ozaki.cuh"
 #include "reflect.cuh"
@@ -107,26 +107,42 @@ cudaError_t launch_gram_beta(cudaStream_t st, const cplx* bn, int N, int K, doub
 }
 
 // ---------------------------------------------------------------------------------------------
-// Warp-per-matrix Cholesky, inverse and condition bound.  Matrix id = bin * P + o.
-// Output Pb[id][i][m] = Ginv[m][i] (so that W = v * Pb), fail[bin] += 1 when the route is refused.
+// Warp-per-matrix inverse and route decision.  Matrix id = bin * P + o.
+// Output Pb[id][i][m] = Ginv[m][i] (so that W = v * Pb), fail[1 + bin] += 1 when the route is refused,
+// sig[id] > 0 for a matrix the Frobenius bound leaves undecided (see gram_classify).
 // ---------------------------------------------------------------------------------------------
 constexpr int GC_WPC = 4;
+// Relative margin of the shifted-Cholesky certificate.  It covers the error of the computed inverse
+// (about cond M u < 1e-10 at cond <= 1e4), the backward error of the Cholesky of sigma I - G (about
+// gamma_{M+1} M sigma < 1e-13 sigma) and the rounding of the assembled G.
+constexpr double GRAM_CERT_DELTA = 1e-6;
 
-__global__ void __launch_bounds__(GC_WPC * 32)
-gram_chol_kernel(const double* __restrict__ Gre, const double* __restrict__ Gim, int Mc, int P, int ne_ld,
-                 long long nmat, double thr, cplx* __restrict__ Pb, int* __restrict__ fail) {
-  extern __shared__ __align__(16) unsigned char gsm_raw[];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const long long id = (long long)blockIdx.x * (blockDim.x >> 5) + warp;   // blockDim.x / 32 matrices per CTA
-  if (id >= nmat) return;
-  const int LD = Mc + 1;
+__device__ __forceinline__ void gram_refuse(long long id, int P, int* fail) {
+  atomicAdd(fail, 1);
+  atomicAdd(fail + 1 + (int)(id / P), 1);
+}
+
+// Route decision from condF = ||G||_F ||X||_F, X the computed inverse (one lane per matrix).  ||X||_F >= ||G^-1||_2
+// and ||G||_F >= lambda_max, so condF <= thr proves cond_2(G) <= thr; each factor exceeds its 2-norm by at most
+// sqrt(Mc), so condF > Mc thr proves cond_2(G) > thr.  In between the matrix is a candidate: sig[id] =
+// thr (1 - delta) / ||X||_F <= thr lambda_min, and gram_certify_kernel accepts it iff sigma I - G is positive definite.
+__device__ __forceinline__ void gram_classify(double fro2, double froi2, double thr, int Mc, long long id, int P,
+                                              double* sig, int* fail) {
+  const double xf = sqrt(froi2), condF = sqrt(fro2) * xf;
+  double s = 0.0;
+  if (condF <= thr) {
+  } else if (condF <= Mc * thr) {
+    s = thr * (1.0 - GRAM_CERT_DELTA) / xf;
+  } else {
+    gram_refuse(id, P, fail);
+  }
+  sig[id] = s;
+}
+
+// Packed lower triangle (entry e = m(m+1)/2 + m', m >= m') into the rows of L (leading dimension LD);
+// returns this lane's share of ||G||_F^2.
+__device__ __forceinline__ double gram_load_lower(cplx* L, int LD, const double* gr, const double* gi, int Mc, int lane) {
   const int ne = Mc * (Mc + 1) / 2;
-  cplx* L = reinterpret_cast<cplx*>(gsm_raw) + (size_t)warp * ((size_t)Mc * LD + (Mc + 1) / 2);
-  double* dinv = reinterpret_cast<double*>(L + (size_t)Mc * LD);  // 1 / L[j][j]
-  const double* gr = Gre + id * ne_ld;
-  const double* gi = Gim + id * ne_ld;
-
-  // load the packed lower triangle; ||G||_F^2
   double fro = 0.0;
   for (int e = lane; e < ne; e += 32) {
     int m = (int)((sqrt(8.0 * e + 1.0) - 1.0) * 0.5);
@@ -137,15 +153,15 @@ gram_chol_kernel(const double* __restrict__ Gre, const double* __restrict__ Gim,
     L[m * LD + mp] = mk(re, im);
     fro += (m == mp) ? re * re : 2.0 * fma(re, re, im * im);
   }
-#pragma unroll
-  for (int s = 16; s > 0; s >>= 1) fro += __shfl_xor_sync(0xffffffffu, fro, s);
-  __syncwarp();
+  return fro;
+}
 
-  // right-looking Cholesky, lane = row
-  bool ok = true;
+// Right-looking Cholesky of the lower triangle of L in place, lane = row; dinv[j] = 1 / L[j][j].
+// Returns false at the first pivot that is not positive and finite.
+__device__ __forceinline__ bool chol_lower(cplx* L, int LD, double* dinv, int Mc, int lane) {
   for (int j = 0; j < Mc; ++j) {
     const double d = L[j * LD + j].x;
-    if (!(d > 0.0) || !(d < 1e300)) { ok = false; break; }
+    if (!(d > 0.0) || !(d < 1e300)) return false;   // warp-uniform
     const double ljj = sqrt(d), inv = 1.0 / ljj;
     __syncwarp();
     for (int r = lane; r < Mc; r += 32) {
@@ -168,8 +184,29 @@ gram_chol_kernel(const double* __restrict__ Gre, const double* __restrict__ Gim,
     }
     __syncwarp();
   }
-  if (!ok) {
-    if (lane == 0) atomicAdd(fail, 1), atomicAdd(fail + 1 + (int)(id / P), 1);
+  return true;
+}
+
+// shared memory of one warp of gram_chol_kernel / gram_certify_kernel: L [Mc][Mc + 1] and dinv [Mc]
+__host__ __device__ inline size_t chol_warp_elems(int Mc) { return (size_t)Mc * (Mc + 1) + (Mc + 1) / 2; }
+
+__global__ void __launch_bounds__(GC_WPC * 32)
+gram_chol_kernel(const double* __restrict__ Gre, const double* __restrict__ Gim, int Mc, int P, int ne_ld,
+                 long long nmat, double thr, cplx* __restrict__ Pb, double* __restrict__ sig, int* __restrict__ fail) {
+  extern __shared__ __align__(16) unsigned char gsm_raw[];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const long long id = (long long)blockIdx.x * (blockDim.x >> 5) + warp;   // blockDim.x / 32 matrices per CTA
+  if (id >= nmat) return;
+  const int LD = Mc + 1;
+  cplx* L = reinterpret_cast<cplx*>(gsm_raw) + (size_t)warp * chol_warp_elems(Mc);
+  double* dinv = reinterpret_cast<double*>(L + (size_t)Mc * LD);  // 1 / L[j][j]
+
+  double fro = gram_load_lower(L, LD, Gre + id * ne_ld, Gim + id * ne_ld, Mc, lane);
+#pragma unroll
+  for (int s = 16; s > 0; s >>= 1) fro += __shfl_xor_sync(0xffffffffu, fro, s);
+  __syncwarp();
+  if (!chol_lower(L, LD, dinv, Mc, lane)) {
+    if (lane == 0) { sig[id] = 0.0; gram_refuse(id, P, fail); }
     return;
   }
   // Li = L^-1 (lower), stored transposed in the strict upper triangle: Li[r][c] -> L[c*LD + r]
@@ -208,10 +245,7 @@ gram_chol_kernel(const double* __restrict__ Gre, const double* __restrict__ Gim,
   }
 #pragma unroll
   for (int s = 16; s > 0; s >>= 1) froi += __shfl_xor_sync(0xffffffffu, froi, s);
-  const double condF = sqrt(fro) * sqrt(froi);
-  if (!(condF <= thr)) {
-    if (lane == 0) atomicAdd(fail, 1), atomicAdd(fail + 1 + (int)(id / P), 1);
-  }
+  if (lane == 0) gram_classify(fro, froi, thr, Mc, id, P, sig, fail);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -222,11 +256,11 @@ gram_chol_kernel(const double* __restrict__ Gre, const double* __restrict__ Gim,
 // positive-definiteness test is the same; every step is a full rank-1 update with no triangular load
 // imbalance, no square root and one reciprocal; only the pivot column (512 B per warp) goes through
 // shared memory and is read back as broadcasts.  The k loop is fully unrolled so that the row stays in
-// registers.  Same output and refusal rule as gram_chol_kernel.
+// registers.  Same outputs and route decision as gram_chol_kernel.
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(GC_WPC * 32, 3)
 gram_sweep_kernel(const double* __restrict__ Gre, const double* __restrict__ Gim, int Mc, int P, int ne_ld,
-                  long long nmat, double thr, cplx* __restrict__ Pb, int* __restrict__ fail) {
+                  long long nmat, double thr, cplx* __restrict__ Pb, double* __restrict__ sig, int* __restrict__ fail) {
   __shared__ cplx colbuf[GC_WPC][32];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const long long id = (long long)blockIdx.x * GC_WPC + warp;
@@ -286,7 +320,7 @@ gram_sweep_kernel(const double* __restrict__ Gre, const double* __restrict__ Gim
     }
   }
   if (!ok) {
-    if (lane == 0) atomicAdd(fail, 1), atomicAdd(fail + 1 + (int)(id / P), 1);
+    if (lane == 0) { sig[id] = 0.0; gram_refuse(id, P, fail); }
     return;
   }
   // Ginv = -A;  Pb[m][i] = Ginv[i][m]  (W = v * Pb): lane i writes column i, coalesced over the lanes
@@ -301,29 +335,88 @@ gram_sweep_kernel(const double* __restrict__ Gre, const double* __restrict__ Gim
   }
 #pragma unroll
   for (int s = 16; s > 0; s >>= 1) froi += __shfl_xor_sync(0xffffffffu, froi, s);
-  const double condF = sqrt(fro) * sqrt(froi);
-  if (!(condF <= thr)) {
-    if (lane == 0) atomicAdd(fail, 1), atomicAdd(fail + 1 + (int)(id / P), 1);
+  if (lane == 0) gram_classify(fro, froi, thr, Mc, id, P, sig, fail);
+}
+
+// ---------------------------------------------------------------------------------------------
+// Certificate for the candidates of the inversion kernels (Mc <= 64).  sigma = sig[id] <= thr lambda_min(G), so a
+// Cholesky of sigma I - G with every pivot positive proves lambda_max(G) < sigma, i.e. cond_2(G) < thr; the first
+// pivot that is not positive refuses the matrix.  lambda_max >= max_i G_ii refuses without factoring when a diagonal
+// entry reaches sigma.  Candidates are a few per cent of the matrices and sit in a few neighbouring bins (contiguous
+// ids), so with W warps in the grid warp w reads the 32 ids w + W l (l = lane) per round, which spreads them over all
+// warps, and factors the candidates among them one after the other, skipping those of a bin that is refused already.
+// ---------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(GC_WPC * 32)
+gram_certify_kernel(const double* __restrict__ Gre, const double* __restrict__ Gim, int Mc, int P, int ne_ld,
+                    long long nmat, const double* __restrict__ sig, int* fail) {
+  extern __shared__ __align__(16) unsigned char gsm_raw[];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int LD = Mc + 1;
+  cplx* L = reinterpret_cast<cplx*>(gsm_raw) + (size_t)warp * chol_warp_elems(Mc);
+  double* dinv = reinterpret_cast<double*>(L + (size_t)Mc * LD);
+  const long long nw = (long long)gridDim.x * (blockDim.x >> 5);
+  for (long long base = (long long)blockIdx.x * (blockDim.x >> 5) + warp; base < nmat; base += 32 * nw) {
+    const long long mine = base + nw * lane;
+    const double s_lane = (mine < nmat) ? sig[mine] : 0.0;
+    unsigned cand = __ballot_sync(0xffffffffu, s_lane > 0.0);
+    while (cand) {
+      const int l = __ffs(cand) - 1;
+      cand &= cand - 1;
+      const long long id = base + nw * l;
+      const double s = __shfl_sync(0xffffffffu, s_lane, l);
+      int refused = 0;
+      if (lane == 0) refused = *reinterpret_cast<volatile const int*>(fail + 1 + id / P);
+      if (__shfl_sync(0xffffffffu, refused, 0) != 0) continue;
+      const double* gr = Gre + id * ne_ld;
+      double dmax = 0.0;
+      for (int m = lane; m < Mc; m += 32) dmax = fmax(dmax, gr[m * (m + 1) / 2 + m]);
+#pragma unroll
+      for (int sh = 16; sh > 0; sh >>= 1) dmax = fmax(dmax, __shfl_xor_sync(0xffffffffu, dmax, sh));
+      bool ok = dmax < s;
+      if (ok) {
+        gram_load_lower(L, LD, gr, Gim + id * ne_ld, Mc, lane);
+        __syncwarp();
+        for (int r = lane; r < Mc; r += 32)   // sigma I - G
+          for (int c = 0; c <= r; ++c) {
+            const cplx g = L[r * LD + c];
+            L[r * LD + c] = mk((c == r ? s : 0.0) - g.x, -g.y);
+          }
+        __syncwarp();
+        ok = chol_lower(L, LD, dinv, Mc, lane);
+        __syncwarp();                          // L is reloaded for the next candidate
+      }
+      if (!ok && lane == 0) gram_refuse(id, P, fail);
+    }
   }
 }
 
 cudaError_t launch_gram_chol(cudaStream_t st, const double* Gre, const double* Gim, int Mc, int P,
-                             int ne_ld, int nbins, double thr, cplx* Pb, int* fail) {
+                             int ne_ld, int nbins, double thr, cplx* Pb, double* sig, int* fail) {
+  if (Mc > 64) return cudaErrorInvalidValue;
   const long long nmat = (long long)nbins * P;
-  if (Mc <= 32) {
-    gram_sweep_kernel<<<(unsigned)((nmat + GC_WPC - 1) / GC_WPC), GC_WPC * 32, 0, st>>>(Gre, Gim, Mc, P, ne_ld, nmat, thr,
-                                                                                    Pb, fail);
-    return cudaGetLastError();
-  }
-  size_t per_warp = ((size_t)Mc * (Mc + 1) + (Mc + 1) / 2) * sizeof(cplx);
+  const size_t per_warp = chol_warp_elems(Mc) * sizeof(cplx);
   // as many warps (matrices) per CTA as the 227 KB of shared memory hold (4 up to Mc = 58, 3 at Mc = 64)
   int wpc = GC_WPC;
   while (wpc > 1 && per_warp * wpc > 227 * 1024) --wpc;
-  size_t smem = per_warp * wpc;
-  const cudaError_t e = allow_dynamic_smem(gram_chol_kernel, smem);
+  const size_t smem = per_warp * wpc;
+  if (Mc <= 32) {
+    gram_sweep_kernel<<<(unsigned)((nmat + GC_WPC - 1) / GC_WPC), GC_WPC * 32, 0, st>>>(Gre, Gim, Mc, P, ne_ld, nmat, thr,
+                                                                                    Pb, sig, fail);
+  } else {
+    const cudaError_t e = allow_dynamic_smem(gram_chol_kernel, smem);
+    if (e != cudaSuccess) return e;
+    gram_chol_kernel<<<(unsigned)((nmat + wpc - 1) / wpc), wpc * 32, smem, st>>>(Gre, Gim, Mc, P, ne_ld, nmat, thr,
+                                                                                      Pb, sig, fail);
+  }
+  cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return e;
-  gram_chol_kernel<<<(unsigned)((nmat + wpc - 1) / wpc), wpc * 32, smem, st>>>(Gre, Gim, Mc, P, ne_ld, nmat, thr,
-                                                                                    Pb, fail);
+  // certificate: one resident wave of CTAs (228 KB of shared memory per SM, 1 KB of it reserved per CTA)
+  e = allow_dynamic_smem(gram_certify_kernel, smem);
+  if (e != cudaSuccess) return e;
+  const long long chunks = (nmat + 31) / 32;
+  const long long resident = (long long)sm_count() * std::max<size_t>(1, (228 * 1024) / (smem + 1024));
+  const unsigned ncta = (unsigned)std::min((chunks + wpc - 1) / wpc, resident);
+  gram_certify_kernel<<<ncta, wpc * 32, smem, st>>>(Gre, Gim, Mc, P, ne_ld, nmat, sig, fail);
   return cudaGetLastError();
 }
 

@@ -120,10 +120,11 @@ cudaError_t launch_interleave(cudaStream_t st, const double* re, const double* i
 cudaError_t launch_build_F(cudaStream_t st, const double* Gh, int S, int N, const double* Y, int Mc,
                            int P, int ne_ld, double* Fs, double* Fa);
 cudaError_t launch_gram_beta(cudaStream_t st, const cplx* bn, int N, int K, double* bre, double* bim);
-// Cholesky + inverse + condition bound of nbins*P packed Hermitian matrices; fail[0] counts all
-// refused matrices, fail[1 + bin] those of one bin.
+// Inverse and condition certificate (cond_2 < thr) of nbins*P packed Hermitian matrices (Mc <= 64), two launches;
+// fail[0] counts refused matrices, fail[1 + bin] those of one bin (zero: the bin may take the Gram route);
+// sig: one double per matrix of scratch.
 cudaError_t launch_gram_chol(cudaStream_t st, const double* Gre, const double* Gim, int Mc, int P,
-                             int ne_ld, int nbins, double thr, cplx* Pb, int* fail);
+                             int ne_ld, int nbins, double thr, cplx* Pb, double* sig, int* fail);
 // forward of every bin: Cv rows (j*2+ear)*2+{re,im} = b_k .* (Y_o^T W_{k-1})
 // EXTENSION: diffuse-field covariance constraint (gram_kernels.cu)
 cudaError_t launch_target_cov(cudaStream_t st, const double* HdL, const double* HdR, int D, int K, double* out);
