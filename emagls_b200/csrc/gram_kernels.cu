@@ -395,7 +395,7 @@ cudaError_t launch_gram_chol(cudaStream_t st, const double* Gre, const double* G
   if (Mc > 64) return cudaErrorInvalidValue;
   const long long nmat = (long long)nbins * P;
   const size_t per_warp = chol_warp_elems(Mc) * sizeof(cplx);
-  // as many warps (matrices) per CTA as the 227 KB of shared memory hold (4 up to Mc = 58, 3 at Mc = 64)
+  // as many warps (matrices) per CTA as the 227 KB of shared memory hold (4 up to Mc = 59, 3 from Mc = 60)
   int wpc = GC_WPC;
   while (wpc > 1 && per_warp * wpc > 227 * 1024) --wpc;
   const size_t smem = per_warp * wpc;

@@ -20,8 +20,11 @@ FWD_NAMES = {0: "raw4", 1: "raw6", 2: "fix6", 3: "fix6_nt80_w20", 4: "launch_oz_
 def compile_harness(out_dir: str) -> str:
     from emagls_b200 import build as b
     so = os.path.join(out_dir, "ozaki_harness.so")
-    subprocess.run([b._nvcc(), *b.ARCH, "-O3", "-std=c++17", "-Xcompiler", "-fPIC", "-shared", "-o", so, SRC],
-                   check=True, capture_output=True, text=True)
+    # -Bsymbolic: the harness calls its own copies of the library's functions.  The library is loaded RTLD_GLOBAL, so
+    # without it, once the library is loaded in the same process, its definitions would take over some of the harness's
+    # calls: kernels compiled into the harness would then reach the library's CUDA runtime, which does not know them.
+    subprocess.run([b._nvcc(), *b.ARCH, "-O3", "-std=c++17", "-Xcompiler", "-fPIC", "-shared", "-Xlinker", "-Bsymbolic",
+                    "-o", so, SRC], check=True, capture_output=True, text=True)
     return so
 
 
