@@ -89,6 +89,10 @@ SIGNATURES = {
                                               C.c_int, C.POINTER(C.c_void_p)]),
     "emagls_render_stream_create_sh": (C.c_int, [C.c_void_p, c_dp, c_dp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                                  C.POINTER(C.c_void_p)]),
+    "emagls_render_stream_create_listeners": (C.c_int, [C.c_void_p, c_dp, c_dp, C.c_int, C.c_int, C.c_int, C.c_int,
+                                                        C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
+    "emagls_render_stream_create_sh_listeners": (C.c_int, [C.c_void_p, c_dp, c_dp, C.c_int, C.c_int, C.c_int, C.c_int,
+                                                           C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "emagls_render_stream_process": (C.c_int, [C.c_void_p, c_dp, C.c_longlong, C.c_void_p, c_dp, C.c_longlong, c_dp]),
     "emagls_render_stream_process_dev": (C.c_int, [C.c_void_p, c_dp, C.c_longlong, C.c_void_p, c_dp, C.c_longlong,
                                                    c_dp]),

@@ -506,10 +506,11 @@ def binauralDecodeShTracked(inp, wL, wR, rotations, hop, fade=None, compensateDe
 class _Session:
     """One render session (emagls_render_stream_*): owns the C session and frees it on close()."""
 
-    def __init__(self, h, ptr, num_ch):
+    def __init__(self, h, ptr, num_ch, listeners):
         self.handle = h
         self._s = ptr
         self.num_ch = num_ch
+        self.listeners = listeners
 
     @property
     def ptr(self):
@@ -539,10 +540,11 @@ class _Session:
         x = _f(x)
         if x.ndim != 2 or x.shape[1] != self.num_ch:
             raise ValueError(f"x must be [samples, {self.num_ch}]")
-        out = np.zeros((x.shape[0], 2), order="F")
+        L = self.listeners
+        out = np.zeros((x.shape[0], 2, L), order="F")
         h = self.handle
         h.check(h.lib.emagls_render_stream_process(self.ptr, _p(x), x.shape[0], _p(track), _p(rotations), nnew, _p(out)))
-        return out
+        return out if L > 1 else out[:, :, 0]
 
 
 class RenderStream(_Session):
@@ -550,9 +552,12 @@ class RenderStream(_Session):
     emagls_render_stream_create): ``wL``, ``wR`` [len, ch] (static) or [len, ch, pages] (bank).  ``process(x, track)``
     renders the next ``x`` [n, ch] (n a multiple of ``block``) and returns [n, 2]; ``track`` holds the next tracker
     entries (0-based pages of frames of ``hop`` samples, crossfaded over ``fade`` samples, default ``hop``).  The
-    concatenated outputs equal binauralDecode / binauralDecodeTracked of the concatenated input."""
+    concatenated outputs equal binauralDecode / binauralDecodeTracked of the concatenated input.  A bank session may
+    serve ``listeners`` > 1 listeners who hear the same input (emagls_render_stream_create_listeners): ``track`` is then
+    [k, listeners] and ``process`` returns [n, 2, listeners], listener l's output being that of a one-listener session
+    on ``track[:, l]``."""
 
-    def __init__(self, wL, wR, block, hop=None, fade=None, *, handle=None):
+    def __init__(self, wL, wR, block, hop=None, fade=None, *, listeners=1, handle=None):
         h = handle or default_handle()
         wl, wr = _f(wL), _f(wR)
         if wl.ndim == 2:
@@ -566,19 +571,26 @@ class RenderStream(_Session):
         hop = 1 if hop is None else int(hop)
         fade = (hop if pages > 1 else 0) if fade is None else int(fade)
         s = C.c_void_p()
-        h.check(h.lib.emagls_render_stream_create(h.ptr, _p(wl), _p(wr), ln, ch, pages, int(block), hop, fade,
-                                                  C.byref(s)))
-        super().__init__(h, s, ch)
+        h.check(h.lib.emagls_render_stream_create_listeners(h.ptr, _p(wl), _p(wr), ln, ch, pages, int(listeners),
+                                                            int(block), hop, fade, C.byref(s)))
+        super().__init__(h, s, ch, int(listeners))
         self.block, self.hop, self.fade, self.pages = int(block), hop, fade, pages
 
     def process(self, x, track=None):
         trk, n = None, 0
         if track is not None:
-            trk = np.ascontiguousarray(np.asarray(track).ravel())
+            trk = np.asarray(track)
+            if self.listeners > 1:
+                if trk.ndim != 2 or trk.shape[1] != self.listeners:
+                    raise ValueError(f"track must be [frames, {self.listeners}]")
+                n = trk.shape[0]
+                trk = trk.T                         # listener-major: track[l * frames + j]
+            trk = np.ascontiguousarray(trk.ravel())
             if not np.issubdtype(trk.dtype, np.integer) or (trk.size and (trk.min() < -2**31 or trk.max() >= 2**31)):
                 raise ValueError("track must hold integer page numbers")
             trk = trk.astype(np.int32)
-            n = trk.size
+            if self.listeners == 1:
+                n = trk.size
         return self._process(x, trk, None, n)
 
 
@@ -586,9 +598,11 @@ class ShRenderStream(_Session):
     """Render session of the SH head-tracked render (not in the reference API; emagls_render_stream_create_sh): one
     filter pair ``wL``, ``wR`` [len, (order+1)^2]; ``process(x, rotations)`` renders the next ``x`` [n, (order+1)^2]
     (n a multiple of ``block``) with the next head orientations ``rotations`` [k, 3, 3] (one per frame of ``hop``
-    samples) and returns [n, 2].  The concatenated outputs equal binauralDecodeShTracked of the concatenated input."""
+    samples) and returns [n, 2].  The concatenated outputs equal binauralDecodeShTracked of the concatenated input.
+    With ``listeners`` > 1 (emagls_render_stream_create_sh_listeners) every listener hears the same input with their
+    own head orientations: ``rotations`` is [k, listeners, 3, 3] and ``process`` returns [n, 2, listeners]."""
 
-    def __init__(self, wL, wR, block, hop, fade=None, *, handle=None):
+    def __init__(self, wL, wR, block, hop, fade=None, *, listeners=1, handle=None):
         h = handle or default_handle()
         wl, wr = _f(wL), _f(wR)
         if wl.shape != wr.shape or wl.ndim != 2:
@@ -600,18 +614,24 @@ class ShRenderStream(_Session):
         hop = int(hop)
         fade = hop if fade is None else int(fade)
         s = C.c_void_p()
-        h.check(h.lib.emagls_render_stream_create_sh(h.ptr, _p(wl), _p(wr), ln, order, int(block), hop, fade,
-                                                     C.byref(s)))
-        super().__init__(h, s, ch)
+        h.check(h.lib.emagls_render_stream_create_sh_listeners(h.ptr, _p(wl), _p(wr), ln, order, int(listeners),
+                                                               int(block), hop, fade, C.byref(s)))
+        super().__init__(h, s, ch, int(listeners))
         self.block, self.hop, self.fade, self.order = int(block), hop, fade, order
 
     def process(self, x, rotations=None):
         R, n = None, 0
         if rotations is not None:
-            R = np.ascontiguousarray(np.asarray(rotations, dtype=np.float64))
-            if R.ndim != 3 or R.shape[1:] != (3, 3):
+            R = np.asarray(rotations, dtype=np.float64)
+            L = self.listeners
+            if L > 1:
+                if R.ndim != 4 or R.shape[1:] != (L, 3, 3):
+                    raise ValueError(f"rotations must be [frames, {L}, 3, 3]")
+                R = R.transpose(1, 0, 2, 3)          # listener-major: matrix l * frames + j
+            elif R.ndim != 3 or R.shape[1:] != (3, 3):
                 raise ValueError("rotations must be [frames, 3, 3]")
-            n = R.shape[0]
+            n = R.shape[-3]
+            R = np.ascontiguousarray(R)
         return self._process(x, None, R, n)
 
 

@@ -38,21 +38,26 @@ void binaural_decode_rows(emagls_ctx* h, const double* in, long long num_samples
 __host__ __device__ constexpr int band_offset(int l) { return l * (4 * l * l - 1) / 3; }
 
 // Q[j][band_offset(l) + r (2l+1) + c] = getSHrotMtx(rot[f], order, 'real')[l^2 + r][l^2 + c] for frame f = f_base + j,
-// and same[j] = 1 when rot[f] is bitwise equal to rot[f - 1] (rot[k] holds frame rot_base + k)
-__global__ void frame_rotations_kernel(const double* __restrict__ rot, long long rot_base, long long f_base, int order,
-                                       double* __restrict__ Q, int* __restrict__ same);
+// and same[j] = 1 when rot[f] is bitwise equal to rot[f - 1] (rot[k] holds frame rot_base + k).  Listener y
+// (blockIdx.y; the whole-signal render launches one with zero strides) reads rot + y rot_ls and writes
+// Q + y nfr_ls band_offset(order + 1) and same + y nfr_ls.
+__global__ void frame_rotations_kernel(const double* __restrict__ rot, long long rot_ls, long long rot_base,
+                                       long long f_base, int order, double* __restrict__ Q, int* __restrict__ same,
+                                       long long nfr_ls);
 // out[ch][q] = (in[h0 + q, :] @ M)[ch] for q < m with the blended frame matrices of the contract; in has leading
 // dimension ld_in and in[0] sits at first_sample on the track's time axis; Q and same hold frames f_base ...
+// Listener y (blockIdx.y) rotates the shared input with its own Q and same (strides as above) into out + y out_ls.
 __global__ void sh_track_rotate_kernel(const double* __restrict__ in, long long ld_in, long long h0, long long m,
                                        int order, const double* __restrict__ Q, const int* __restrict__ same,
-                                       long long f_base, long long first_sample, int hop, int fade,
-                                       double* __restrict__ out);
-// the two kernels above for nfr frames / m samples on h->stream (launch counting and profiling are the caller's)
-void launch_frame_rotations(emagls_ctx* h, const double* rot, long long rot_base, long long f_base, long long nfr,
-                            int order, double* Q, int* same);
-void launch_sh_track_rotate(emagls_ctx* h, const double* in, long long ld_in, long long h0, long long m, int order,
-                            const double* Q, const int* same, long long f_base, long long first_sample, int hop,
-                            int fade, double* out);
+                                       long long nfr_ls, long long f_base, long long first_sample, int hop, int fade,
+                                       double* __restrict__ out, long long out_ls);
+// the two kernels above for nl listeners x nfr frames / m samples on h->stream (launch counting and profiling are the
+// caller's)
+void launch_frame_rotations(emagls_ctx* h, int nl, const double* rot, long long rot_ls, long long rot_base,
+                            long long f_base, long long nfr, int order, double* Q, int* same, long long nfr_ls);
+void launch_sh_track_rotate(emagls_ctx* h, int nl, const double* in, long long ld_in, long long h0, long long m,
+                            int order, const double* Q, const int* same, long long nfr_ls, long long f_base,
+                            long long first_sample, int hop, int fade, double* out, long long out_ls);
 
 // Forward transforms of the overlap-save blocks of a multichannel signal into X[ch][nbc][F].  Block b takes the N
 // input samples starting at b*L - ov.  Direct route (default when every channel of the signal is 16-byte aligned):

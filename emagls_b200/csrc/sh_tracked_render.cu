@@ -21,14 +21,18 @@ constexpr int SHT_S = 4;           // samples per thread (strided by 32: every l
 // Q[j][band_offset(l) + r (2l+1) + c] = getSHrotMtx(rot[f], order, 'real')[l^2 + r][l^2 + c] for frame f = f_base + j
 // (blockIdx.x), and same[j] = 1 when rot[f] is bitwise equal to rot[f - 1].  rot[k] holds frame rot_base + k.
 // One CTA per frame: the band recursion of shrot.cuh builds the full matrix in shared memory, of which only the
-// diagonal blocks are stored.
-__global__ void frame_rotations_kernel(const double* __restrict__ rot, long long rot_base, long long f_base, int order,
-                                       double* __restrict__ Q, int* __restrict__ same) {
+// diagonal blocks are stored.  Listener blockIdx.y reads rot + y rot_ls and writes Q + y nfr_ls blk, same + y nfr_ls.
+__global__ void frame_rotations_kernel(const double* __restrict__ rot, long long rot_ls, long long rot_base,
+                                       long long f_base, int order, double* __restrict__ Q, int* __restrict__ same,
+                                       long long nfr_ls) {
   extern __shared__ double fr_Rr[];
   __shared__ Rot1 R1;
   __shared__ int rotate;
   const int nsh = (order + 1) * (order + 1), blk = band_offset(order + 1);
   const long long j = blockIdx.x, f = f_base + j;
+  rot += blockIdx.y * rot_ls;
+  Q += blockIdx.y * nfr_ls * blk;
+  same += blockIdx.y * nfr_ls;
   const double* E = rot + (f - rot_base) * 9;
   if (threadIdx.x == 0) {
     double M[3][3];
@@ -109,11 +113,15 @@ __device__ __forceinline__ void rotate_samples(const double* __restrict__ in, lo
 // i >= fade.  Q and same hold frames f_base ... (frame_rotations_kernel).  Each warp covers 32 S consecutive samples,
 // lane + 32 s for thread s; a thread whose samples share a frame applies each loaded matrix entry to all of them, the
 // others (a frame boundary inside the warp's span, or hops shorter than that span) take them one at a time.
+// Listener blockIdx.y rotates the same input with Q + y nfr_ls blk, same + y nfr_ls into out + y out_ls.
 __global__ void __launch_bounds__(SHT_T, 1)
 sh_track_rotate_kernel(const double* __restrict__ in, long long ld_in, long long h0, long long m, int order,
-                       const double* __restrict__ Q, const int* __restrict__ same, long long f_base,
-                       long long first_sample, int hop, int fade, double* __restrict__ out) {
+                       const double* __restrict__ Q, const int* __restrict__ same, long long nfr_ls, long long f_base,
+                       long long first_sample, int hop, int fade, double* __restrict__ out, long long out_ls) {
   const int blk = band_offset(order + 1);
+  Q += blockIdx.y * nfr_ls * blk;
+  same += blockIdx.y * nfr_ls;
+  out += blockIdx.y * out_ls;
   const long long warp = ((long long)blockIdx.x * SHT_T + threadIdx.x) / 32;
   const int lane = threadIdx.x & 31;
   long long src[SHT_S], dst[SHT_S], fr[SHT_S];
@@ -154,20 +162,20 @@ sh_track_rotate_kernel(const double* __restrict__ in, long long ld_in, long long
   }
 }
 
-void launch_frame_rotations(emagls_ctx* h, const double* rot, long long rot_base, long long f_base, long long nfr,
-                            int order, double* Q, int* same) {
+void launch_frame_rotations(emagls_ctx* h, int nl, const double* rot, long long rot_ls, long long rot_base,
+                            long long f_base, long long nfr, int order, double* Q, int* same, long long nfr_ls) {
   const int C = (order + 1) * (order + 1);
-  frame_rotations_kernel<<<(unsigned)nfr, 128, (size_t)C * C * sizeof(double), h->stream>>>(rot, rot_base, f_base,
-                                                                                           order, Q, same);
+  frame_rotations_kernel<<<dim3((unsigned)nfr, (unsigned)nl), 128, (size_t)C * C * sizeof(double), h->stream>>>(
+      rot, rot_ls, rot_base, f_base, order, Q, same, nfr_ls);
   EM_CUDA(cudaGetLastError());
 }
 
-void launch_sh_track_rotate(emagls_ctx* h, const double* in, long long ld_in, long long h0, long long m, int order,
-                            const double* Q, const int* same, long long f_base, long long first_sample, int hop,
-                            int fade, double* out) {
+void launch_sh_track_rotate(emagls_ctx* h, int nl, const double* in, long long ld_in, long long h0, long long m,
+                            int order, const double* Q, const int* same, long long nfr_ls, long long f_base,
+                            long long first_sample, int hop, int fade, double* out, long long out_ls) {
   const long long warps = (m + 32 * SHT_S - 1) / (32 * SHT_S);
-  sh_track_rotate_kernel<<<(unsigned)((warps * 32 + SHT_T - 1) / SHT_T), SHT_T, 0, h->stream>>>(
-      in, ld_in, h0, m, order, Q, same, f_base, first_sample, hop, fade, out);
+  sh_track_rotate_kernel<<<dim3((unsigned)((warps * 32 + SHT_T - 1) / SHT_T), (unsigned)nl), SHT_T, 0, h->stream>>>(
+      in, ld_in, h0, m, order, Q, same, nfr_ls, f_base, first_sample, hop, fade, out, out_ls);
   EM_CUDA(cudaGetLastError());
 }
 
@@ -238,12 +246,12 @@ void binaural_decode_sh_tracked_dev(emagls_ctx* h, const double* in, long long n
     const long long m = k.c_hi - k.h0;
     {
       ProfSpan ps(h, EM_PROF_RENDER_STAGE);
-      frame_rotations_kernel<<<(unsigned)k.nfr, 128, (size_t)C * C * sizeof(double), st>>>(rot, rot_base, k.f_base,
-                                                                                          order, Q, same);
+      frame_rotations_kernel<<<(unsigned)k.nfr, 128, (size_t)C * C * sizeof(double), st>>>(rot, 0, rot_base,
+                                                                                          k.f_base, order, Q, same, 0);
       EM_CUDA(cudaGetLastError());
       const long long warps = (m + 32 * SHT_S - 1) / (32 * SHT_S);
       sh_track_rotate_kernel<<<(unsigned)((warps * 32 + SHT_T - 1) / SHT_T), SHT_T, 0, st>>>(
-          in, num_samples, k.h0, m, order, Q, same, k.f_base, first_sample, hop, fade, ws);
+          in, num_samples, k.h0, m, order, Q, same, 0, k.f_base, first_sample, hop, fade, ws, 0);
       EM_CUDA(cudaGetLastError());
     }
     h->launches += 2;

@@ -1,13 +1,16 @@
 // Render sessions (contract in include/emagls_cuda.h, DESIGN.md "Render sessions"): the static, bank and SH
-// head-tracked renders streamed block by block.  Uniformly partitioned overlap-save with a frequency-domain delay line
-// (FDL): FFT size N = 2 B for blocks of B samples, P = ceil(len / B) partitions of B taps.  The spectra of every page and
-// partition, H[page][ear][ch][q][F], are built once at creation; every block transforms [previous block | block] of all
-// channels into FDL slot k mod P, and per distinct page it needs (a "pair" as in tracked_render.cu)
+// head-tracked renders streamed block by block, for L listeners (seats) who hear one shared input stream with their own
+// tracker entries.  Uniformly partitioned overlap-save with a frequency-domain delay line (FDL): FFT size N = 2 B for
+// blocks of B samples, P = ceil(len / B) partitions of B taps.  The spectra of every page and partition,
+// H[page][ear][ch][q][F], are built once at creation; every block transforms [previous block | block] of all channels
+// into FDL slot k mod P, and per distinct page it needs (a "pair" as in tracked_render.cu)
 //     Y[pair][ear][f] = sum_q sum_ch X[slot(k - q)][ch][f] H[page][ear][ch][q][f],
-// whose inverse transforms (second half, 1/N) are mixed with the crossfade weights of the tracked render.  SH sessions
-// rotate the block first (the rotation stage of sh_tracked_render.cu) and render the rotated block with one page.
-// Everything a block needs is allocated at creation: the per-call path allocates nothing, builds no plan and reads no
-// device property; its host work is O(frames + pages in the call).
+// whose inverse transforms (second half, 1/N) are mixed per listener with the crossfade weights of the tracked render.
+// A bank session's listeners share the stage, the FDL and the pairs: a block renders the union of the pages its
+// listeners need, once.  SH sessions rotate the block per listener first (the rotation stage of sh_tracked_render.cu),
+// keep an FDL per listener and render each rotated block with the one page.  Either way a block takes the same number
+// of launches whatever L.  Everything a block needs is allocated at creation: the per-call path allocates nothing,
+// builds no plan and reads no device property; its host work is O(L frames + pages in the call).
 #include <algorithm>
 #include <array>
 #include <cstdint>
@@ -23,13 +26,18 @@ struct emagls_stream_ctx {
   emagls_ctx* h = nullptr;
   int kind = EM_STREAM_STATIC;
   int num_ch = 0, len = 0, num_pages = 1, order = 0, B = 0, hop = 1, fade = 0;
+  int nl = 1;                 // listeners (seats); they share the input stream
+  int xch = 0;                // channels of the FDL: num_ch (static, bank) or nl num_ch (SH: one FDL per listener)
   int N = 0, F = 0, P = 0;
   int cb = 1;                 // blocks per chunk: capacity of the staging buffers and of one table upload
-  int pmax = 1, pcap = 1;     // distinct pages one block can need; pmax rounded up to a power of two
+  int pmax = 1;               // distinct pages one listener's block can need
+  int pcap = 1;               // pairs Y and yseg hold: pow2(min(num_pages, nl pmax)) (bank), nl (SH), 1 (static)
+  long long fr_blk = 0;       // frames one block's samples fall in
   long long nfr_blk = 0;      // frames one block's rotation stage covers (previous frame included)
-  long long nfr_chunk = 0;    // tracker entries one chunk's table holds
+  long long nfr_chunk = 0;    // tracker entries per listener one chunk's table holds
   long long T = 0;            // samples processed
-  // tracker entries from frame trk_base / rot_base on (the previous frame and the look-ahead)
+  // tracker entries from frame trk_base / rot_base on (the previous frame and the look-ahead), nl per frame:
+  // trk[(f - trk_base) nl + l] is listener l's page of frame f
   std::deque<int32_t> trk;
   long long trk_base = 0;
   std::deque<std::array<double, 9>> rot;
@@ -37,18 +45,18 @@ struct emagls_stream_ctx {
   // device memory (from the handle's pool)
   std::vector<void*> dev;
   emagls::cplx* H = nullptr;  // [pages][2][ch][P][F]
-  emagls::cplx* X = nullptr;  // FDL ring [P][ch][F]
-  double* seg = nullptr;      // [ch][N]: previous block | this block
-  double* prev = nullptr;     // [ch][B]
+  emagls::cplx* X = nullptr;  // FDL ring [P][xch][F]
+  double* seg = nullptr;      // [xch][N]: previous block | this block
+  double* prev = nullptr;     // [xch][B]
   emagls::cplx* Y = nullptr;  // [pcap][2][F]
   double* yseg = nullptr;     // [pcap][2][N]
-  int* d_tab = nullptr;       // block offsets, pages, track frames of one chunk
+  int* d_tab = nullptr;       // bank: the combine's pair slots and the union pages of one chunk
   int* d_zero = nullptr;      // page 0 (static and SH sessions)
-  double* d_rot = nullptr;    // rotation matrices of one chunk (SH)
-  double* Q = nullptr;        // frame rotations of one block (SH)
-  int* same = nullptr;
-  double* rbuf = nullptr;     // rotated block [ch][B] (SH)
-  double* d_in = nullptr;     // host variant: one chunk of input [ch][cb B] and output [2][cb B]
+  double* d_rot = nullptr;    // rotation matrices of one chunk [nl][frames][9] (SH)
+  double* Q = nullptr;        // frame rotations of one block [nl][nfr_blk][band_offset(order + 1)] (SH)
+  int* same = nullptr;        // [nl][nfr_blk]
+  double* rbuf = nullptr;     // rotated block [nl][ch][B] (SH)
+  double* d_in = nullptr;     // host variant: one chunk of input [ch][cb B] and output [nl][2][cb B]
   double* d_out = nullptr;
   // pinned host staging
   double* h_in = nullptr;
@@ -59,14 +67,15 @@ struct emagls_stream_ctx {
   cudaEvent_t tab_ev = nullptr;  // the last table upload: the pinned table is rewritten only after it has run
   cufftHandle fwd = 0;
   std::vector<cufftHandle> inv;  // inv[j]: 2 * 2^j inverse transforms; all per-block plans share one work area
-  // host scratch of a chunk (sized at creation): block offsets into the page list, a block's candidate pages
-  std::vector<int> blk_off, cand;
+  // host scratch of a chunk (sized at creation): block offsets into the union pages and the slot table, a block's
+  // union, and the union slot of every page (-1: not in the block's union)
+  std::vector<int> blk_off, cmb_off, uni, mark;
 };
 
 namespace emagls {
 namespace {
 
-constexpr int ST_MIN_BLOCK = 16, ST_MAX_BLOCK = 8192, ST_MAX_ORDER = 7;
+constexpr int ST_MIN_BLOCK = 16, ST_MAX_BLOCK = 8192, ST_MAX_ORDER = 7, ST_MAX_LISTENERS = 4096;
 constexpr long long ST_CHUNK_SAMPLES = 16384;   // samples per chunk of the staging buffers
 
 // wp[u][ear][ch][q][N] = taps [q B, (q + 1) B) of page u0 + u, zero-padded to N (pages past nu: zeros)
@@ -87,14 +96,14 @@ __global__ void stream_pad_partitions_kernel(const double* __restrict__ wL, cons
   wp[idx] = (u < nu && t < B && tap < len) ? w[((u0 + u) * num_ch + ch) * len + tap] : 0.0;
 }
 
-// seg[ch] = prev[ch] | in[ch][0 .. B), prev[ch] = in[ch][0 .. B)
+// seg[ch] = prev[ch] | in[ch][0 .. B), prev[ch] = in[ch][0 .. B).  num_ch B reaches 2^31 with many SH listeners.
 __global__ void stream_stage_kernel(const double* __restrict__ in, long long ld_in, int num_ch, int B,
                                     double* __restrict__ prev, double* __restrict__ seg) {
-  const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= num_ch * B) return;
-  const int ch = idx / B, i = idx - ch * B;
-  const double x = in[(long long)ch * ld_in + i];
-  double* s = seg + (long long)ch * 2 * B;
+  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= (long long)num_ch * B) return;
+  const long long ch = idx / B, i = idx - ch * B;
+  const double x = in[ch * ld_in + i];
+  double* s = seg + ch * 2 * B;
   s[i] = prev[idx];
   s[B + i] = x;
   prev[idx] = x;
@@ -103,13 +112,15 @@ __global__ void stream_stage_kernel(const double* __restrict__ in, long long ld_
 // Y[p][ear][f] = sum_q sum_ch X[(slot - q) mod P][ch][f] * H[pages[p]][ear][ch][q][f] for the np pages of one block.
 // One thread per (f, group of G pages, blockIdx.y) keeps the G pairs' accumulators in registers, so every FDL value is
 // read once per page group; the channel loop is unrolled by two, so 2 (2 G + 1) independent 16-byte loads are in
-// flight per thread.  Slots and the page count are uniform over the grid, so no predicate diverges.
+// flight per thread.  Slots and the page count are uniform over the grid, so no predicate diverges.  blockIdx.z
+// selects a listener's FDL (SH sessions): X + z num_ch F within each slot of xs values, and Y + z np 2 F.
 template <int G>
 __global__ void __launch_bounds__(128)
-stream_mac_kernel(const cplx* __restrict__ X, const cplx* __restrict__ H, const int* __restrict__ pages, int np,
-                  int num_ch, int P, int F, int slot, cplx* __restrict__ Y) {
+stream_mac_kernel(const cplx* __restrict__ X, long long xs, const cplx* __restrict__ H, const int* __restrict__ pages,
+                  int np, int num_ch, int P, int F, int slot, cplx* __restrict__ Y) {
   const int f = blockIdx.x * blockDim.x + threadIdx.x;
   if (f >= F) return;
+  const long long xz = (long long)blockIdx.z * num_ch * F;   // this listener's FDL within a slot
   const int g0 = blockIdx.y * G, n = min(G, np - g0);
   const long long cs = (long long)P * F;          // channel stride of H
   const long long es = (long long)num_ch * cs;    // ear stride of H
@@ -122,7 +133,7 @@ stream_mac_kernel(const cplx* __restrict__ X, const cplx* __restrict__ H, const 
   }
   for (int d = 0; d < P; ++d) {
     const int sl = slot - d < 0 ? slot - d + P : slot - d;
-    const cplx* x = X + (long long)sl * num_ch * F + f;
+    const cplx* x = X + xz + sl * xs + f;
     const long long ho = (long long)d * F;
     int ch = 0;
     for (; ch + 2 <= num_ch; ch += 2) {
@@ -156,42 +167,56 @@ stream_mac_kernel(const cplx* __restrict__ X, const cplx* __restrict__ H, const 
 #pragma unroll
   for (int q = 0; q < G; ++q)
     if (q < n) {
-      const long long o = (long long)(g0 + q) * 2 * F + f;
+      const long long o = ((long long)blockIdx.z * np + g0 + q) * 2 * F + f;
       Y[o] = yl[q];
       Y[o + F] = yr[q];
     }
 }
 
-// out[ear * ld_out + i] = sum_p weight(pages[p]) * yseg[p][ear][B + i] / N for sample t = t0 + i of one block, with the
-// weights of tracked_combine_kernel: weight(page) = (page == c ? g : 0) + (page == a ? 1 - g : 0), g = 1 when a == c.
-// trk holds track[f_base ..]; without a track every sample takes page pages[0] with weight 1.
-__global__ void stream_combine_kernel(const double* __restrict__ yseg, const int* __restrict__ pages, int np,
-                                      const int* __restrict__ trk, long long f_base, long long t0, int B, int hop,
-                                      int fade, long long ld_out, double* __restrict__ out) {
+// out[(2 l + ear) ld_out + i] = sum over pages of weight(page) yseg[slot(page)][ear][B + i] / N for sample t = t0 + i of
+// one block and listener l = blockIdx.y, with the weights of tracked_combine_kernel: c = track[f], a = track[max(f-1, 0)],
+// weight(page) = (page == c ? g : 0) + (page == a ? 1 - g : 0), g = 1 when a == c.  slots[(l nfb + f - fb0) 2 + {0, 1}]
+// are the union slots of a and c (the union is in ascending page order, so the two pages are added in that order, as
+// the one-listener sum over the block's sorted pages; -1 marks an a outside the union, whose weight is 0 then).
+// Without slots (static and SH sessions) listener l takes pair l with weight 1.
+__global__ void stream_combine_kernel(const double* __restrict__ yseg, const int* __restrict__ slots, long long fb0,
+                                      int nfb, long long t0, int B, int hop, int fade, long long ld_out,
+                                      double* __restrict__ out) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= B) return;
-  const int N = 2 * B;
-  int c = pages[0], a = c;
+  const int l = blockIdx.y, N = 2 * B;
+  int sa = l, sc = l;
   double g = 1.0;
-  if (trk) {
+  if (slots) {
     const long long t = t0 + i, f = t / hop;
     const int ii = (int)(t - f * hop);
-    c = trk[f - f_base];
-    a = trk[(f > 0 ? f - 1 : 0) - f_base];
-    g = (a != c && ii < fade) ? ((double)ii + 0.5) / (double)fade : 1.0;
+    const int* e = slots + ((long long)l * nfb + (f - fb0)) * 2;
+    sa = e[0];
+    sc = e[1];
+    g = (sa != sc && ii < fade) ? ((double)ii + 0.5) / (double)fade : 1.0;
+  }
+  // (page, weight) in ascending page order; a == c takes g + (1 - g) = 1
+  int p0 = sc, p1 = -1;
+  double w0 = 1.0, w1 = 0.0;
+  if (sa != sc) {
+    if (sa < sc) { p0 = sa; w0 = 1.0 - g; p1 = sc; w1 = g; }
+    else         { p0 = sc; w0 = g;       p1 = sa; w1 = 1.0 - g; }
   }
   double yl = 0.0, yr = 0.0;
-  for (int p = 0; p < np; ++p) {
-    const int pg = pages[p];
-    const double w = (pg == c ? g : 0.0) + (pg == a ? 1.0 - g : 0.0);
-    if (w == 0.0) continue;
-    const double* y = yseg + (long long)p * 2 * N + B + i;
-    yl = fma(w, y[0], yl);
-    yr = fma(w, y[N], yr);
+  if (w0 != 0.0) {
+    const double* y = yseg + (long long)p0 * 2 * N + B + i;
+    yl = fma(w0, y[0], yl);
+    yr = fma(w0, y[N], yr);
+  }
+  if (w1 != 0.0) {
+    const double* y = yseg + (long long)p1 * 2 * N + B + i;
+    yl = fma(w1, y[0], yl);
+    yr = fma(w1, y[N], yr);
   }
   const double inv_n = 1.0 / (double)N;
-  out[i] = yl * inv_n;
-  out[ld_out + i] = yr * inv_n;
+  double* o = out + 2 * l * ld_out + i;
+  o[0] = yl * inv_n;
+  o[ld_out] = yr * inv_n;
 }
 
 int pow2_at_least(long long v) {
@@ -242,59 +267,72 @@ struct SessionDeleter {
 
 // Geometry, buffers, plans and the filter spectra of a new session (the caller has checked the arguments)
 emagls_stream_ctx* create_session(emagls_ctx* h, int kind, const double* wL, const double* wR, int len, int num_ch,
-                                  int num_pages, int order, int block, int hop, int fade) {
+                                  int num_pages, int order, int nl, int block, int hop, int fade) {
   std::unique_ptr<emagls_stream_ctx, SessionDeleter> s(new emagls_stream_ctx());
   s->h = h;
   s->kind = kind;
-  s->num_ch = num_ch; s->len = len; s->num_pages = num_pages; s->order = order;
+  s->num_ch = num_ch; s->len = len; s->num_pages = num_pages; s->order = order; s->nl = nl;
   s->B = block; s->hop = hop; s->fade = fade;
   const int B = block, N = 2 * block, F = block + 1, P = (len + block - 1) / block;
   s->N = N; s->F = F; s->P = P;
-  s->cb = (int)std::max<long long>(1, ST_CHUNK_SAMPLES / B);
+  // the staging buffers hold about ST_CHUNK_SAMPLES samples of every listener's output
+  s->cb = (int)std::max<long long>(1, ST_CHUNK_SAMPLES / ((long long)B * nl));
   // a block intersects at most (B - 1) / hop + 2 frames and may need the frame before its first one
   const long long fr_blk = (B - 1) / hop + 2;
+  s->fr_blk = fr_blk;
   s->pmax = kind == EM_STREAM_BANK ? (int)std::min<long long>(num_pages, fr_blk + 1) : 1;
-  s->pcap = pow2_at_least(s->pmax);
+  s->pcap = kind == EM_STREAM_BANK ? pow2_at_least(std::min<long long>(num_pages, (long long)nl * s->pmax))
+                                   : kind == EM_STREAM_SH ? nl : 1;
+  s->xch = kind == EM_STREAM_SH ? nl * num_ch : num_ch;
   s->nfr_blk = fr_blk + 1;
   s->nfr_chunk = ((long long)s->cb * B - 1) / hop + 3;
+  const long long xch = s->xch;
   cudaStream_t st = h->stream;
 
   s->H = pool_get<cplx>(s.get(), (size_t)num_pages * 2 * num_ch * P * F);
-  s->X = pool_get<cplx>(s.get(), (size_t)P * num_ch * F);
-  s->seg = pool_get<double>(s.get(), (size_t)num_ch * N);
-  s->prev = pool_get<double>(s.get(), (size_t)num_ch * B);
+  s->X = pool_get<cplx>(s.get(), (size_t)P * xch * F);
+  s->seg = pool_get<double>(s.get(), (size_t)xch * N);
+  s->prev = pool_get<double>(s.get(), (size_t)xch * B);
   s->Y = pool_get<cplx>(s.get(), (size_t)s->pcap * 2 * F);
   s->yseg = pool_get<double>(s.get(), (size_t)s->pcap * 2 * N);
   s->d_zero = pool_get<int>(s.get(), 1);
   s->d_in = pool_get<double>(s.get(), (size_t)num_ch * s->cb * B);
-  s->d_out = pool_get<double>(s.get(), (size_t)2 * s->cb * B);
-  s->tab_cap = kind == EM_STREAM_BANK ? (size_t)(s->cb + 1) + (size_t)s->cb * s->pmax + (size_t)s->nfr_chunk : 1;
+  s->d_out = pool_get<double>(s.get(), (size_t)2 * nl * s->cb * B);
+  // bank table of one chunk: per block, 2 pair slots per listener and frame, and the union of pages
+  s->tab_cap = kind == EM_STREAM_BANK
+                   ? (size_t)s->cb * ((size_t)2 * nl * fr_blk + (size_t)std::min<long long>(num_pages, (long long)nl * s->pmax))
+                   : 1;
   s->d_tab = pool_get<int>(s.get(), s->tab_cap);
   if (kind == EM_STREAM_SH) {
     const int blk = band_offset(order + 1);
-    s->d_rot = pool_get<double>(s.get(), (size_t)s->nfr_chunk * 9);
-    s->Q = pool_get<double>(s.get(), (size_t)s->nfr_blk * blk);
-    s->same = pool_get<int>(s.get(), (size_t)s->nfr_blk);
-    s->rbuf = pool_get<double>(s.get(), (size_t)num_ch * B);
-    s->h_rot = pinned_get<double>((size_t)s->nfr_chunk * 9);
+    s->d_rot = pool_get<double>(s.get(), (size_t)nl * s->nfr_chunk * 9);
+    s->Q = pool_get<double>(s.get(), (size_t)nl * s->nfr_blk * blk);
+    s->same = pool_get<int>(s.get(), (size_t)nl * s->nfr_blk);
+    s->rbuf = pool_get<double>(s.get(), (size_t)xch * B);
+    s->h_rot = pinned_get<double>((size_t)nl * s->nfr_chunk * 9);
   }
   s->h_in = pinned_get<double>((size_t)num_ch * s->cb * B);
-  s->h_out = pinned_get<double>((size_t)2 * s->cb * B);
+  s->h_out = pinned_get<double>((size_t)2 * nl * s->cb * B);
   s->h_tab = pinned_get<int>(s->tab_cap);
   EM_CUDA(cudaEventCreateWithFlags(&s->tab_ev, cudaEventDisableTiming));
-  EM_CUDA(cudaMemsetAsync(s->X, 0, (size_t)P * num_ch * F * sizeof(cplx), st));
-  EM_CUDA(cudaMemsetAsync(s->seg, 0, (size_t)num_ch * N * sizeof(double), st));
-  EM_CUDA(cudaMemsetAsync(s->prev, 0, (size_t)num_ch * B * sizeof(double), st));
+  EM_CUDA(cudaMemsetAsync(s->X, 0, (size_t)P * xch * F * sizeof(cplx), st));
+  EM_CUDA(cudaMemsetAsync(s->seg, 0, (size_t)xch * N * sizeof(double), st));
+  EM_CUDA(cudaMemsetAsync(s->prev, 0, (size_t)xch * B * sizeof(double), st));
   EM_CUDA(cudaMemsetAsync(s->Y, 0, (size_t)s->pcap * 2 * F * sizeof(cplx), st));
   EM_CUDA(cudaMemsetAsync(s->d_zero, 0, sizeof(int), st));
 
   s->blk_off.resize((size_t)s->cb + 1);
-  s->cand.reserve((size_t)2 * fr_blk + 2);
+  s->cmb_off.resize((size_t)s->cb + 1);
+  if (kind == EM_STREAM_BANK) {
+    s->uni.reserve((size_t)std::min<long long>(num_pages, (long long)nl * s->pmax));
+    s->mark.assign((size_t)num_pages, -1);
+  }
 
-  // plans of the per-block path: the forward transform of all channels, and inverse transforms of 2 pairs, 4 pairs, ...
-  // up to pcap pairs (a block with np pages runs the smallest that holds them; the transforms of the pairs past np
-  // read stale spectra and are never combined).  They run one after the other on the handle's stream, so they share
-  // one work area, the largest any of them needs, from the handle's pool.
+  // plans of the per-block path: the forward transform of all FDL channels, and inverse transforms of the pairs.  A
+  // bank session has plans of 2 pairs, 4 pairs, ... up to pcap pairs (a block with np pages runs the smallest that
+  // holds them; the transforms of the pairs past np read stale spectra and are never combined); the others one plan
+  // of exactly pcap pairs.  They run one after the other on the handle's stream, so they share one work area, the
+  // largest any of them needs, from the handle's pool.
   int n[1] = {N};
   size_t ws_max = 0;
   auto make_plan = [&](cufftType type, int idist, int odist, int batch) {
@@ -311,8 +349,12 @@ emagls_stream_ctx* create_session(emagls_ctx* h, int kind, const double* wL, con
     ws_max = std::max(ws_max, ws);
     return p;
   };
-  s->fwd = make_plan(CUFFT_D2Z, N, F, num_ch);
-  for (int b = 1; b <= s->pcap; b <<= 1) s->inv.push_back(make_plan(CUFFT_Z2D, F, N, 2 * b));
+  s->fwd = make_plan(CUFFT_D2Z, N, F, xch);
+  if (kind == EM_STREAM_BANK) {
+    for (int b = 1; b <= s->pcap; b <<= 1) s->inv.push_back(make_plan(CUFFT_Z2D, F, N, 2 * b));
+  } else {
+    s->inv.push_back(make_plan(CUFFT_Z2D, F, N, 2 * s->pcap));
+  }
   {
     void* ws = pool_get<char>(s.get(), ws_max);
     EM_FFT(cufftSetWorkArea(s->fwd, ws));
@@ -376,84 +418,119 @@ void check_process(const emagls_stream_ctx* s, const double* in, long long num_s
   if (s->kind == EM_STREAM_BANK) {
     EM_REQUIRE(!rotations, "a bank session takes a track of pages, not rotations");
     EM_REQUIRE(track || num_new == 0, "null track");
-    for (long long j = 0; j < num_new; ++j)
+    for (long long j = 0; j < num_new * s->nl; ++j)
       EM_REQUIRE(track[j] >= 0 && track[j] < s->num_pages, "track entry outside [0, num_pages)");
-    EM_REQUIRE(s->trk_base + (long long)s->trk.size() + num_new > f_need, "track does not cover the call");
+    EM_REQUIRE(s->trk_base + (long long)s->trk.size() / s->nl + num_new > f_need, "track does not cover the call");
   } else {
     EM_REQUIRE(!track, "an SH session takes rotations, not a track of pages");
     EM_REQUIRE(rotations || num_new == 0, "null rotations");
-    EM_REQUIRE(s->rot_base + (long long)s->rot.size() + num_new > f_need, "rotations do not cover the call");
+    EM_REQUIRE(s->rot_base + (long long)s->rot.size() / s->nl + num_new > f_need, "rotations do not cover the call");
   }
 }
 
+// Entries arrive per listener ([num_new x nl], column-major) and are kept per frame (nl consecutive entries)
 void append_entries(emagls_stream_ctx* s, const int32_t* track, const double* rotations, long long num_new) {
-  if (s->kind == EM_STREAM_BANK) {
-    s->trk.insert(s->trk.end(), track, track + num_new);
-  } else if (s->kind == EM_STREAM_SH) {
-    for (long long j = 0; j < num_new; ++j) {
-      std::array<double, 9> r;
-      std::memcpy(r.data(), rotations + 9 * j, sizeof(r));
-      s->rot.push_back(r);
+  const int L = s->nl;
+  for (long long j = 0; j < num_new; ++j)
+    for (int l = 0; l < L; ++l) {
+      if (s->kind == EM_STREAM_BANK) {
+        s->trk.push_back(track[(long long)l * num_new + j]);
+      } else if (s->kind == EM_STREAM_SH) {
+        std::array<double, 9> r;
+        std::memcpy(r.data(), rotations + 9 * ((long long)l * num_new + j), sizeof(r));
+        s->rot.push_back(r);
+      }
     }
-  }
 }
 
 // Drop the entries no later block needs: blocks from sample T on use frame T / hop - 1 at the earliest
 void trim_entries(emagls_stream_ctx* s) {
   const long long keep = std::max<long long>(s->T / s->hop - 1, 0);
-  while (s->trk_base < keep && !s->trk.empty()) { s->trk.pop_front(); ++s->trk_base; }
-  while (s->rot_base < keep && !s->rot.empty()) { s->rot.pop_front(); ++s->rot_base; }
+  const size_t L = (size_t)s->nl;
+  while (s->trk_base < keep && !s->trk.empty()) { s->trk.erase(s->trk.begin(), s->trk.begin() + L); ++s->trk_base; }
+  while (s->rot_base < keep && !s->rot.empty()) { s->rot.erase(s->rot.begin(), s->rot.begin() + L); ++s->rot_base; }
 }
 
-// Blocks [T, T + nb B) of the stream: in[ch * ld_in + i] (i < nb B) -> out[ear * ld_out + i]
+// Blocks [T, T + nb B) of the stream: in[ch * ld_in + i] (i < nb B) -> out[(2 l + ear) * ld_out + i]
 void run_chunk(emagls_stream_ctx* s, const double* in, long long ld_in, int nb, double* out, long long ld_out) {
   emagls_ctx* h = s->h;
   cudaStream_t st = h->stream;
-  const int B = s->B, F = s->F, P = s->P, num_ch = s->num_ch;
+  const int B = s->B, F = s->F, P = s->P, num_ch = s->num_ch, L = s->nl, hop = s->hop;
   const long long t_first = s->T, t_last = s->T + (long long)nb * B - 1;
-  const long long f_first = std::max<long long>(t_first / s->hop - 1, 0), f_last = t_last / s->hop;
+  const long long f_first = std::max<long long>(t_first / hop - 1, 0), f_last = t_last / hop;
+  const long long nfr_c = f_last - f_first + 1;
 
-  // per block: its distinct pages (sorted: the combine sums them in a fixed order whatever the call split), by the
-  // rule of build_pairs in tracked_render.cu; one upload of the chunk's table
+  // bank: per block, the union of the pages its listeners need, by the rule of build_pairs in tracked_render.cu, in
+  // ascending page order (so the combine adds a listener's pages in the order of a one-listener session, whatever the
+  // other listeners or the call split), and per listener and frame of the block the union slots of pages a and c;
+  // one upload of the chunk's table
   std::vector<int>& blk_off = s->blk_off;
+  std::vector<int>& cmb_off = s->cmb_off;
   std::fill(blk_off.begin(), blk_off.begin() + nb + 1, 0);
   if (s->kind == EM_STREAM_BANK || s->kind == EM_STREAM_SH) {
     EM_CUDA(cudaEventSynchronize(s->tab_ev));
   }
+  auto blk_frames = [&](int b, long long& f0, int& nfb) {
+    const long long t_lo = t_first + (long long)b * B;
+    f0 = t_lo / hop;
+    nfb = (int)((t_lo + B - 1) / hop - f0 + 1);
+  };
   if (s->kind == EM_STREAM_BANK) {
+    const auto page = [&](long long f, int l) { return s->trk[(size_t)((f - s->trk_base) * L + l)]; };
+    std::vector<int>& uni = s->uni;
+    std::vector<int>& mark = s->mark;
+    const auto add = [&](int p) {
+      if (mark[p] < 0) { mark[p] = 0; uni.push_back(p); }
+    };
     int* tab = s->h_tab;
-    int* pg = tab + (nb + 1);
-    int np_total = 0;
-    std::vector<int>& cand = s->cand;
+    int n_cmb = 0;
     for (int b = 0; b < nb; ++b) {
-      tab[b] = np_total;
-      blk_off[b] = np_total;
-      const long long t_lo = t_first + (long long)b * B, t_hi = t_lo + B - 1;
-      cand.clear();
-      for (long long f = t_lo / s->hop; f <= t_hi / s->hop; ++f) {
-        cand.push_back(s->trk[f - s->trk_base]);
-        if (f > 0 && s->fade > 0 && f * s->hop + s->fade - 1 >= t_lo) cand.push_back(s->trk[f - 1 - s->trk_base]);
-      }
-      std::sort(cand.begin(), cand.end());
-      cand.erase(std::unique(cand.begin(), cand.end()), cand.end());
-      for (int p : cand) pg[np_total++] = p;
+      long long f0;
+      int nfb;
+      blk_frames(b, f0, nfb);
+      cmb_off[b] = n_cmb;
+      n_cmb += 2 * L * nfb;
     }
-    tab[nb] = np_total;
+    cmb_off[nb] = n_cmb;
+    int* pg = tab + n_cmb;
+    int np_total = 0;
+    for (int b = 0; b < nb; ++b) {
+      const long long t_lo = t_first + (long long)b * B;
+      long long f0;
+      int nfb;
+      blk_frames(b, f0, nfb);
+      blk_off[b] = np_total;
+      uni.clear();
+      for (int l = 0; l < L; ++l)
+        for (long long f = f0; f < f0 + nfb; ++f) {
+          add(page(f, l));
+          if (f > 0 && s->fade > 0 && f * hop + s->fade - 1 >= t_lo) add(page(f - 1, l));
+        }
+      std::sort(uni.begin(), uni.end());
+      for (int k = 0; k < (int)uni.size(); ++k) {
+        mark[uni[k]] = k;
+        pg[np_total++] = uni[k];
+      }
+      int* e = tab + cmb_off[b];
+      for (int l = 0; l < L; ++l)
+        for (long long f = f0; f < f0 + nfb; ++f, e += 2) {
+          const int c = page(f, l);
+          e[0] = mark[f > 0 ? page(f - 1, l) : c];
+          e[1] = mark[c];
+        }
+      for (int p : uni) mark[p] = -1;
+    }
     blk_off[nb] = np_total;
-    int* tk = pg + np_total;
-    for (long long f = f_first; f <= f_last; ++f) tk[f - f_first] = s->trk[f - s->trk_base];
-    const size_t n_tab = (size_t)(nb + 1) + np_total + (size_t)(f_last - f_first + 1);
-    EM_CUDA(cudaMemcpyAsync(s->d_tab, tab, n_tab * sizeof(int), cudaMemcpyHostToDevice, st));
+    EM_CUDA(cudaMemcpyAsync(s->d_tab, tab, (size_t)(n_cmb + np_total) * sizeof(int), cudaMemcpyHostToDevice, st));
     EM_CUDA(cudaEventRecord(s->tab_ev, st));
   } else if (s->kind == EM_STREAM_SH) {
-    for (long long f = f_first; f <= f_last; ++f)
-      std::memcpy(s->h_rot + 9 * (f - f_first), s->rot[f - s->rot_base].data(), 9 * sizeof(double));
-    EM_CUDA(cudaMemcpyAsync(s->d_rot, s->h_rot, (size_t)(f_last - f_first + 1) * 9 * sizeof(double),
-                            cudaMemcpyHostToDevice, st));
+    for (int l = 0; l < L; ++l)
+      for (long long f = f_first; f <= f_last; ++f)
+        std::memcpy(s->h_rot + 9 * (l * nfr_c + f - f_first), s->rot[(size_t)((f - s->rot_base) * L + l)].data(),
+                    9 * sizeof(double));
+    EM_CUDA(cudaMemcpyAsync(s->d_rot, s->h_rot, (size_t)L * nfr_c * 9 * sizeof(double), cudaMemcpyHostToDevice, st));
     EM_CUDA(cudaEventRecord(s->tab_ev, st));
   }
-  const int* d_pages = s->d_tab + (nb + 1);
-  const int* d_trk = d_pages + blk_off[nb];
 
   for (int b = 0; b < nb; ++b) {
     const long long k = s->T / B, t_lo = s->T;
@@ -462,31 +539,33 @@ void run_chunk(emagls_stream_ctx* s, const double* in, long long ld_in, int nb, 
     long long ld = ld_in;
     if (s->kind == EM_STREAM_SH) {
       ProfSpan ps(h, EM_PROF_RENDER_STAGE);
-      const long long fb = std::max<long long>(t_lo / s->hop - 1, 0), fh = (t_lo + B - 1) / s->hop;
-      launch_frame_rotations(h, s->d_rot, f_first, fb, fh - fb + 1, s->order, s->Q, s->same);
-      launch_sh_track_rotate(h, in, ld_in, (long long)b * B, B, s->order, s->Q, s->same, fb, t_first, s->hop, s->fade,
-                             s->rbuf);
+      const long long fb = std::max<long long>(t_lo / hop - 1, 0), fh = (t_lo + B - 1) / hop;
+      launch_frame_rotations(h, L, s->d_rot, nfr_c * 9, f_first, fb, fh - fb + 1, s->order, s->Q, s->same, s->nfr_blk);
+      launch_sh_track_rotate(h, L, in, ld_in, (long long)b * B, B, s->order, s->Q, s->same, s->nfr_blk, fb, t_first,
+                             hop, s->fade, s->rbuf, (long long)num_ch * B);
       h->launches += 2;
       src = s->rbuf;
       ld = B;
     }
+    const long long xs = (long long)s->xch * F;   // slot stride of the FDL
     {
       ProfSpan ps(h, EM_PROF_RENDER_STAGE);
-      stream_stage_kernel<<<(num_ch * B + 255) / 256, 256, 0, st>>>(src, ld, num_ch, B, s->prev, s->seg);
+      const long long n = (long long)s->xch * B;
+      stream_stage_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(src, ld, s->xch, B, s->prev, s->seg);
       EM_CUDA(cudaGetLastError());
     }
     {
       ProfSpan ps(h, EM_PROF_RENDER_FFT);
-      EM_FFT(cufftExecD2Z(s->fwd, s->seg, reinterpret_cast<cufftDoubleComplex*>(s->X + (long long)slot * num_ch * F)));
+      EM_FFT(cufftExecD2Z(s->fwd, s->seg, reinterpret_cast<cufftDoubleComplex*>(s->X + slot * xs)));
     }
     const bool bank = s->kind == EM_STREAM_BANK;
     const int np = bank ? blk_off[b + 1] - blk_off[b] : 1;
-    const int* pages = bank ? d_pages + blk_off[b] : s->d_zero;
+    const int* pages = bank ? s->d_tab + cmb_off[nb] + blk_off[b] : s->d_zero;
     constexpr int G = 4;
     {
       ProfSpan ps(h, EM_PROF_RENDER_MAC);
-      dim3 grid((unsigned)((F + 127) / 128), (unsigned)((np + G - 1) / G));
-      stream_mac_kernel<G><<<grid, 128, 0, st>>>(s->X, s->H, pages, np, num_ch, P, F, slot, s->Y);
+      dim3 grid((unsigned)((F + 127) / 128), (unsigned)((np + G - 1) / G), bank ? 1u : (unsigned)s->pcap);
+      stream_mac_kernel<G><<<grid, 128, 0, st>>>(s->X, xs, s->H, pages, np, num_ch, P, F, slot, s->Y);
       EM_CUDA(cudaGetLastError());
     }
     {
@@ -497,8 +576,12 @@ void run_chunk(emagls_stream_ctx* s, const double* in, long long ld_in, int nb, 
     }
     {
       ProfSpan ps(h, EM_PROF_RENDER_STAGE);
-      stream_combine_kernel<<<(B + 127) / 128, 128, 0, st>>>(s->yseg, pages, np, bank ? d_trk : nullptr, f_first,
-                                                             t_lo, B, s->hop, s->fade, ld_out, out + (long long)b * B);
+      long long f0 = 0;
+      int nfb = 0;
+      blk_frames(b, f0, nfb);
+      stream_combine_kernel<<<dim3((unsigned)((B + 127) / 128), (unsigned)L), 128, 0, st>>>(
+          s->yseg, bank ? s->d_tab + cmb_off[b] : nullptr, f0, nfb, t_lo, B, hop, s->fade, ld_out,
+          out + (long long)b * B);
       EM_CUDA(cudaGetLastError());
     }
     h->launches += 5;
@@ -513,6 +596,7 @@ void process(emagls_stream_ctx* s, const double* in, long long num_samples, cons
   emagls_ctx* h = s->h;
   cudaStream_t st = h->stream;
   const long long cs = (long long)s->cb * s->B;
+  const int no = 2 * s->nl;   // output rows: (listener, ear)
   for (long long c0 = 0; c0 < num_samples; c0 += cs) {
     const long long cn = std::min(cs, num_samples - c0);
     const int nb = (int)(cn / s->B);
@@ -523,19 +607,20 @@ void process(emagls_stream_ctx* s, const double* in, long long num_samples, cons
         std::memcpy(s->h_in + (long long)ch * cn, in + (long long)ch * num_samples + c0, (size_t)cn * sizeof(double));
       EM_CUDA(cudaMemcpyAsync(s->d_in, s->h_in, (size_t)s->num_ch * cn * sizeof(double), cudaMemcpyHostToDevice, st));
       run_chunk(s, s->d_in, cn, nb, s->d_out, cn);
-      EM_CUDA(cudaMemcpyAsync(s->h_out, s->d_out, (size_t)2 * cn * sizeof(double), cudaMemcpyDeviceToHost, st));
+      EM_CUDA(cudaMemcpyAsync(s->h_out, s->d_out, (size_t)no * cn * sizeof(double), cudaMemcpyDeviceToHost, st));
       EM_CUDA(cudaStreamSynchronize(st));
-      for (int ear = 0; ear < 2; ++ear)
-        std::memcpy(out + (long long)ear * num_samples + c0, s->h_out + (long long)ear * cn, (size_t)cn * sizeof(double));
+      for (int r = 0; r < no; ++r)
+        std::memcpy(out + (long long)r * num_samples + c0, s->h_out + (long long)r * cn, (size_t)cn * sizeof(double));
     }
     trim_entries(s);
   }
 }
 
-void check_create(const double* wL, const double* wR, int len, int num_ch, int num_pages, int block, int hop, int fade,
-                  const emagls_render_stream* out) {
+void check_create(const double* wL, const double* wR, int len, int num_ch, int num_pages, int num_listeners, int block,
+                  int hop, int fade, const emagls_render_stream* out) {
   EM_REQUIRE(wL && wR && out, "null argument");
   EM_REQUIRE(len > 0 && num_ch > 0 && num_pages > 0, "empty filters");
+  EM_REQUIRE(num_listeners >= 1 && num_listeners <= ST_MAX_LISTENERS, "num_listeners must lie in [1, 4096]");
   EM_REQUIRE(block >= ST_MIN_BLOCK && block <= ST_MAX_BLOCK, "block must lie in [16, 8192]");
   EM_REQUIRE(hop >= 1, "hop must be >= 1");
   EM_REQUIRE(fade >= 0 && fade <= hop, "fade must lie in [0, hop]");
@@ -559,25 +644,41 @@ using namespace emagls;
 
 extern "C" {
 
-int emagls_render_stream_create(emagls_handle h, const double* wL, const double* wR, int len, int num_ch,
-                                int num_pages, int block, int hop, int fade, emagls_render_stream* out) {
+int emagls_render_stream_create_listeners(emagls_handle h, const double* wL, const double* wR, int len, int num_ch,
+                                          int num_pages, int num_listeners, int block, int hop, int fade,
+                                          emagls_render_stream* out) {
   if (out) *out = nullptr;
   return guarded(h, [&] {
-    check_create(wL, wR, len, num_ch, num_pages, block, hop, fade, out);
+    check_create(wL, wR, len, num_ch, num_pages, num_listeners, block, hop, fade, out);
+    EM_REQUIRE(num_listeners == 1 || num_pages > 1, "a static session (num_pages == 1) serves one listener");
     const int kind = num_pages == 1 ? EM_STREAM_STATIC : EM_STREAM_BANK;
-    open_session(h, create_session(h, kind, wL, wR, len, num_ch, num_pages, 0, block, hop, fade), out);
+    open_session(h, create_session(h, kind, wL, wR, len, num_ch, num_pages, 0, num_listeners, block, hop, fade), out);
+  });
+}
+
+int emagls_render_stream_create(emagls_handle h, const double* wL, const double* wR, int len, int num_ch,
+                                int num_pages, int block, int hop, int fade, emagls_render_stream* out) {
+  return emagls_render_stream_create_listeners(h, wL, wR, len, num_ch, num_pages, 1, block, hop, fade, out);
+}
+
+int emagls_render_stream_create_sh_listeners(emagls_handle h, const double* wL, const double* wR, int len, int order,
+                                             int num_listeners, int block, int hop, int fade,
+                                             emagls_render_stream* out) {
+  if (out) *out = nullptr;
+  return guarded(h, [&] {
+    EM_REQUIRE(order >= 0 && order <= ST_MAX_ORDER, "order must lie in [0, 7]");
+    const int C = (order + 1) * (order + 1);
+    check_create(wL, wR, len, C, 1, num_listeners, block, hop, fade, out);
+    // the per-block forward transform (one cuFFT plan of 32-bit sizes) takes every listener's rotated block
+    EM_REQUIRE((long long)num_listeners * C * 2 * block <= 2147483647LL,
+               "num_listeners (order + 1)^2 2 block must stay below 2^31");
+    open_session(h, create_session(h, EM_STREAM_SH, wL, wR, len, C, 1, order, num_listeners, block, hop, fade), out);
   });
 }
 
 int emagls_render_stream_create_sh(emagls_handle h, const double* wL, const double* wR, int len, int order,
                                    int block, int hop, int fade, emagls_render_stream* out) {
-  if (out) *out = nullptr;
-  return guarded(h, [&] {
-    EM_REQUIRE(order >= 0 && order <= ST_MAX_ORDER, "order must lie in [0, 7]");
-    const int C = (order + 1) * (order + 1);
-    check_create(wL, wR, len, C, 1, block, hop, fade, out);
-    open_session(h, create_session(h, EM_STREAM_SH, wL, wR, len, C, 1, order, block, hop, fade), out);
-  });
+  return emagls_render_stream_create_sh_listeners(h, wL, wR, len, order, 1, block, hop, fade, out);
 }
 
 int emagls_render_stream_process(emagls_render_stream s, const double* in, long long num_samples,

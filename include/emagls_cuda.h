@@ -308,12 +308,37 @@ int emagls_binaural_decode_sh_tracked_dev(emagls_handle h, const double* in, lon
  * (appended entries included): create: a null pointer, block outside [16, 8192], hop < 1, fade outside [0, hop],
  * num_pages < 1, order outside [0, 7]; process: a null pointer, num_samples not a positive multiple of block, entries
  * that do not cover the call, a page outside [0, num_pages), the wrong kind of tracker pointer for the session, a
- * track on a static session, num_new_frames < 0.                                                                     */
+ * track on a static session, num_new_frames < 0.
+ * Listeners: _create_listeners / _create_sh_listeners open a session for num_listeners (L) listeners who hear one
+ * shared input stream, each with their own tracker entries; _create and _create_sh mean L = 1.  The layouts below
+ * generalise those above and are them for L = 1: in [num_samples x num_ch] (shared); track [num_new_frames x L],
+ * column-major: track[l * num_new_frames + j] is listener l's page of the j-th new frame; rotations: one row-major
+ * 3x3 matrix at rotations + 9 * (l * num_new_frames + j); out [num_samples x 2 x L]: out[(2 l + ear) * num_samples + i].
+ * Every listener appends the same num_new_frames per call, and the coverage rule is the one above.  After T samples,
+ * listener l's concatenated output equals what a one-listener session fed the same input and listener l's entries
+ * returns, and so the whole-signal render above of x[0:T] with listener l's entries; it does not depend on the
+ * other listeners or their order.  A block of a bank session renders each page its listeners need once (the union of
+ * at most num_pages pages), and a block takes the same number of launches whatever L (DESIGN.md section 14).
+ * Memory: the bank's spectra once per session (size above); per listener, the pair buffers
+ * (2 (2 block + 1) 16 + 4 block 8 bytes per pair, up to the next power of two of min(num_pages, L pmax) pairs for a
+ * bank session, pmax = min(num_pages, (block - 1) / hop + 3)), the output staging (2 * 8 bytes per sample of a chunk,
+ * host and device) and, for SH sessions, the FDL (num_ch ceil(len / block) (block + 1) 16 bytes), the rotated and
+ * staged block (4 num_ch block 8 bytes) and the frame rotations.  Listeners are fixed seats: a server gives a free seat
+ * to a new listener.  The shared input's history is right for the newcomer; in an SH seat the previous occupant's
+ * rotations leave the output within len samples.  EMAGLS_ERR_INVALID, besides the cases above: num_listeners outside
+ * [1, 4096], num_listeners > 1 with num_pages == 1 (a static session), num_listeners (order + 1)^2 2 block >= 2^31
+ * (SH); every check of a process call applies to the entries of every listener.                                                                                         */
 typedef struct emagls_stream_ctx* emagls_render_stream;
 int emagls_render_stream_create(emagls_handle h, const double* wL, const double* wR, int len, int num_ch,
                                 int num_pages, int block, int hop, int fade, emagls_render_stream* out);
 int emagls_render_stream_create_sh(emagls_handle h, const double* wL, const double* wR, int len, int order,
                                    int block, int hop, int fade, emagls_render_stream* out);
+int emagls_render_stream_create_listeners(emagls_handle h, const double* wL, const double* wR, int len, int num_ch,
+                                          int num_pages, int num_listeners, int block, int hop, int fade,
+                                          emagls_render_stream* out);
+int emagls_render_stream_create_sh_listeners(emagls_handle h, const double* wL, const double* wR, int len, int order,
+                                             int num_listeners, int block, int hop, int fade,
+                                             emagls_render_stream* out);
 int emagls_render_stream_process(emagls_render_stream s, const double* in, long long num_samples,
                                  const int32_t* track, const double* rotations, long long num_new_frames,
                                  double* out);
